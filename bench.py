@@ -63,7 +63,14 @@ def parse():
                          "(sharded storage + the library's NCCL at N > 1; extra JSON key `ransac`): c4 = the 10 M-point "
                          "CAD-like scene BASELINE.json's second headline is quoted on, c5 = the 100 M-point LiDAR-like scan")
     ap.add_argument("--no-strong", action="store_true", help="skip the strong-scaled c3 leg at N > 1")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed calls returned in their last step to DIR/<name>.npy (float32 / float64): the "
+                         "per-candidate counts and, for every --ransac scene, the extracted shapes, their inlier totals and "
+                         "(at N = 1) the shape each point of a fixed strided sample went to")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 class ClockSampler:
@@ -304,6 +311,7 @@ def main():
         b.record()
     t_b.record()
     torch.cuda.synchronize()
+    counts_host = d_counts.cpu().numpy()  # the counts of the last timed step
     if world > 1:
         dist.barrier()
     total_ms = t_a.elapsed_time(t_b)
@@ -324,7 +332,6 @@ def main():
         k, guard = _last_kernel(pc)
         kms.append(k)
     kernel_ms = float(np.mean(kms))
-    counts_host = d_counts.cpu().numpy()
 
     # ---- e2e arm: host buffers through the public call -----------------------------------------
     e2e = None
@@ -395,6 +402,7 @@ def main():
 
     # ---- end-to-end ransac() at this N (all ranks take part) ----
     ransac_out = None
+    extracted = {}  # scene -> what ransac() returned in the last timed run
     scenes_req = [s for s in args.ransac.split(",") if s and s != "none"]
     if scenes_req:
         # free the microbenchmark's device buffers first (c5 needs 2.4 GB per replica at N = 1)
@@ -404,8 +412,9 @@ def main():
         ransac_out = {}
         for which in scenes_req:
             try:
-                ransac_out[which] = ransac_e2e.run(which, rank, world, local, dist if world > 1 else None,
-                                                   cpu_loop=not args.no_cpu)
+                ransac_out[which], extracted[which] = ransac_e2e.run(which, rank, world, local, dist if world > 1 else None,
+                                                                     cpu_loop=not args.no_cpu, reps=args.steps,
+                                                                     return_extracted=True)
             except Exception as e:  # informational keys: never lose the headline line
                 ransac_out[which] = {"error": repr(e)}
                 if world > 1:
@@ -504,9 +513,34 @@ def main():
             out["culled_variant"] = time_culled_variant(R, pc, cands, params)
         except Exception as e:
             out["culled_variant"] = {"error": repr(e)}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, counts_host, extracted, world)
     print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(dirname, counts, extracted, world, sample=1 << 20):
+    """--dump-outputs: the per-candidate counts of the last timed step and, per ransac() scene, the extracted shapes
+    (rows: type, outwards, p[7]) and their inlier totals.  The full inlier lists (up to 10^8 indices) are represented
+    by a strided sample of about `sample` point indices 0, s, 2s, ...: the extraction order of the shape that took
+    each one, -1 if none.  Rank 0 holds only its own point range at N > 1, so the sample is written at N = 1 only."""
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, "score_counts.npy"), counts.astype(np.float64))
+    for which, ex in extracted.items():
+        cands = [e.shape.to_cand() for e in ex]
+        shapes = np.array([[c.type, c.outwards, *c.p] for c in cands], np.float64).reshape(len(cands), 9)
+        np.save(os.path.join(dirname, f"ransac_{which}_shapes.npy"), shapes)
+        np.save(os.path.join(dirname, f"ransac_{which}_inliers.npy"), np.array([e.total for e in ex], np.float64))
+        if world == 1:
+            from tools.ransac_e2e import SCENES
+
+            n = SCENES[which][0]
+            step = max(1, n // sample)
+            label = np.full((n + step - 1) // step, -1, np.float32)
+            for k, e in enumerate(ex):
+                label[e.inpoints[e.inpoints % step == 0] // step] = k
+            np.save(os.path.join(dirname, f"ransac_{which}_sampled_point_shape.npy"), label)
 
 
 def time_culled_variant(R, pc, cands, params, reps=3):

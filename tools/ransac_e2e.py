@@ -125,7 +125,8 @@ def replay_local(extracted, V, N, params, nthreads):
 
 
 def run(which: str, rank: int, world: int, local: int, dist=None, n_override: int = 0, check: bool = True, cpu_loop: bool = True,
-        reps: int = 5):
+        reps: int = 5, return_extracted: bool = False):
+    """The JSON record of `which`; with return_extracted, (record, what ransac() returned in the last timed run)."""
     import torch
 
     import ransac_jl_b200 as R
@@ -192,6 +193,7 @@ def run(which: str, rank: int, world: int, local: int, dist=None, n_override: in
         if best is None or res["seconds"] < best[0]["seconds"]:
             best = (res, ex, pc.isenabled)
         pc.close()
+    ex_last = ex
     res, ex, enabled_local = best
     res = dict(res, seconds_all_runs=all_secs, timing=f"best of {reps} runs (all listed), each from pageable host arrays to the result on the host")
     # the same call with the caller's arrays in PAGE-LOCKED memory (include/rsc.h: read by DMA, no staging copy on the host)
@@ -268,7 +270,7 @@ def run(which: str, rank: int, world: int, local: int, dist=None, n_override: in
                                    "timing": "host arrays -> octree cells -> ransac() -> result on the host"}
         except Exception as e:  # informational
             out["cell_sampler"] = {"error": repr(e)}
-    return out
+    return (out, ex_last) if return_extracted else out
 
 
 def recall(sc, ex, thresh=0.5):
