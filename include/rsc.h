@@ -346,6 +346,34 @@ int32_t rsc_run_syncs(const rsc_run* run, int32_t* batches);
 int32_t rsc_run_inpoints(const rsc_run* run, int32_t i, int64_t* out_idx);
 void rsc_run_destroy(rsc_run* run);
 
+/* ---- user-defined shapes on the device (docs/src/newprimitive.md:12-18) ------------------------
+ * A user shape brings its compatibility test as CUDA C source defining
+ *   __device__ bool rsc_user_compatible(const double p[7], int outwards, const double k[8],
+ *                                       double x, double y, double z, double nx, double ny, double nz);
+ * p / outwards are the candidate's rsc_cand fields (cand.type = the id returned below), k the constants
+ * passed with each call (nk <= 8, e.g. eps and cos(alpha), computed on the host), x..nz the point's float32
+ * coordinates and normal widened to double.  The library gates every point on its enabled bit itself.
+ * libnvrtc.so.12 (dlopen-ed on first use) compiles the source with the library's kernel template for sm_100a,
+ * --fmad=false and no fast-math: float64 + - * / sqrt round to nearest, so a host restatement in the same
+ * operation order makes the same decisions (DESIGN.md section 8).  Fitting stays with the caller.  Not for
+ * sharded or ranged clouds (RSC_E_STATE).  The source is passed as bytes + length. */
+#define RSC_USER_TYPE0 16
+/* compile only, no device needed: RSC_OK or RSC_E_ARG (RSC_E_STATE: NVRTC cannot be loaded); NVRTC's log
+ * (ptxas -v included), NUL-terminated, into log[0..log_cap) (nullable) */
+int32_t rsc_user_shape_check(const void* src, int64_t nbytes, void* log, int64_t log_cap);
+/* compile + load on ctx, cached by the source bytes (the same source gives the same id);
+ * *type_id >= RSC_USER_TYPE0.  Failure: RSC_E_ARG with NVRTC's log in rsc_last_error. */
+int32_t rsc_user_shape_compile(rsc_ctx* ctx, const void* src, int64_t nbytes, int32_t* type_id);
+/* rsc_score for C candidates of ONE compiled user type: counts[c] = compatible enabled points of subset
+ * subset_id (-1 = the whole cloud); masks = NULL or C x ceil(M/32) words in rsc_score's layout */
+int32_t rsc_user_score(rsc_cloud* cloud, const double* k, int32_t nk, const rsc_cand* cands, int32_t C,
+                       int32_t subset_id, int32_t* counts, uint32_t* masks);
+/* rsc_refit_extract for one user-shape candidate: ascending global indices of its compatible enabled
+ * points into out_idx (nullable), *out_n how many; disable != 0 clears their enabled bits (and those of
+ * the uploaded subsets) */
+int32_t rsc_user_refit_extract(rsc_cloud* cloud, const double* k, int32_t nk, const rsc_cand* cand,
+                               int64_t* out_idx, int64_t* out_n, int32_t disable);
+
 #ifdef __cplusplus
 }
 #endif

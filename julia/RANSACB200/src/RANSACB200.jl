@@ -279,6 +279,48 @@ function loop_with_sets(pc::RANSACCloud, params, sets)
     extracted, extracted_at, iterations
 end
 
+# ---- user-defined shapes on the device (include/rsc.h "user-defined shapes") -----------------------------
+"""
+    compile_user_shape(src::String) -> type id
+
+Compiles a user shape's CUDA source (it defines `rsc_user_compatible`) with NVRTC on the context's device;
+the same source returns the same id (>= RSC_USER_TYPE0 = 16).  A compile error raises with NVRTC's log.
+"""
+function compile_user_shape(src::String)
+    id = Ref{Int32}(0)
+    check(ccall(fn(:rsc_user_shape_compile), Int32, (Ptr{Cvoid}, Ptr{UInt8}, Int64, Ref{Int32}),
+                context(), src, sizeof(src), id))
+    id[]
+end
+
+"""
+    user_score!(counts, masks, dc, recs, k, subsetID)
+
+`scorecandidate` for user-shape records of ONE compiled type (`RscCand(type_id, outwards, p)`): compatible
+enabled points of subset `subsetID` (1-based; 0 = the whole cloud) into `counts`, and their bitmasks into
+`masks` (`cld(M, 32)` x C `UInt32`, or `nothing`).  `k` = up to 8 constants (e.g. ϵ, cos α).
+"""
+function user_score!(counts::Vector{Int32}, masks::Union{Nothing,Matrix{UInt32}}, dc::DeviceCloud, recs::Vector{RscCand},
+                     k::Vector{Float64}, subsetID::Integer)
+    check(ccall(fn(:rsc_user_score), Int32,
+                (Ptr{Cvoid}, Ptr{Float64}, Int32, Ptr{RscCand}, Int32, Int32, Ptr{Int32}, Ptr{UInt32}),
+                dc.h, k, length(k), recs, length(recs), subsetID - 1, counts,
+                masks === nothing ? Ptr{UInt32}(C_NULL) : masks))
+    counts
+end
+
+"`refit` + `invalidate_indexes!` of a user-shape record on the device: 1-based inlier indices."
+function user_refit_extract(dc::DeviceCloud, rec::RscCand, k::Vector{Float64}; disable::Bool=true)
+    out = Vector{Int64}(undef, dc.pc.size)
+    n = Ref{Int64}(0)
+    check(ccall(fn(:rsc_user_refit_extract), Int32,
+                (Ptr{Cvoid}, Ptr{Float64}, Int32, Ref{RscCand}, Ptr{Int64}, Ref{Int64}, Int32),
+                dc.h, k, length(k), Ref(rec), out, n, disable))
+    resize!(out, n[])
+    disable && pull_enabled!(dc)
+    out .+ 1
+end
+
 # ---- one process per GPU: sharded storage (include/rsc.h "point-range sharding") ---------------------
 "rank 0: the 128-byte NCCL id to hand to the other ranks (MPI.jl bcast, a socket, a file)"
 function comm_unique_id()

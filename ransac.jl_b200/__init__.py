@@ -27,6 +27,7 @@ from .fitting import (
     scorecandidate,
     scorecandidates,
     unpack_mask,
+    user_score_counts,
 )
 from .iterations import ransac
 from .jsonyaml import dict2nt, exportJSON, readconfig, toDict

@@ -16,6 +16,8 @@ RSC_NTYPES = 4
 RSC_S_LENGTHC, RSC_S_ALLCAND, RSC_S_NOFMINSET = 0, 1, 2
 RSC_COMPAT_SPHERE_IGNORES_ENABLED = 1
 RSC_E_NODEVICE = -3
+RSC_E_ARG, RSC_E_STATE = -1, -5
+RSC_USER_TYPE0 = 16  # type ids of user-defined shapes compiled on a context (rsc_user_shape_compile)
 
 ERRORS = {-1: "RSC_E_ARG", -2: "RSC_E_CUDA", -3: "RSC_E_NODEVICE", -4: "RSC_E_NOMEM", -5: "RSC_E_STATE", -6: "RSC_E_NCCL"}
 
@@ -125,6 +127,10 @@ SIGNATURES = {
     "rsc_run_shape": (C.c_int32, [_P, C.c_int32, C.POINTER(rsc_cand), C.POINTER(C.c_int64)]),
     "rsc_run_inpoints": (C.c_int32, [_P, C.c_int32, _P]),
     "rsc_run_destroy": (None, [_P]),
+    "rsc_user_shape_check": (C.c_int32, [_P, C.c_int64, _P, C.c_int64]),
+    "rsc_user_shape_compile": (C.c_int32, [_P, _P, C.c_int64, C.POINTER(C.c_int32)]),
+    "rsc_user_score": (C.c_int32, [_P, _P, C.c_int32, _P, C.c_int32, C.c_int32, _P, _P]),
+    "rsc_user_refit_extract": (C.c_int32, [_P, _P, C.c_int32, C.POINTER(rsc_cand), _P, C.POINTER(C.c_int64), C.c_int32]),
 }
 
 if not os.path.exists(LIB_PATH):
@@ -191,6 +197,7 @@ class Context:
             raise RscError(rc, "rsc_ctx_create failed (an sm_100 / B200 device is required; no CPU fallback)")
         self.h = h
         self.device = device
+        self._user_types: dict = {}  # user shape class -> type id of its compiled cuda_source
 
     @classmethod
     def get(cls, device: int = 0) -> "Context":
@@ -206,6 +213,17 @@ class Context:
         s = rsc_stats()
         self.check(lib.rsc_ctx_stats(self.h, C.byref(s)))
         return s
+
+    def user_type(self, shape_class) -> int:
+        """Type id of a user-defined shape class with `cuda_source` on this context: compiled with NVRTC on first
+        use (rsc_user_shape_compile; the library caches by source, so equal sources share one id)."""
+        tid = self._user_types.get(shape_class)
+        if tid is None:
+            src = shape_class.cuda_source.encode()
+            out = C.c_int32()
+            self.check(lib.rsc_user_shape_compile(self.h, src, len(src), C.byref(out)))
+            tid = self._user_types[shape_class] = out.value
+        return tid
 
     @property
     def stream(self) -> int:

@@ -130,6 +130,7 @@ void rsc_ctx_destroy(rsc_ctx* ctx) {
                          &ctx->aux,      &ctx->misc,     &ctx->misc2,    &ctx->idxbuf,  &ctx->fitbuf, &ctx->selbuf, &ctx->exq, &ctx->scanbuf, &ctx->lsqbuf, &ctx->cullbuf, &ctx->shardbuf, &ctx->gselbuf, &ctx->smallbuf, &ctx->viewtmp};
   for (auto* b : bufs) b->release();
   rsc::loop_scratch_free(ctx);
+  rsc::user_shapes_free(ctx);
   if (ctx->comm) rsc_ctx_comm_destroy(ctx);
   ctx->stage[0].release(), ctx->stage[1].release();
   if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);

@@ -111,6 +111,7 @@ struct rsc_ctx {
   int bitmap_eight = 0;
   void* pinned = nullptr;    // small pinned staging area
   size_t pinned_cap = 0;
+  void* user_shapes = nullptr;  // rsc::UserShapes of rsc_user.cu: the NVRTC-compiled programs of user-defined shapes
 };
 
 struct rsc_subset {
@@ -309,6 +310,12 @@ int32_t scan_u32(rsc_ctx* ctx, const uint32_t* counts, int n, unsigned long long
 int32_t refit_mask_enqueue(rsc_cloud* cloud, const Thresh& th, const rsc_cand& cand, cudaStream_t st, int timed_reps = 1);
 int32_t refit_write_enqueue(rsc_cloud* cloud, int64_t* d_out, bool disable, cudaStream_t st);
 int32_t refit_mask_from_list(rsc_cloud* cloud, const int64_t* d_list, int64_t n, cudaStream_t st);
+// for a mask written by another kernel (user shapes, rsc_user.cu): *inl = the n_pad/32 inlier-mask words refit_mask_enqueue
+// would write; refit_scan_enqueue then counts and scans them for refit_write_enqueue (total in ctx->misc2[0])
+int32_t refit_mask_buffer(rsc_cloud* cloud, uint32_t** inl);
+int32_t refit_scan_enqueue(rsc_cloud* cloud, cudaStream_t st);
+// unloads the user-shape programs of a context (rsc_ctx_destroy)
+void user_shapes_free(rsc_ctx* ctx);
 // parameter-space bitmap filter (rsc_bitmap.cu): the points of d_idx whose cell lies in the largest connected
 // component -> d_out (capacity n); synchronises `st`
 int32_t bitmap_filter_dev(rsc_cloud* cloud, const rsc_cand& cand, double beta, bool eight, const int64_t* d_idx, int64_t n,

@@ -309,6 +309,29 @@ int32_t refit_mask_from_list(rsc_cloud* cloud, const int64_t* d_list, int64_t n,
   return scan_u32(ctx, block_counts, nblocks, offsets, ctx->misc2.as<unsigned long long>(), st);
 }
 
+int32_t refit_mask_buffer(rsc_cloud* cloud, uint32_t** inl) {
+  rsc_ctx* ctx = cloud->ctx;
+  const int64_t words = cloud->n_pad / 32;
+  const int nblocks = (int)((cloud->n_pad + kExPts - 1) / kExPts);
+  RSC_CUDA(ctx, ctx->idxbuf.ensure((size_t)words * 4 + (size_t)nblocks * (4 + 8) + 64));
+  RSC_CUDA(ctx, ctx->misc2.ensure(64));
+  *inl = ctx->idxbuf.as<uint32_t>();
+  return RSC_OK;
+}
+
+int32_t refit_scan_enqueue(rsc_cloud* cloud, cudaStream_t st) {
+  rsc_ctx* ctx = cloud->ctx;
+  const int64_t words = cloud->n_pad / 32;
+  const int nblocks = (int)((cloud->n_pad + kExPts - 1) / kExPts);
+  char* b = ctx->idxbuf.as<char>();
+  const uint32_t* inl = reinterpret_cast<const uint32_t*>(b);
+  unsigned long long* offsets = reinterpret_cast<unsigned long long*>(b + ((size_t)words * 4 + 15) / 16 * 16);
+  uint32_t* block_counts = reinterpret_cast<uint32_t*>(offsets + nblocks);
+  block_count_kernel<<<(unsigned)(((int64_t)nblocks * 32 + 255) / 256), 256, 0, st>>>(inl, words, block_counts, nblocks);
+  RSC_CUDA(ctx, cudaGetLastError());
+  return scan_u32(ctx, block_counts, nblocks, offsets, ctx->misc2.as<unsigned long long>(), st);
+}
+
 int32_t refit_write_enqueue(rsc_cloud* cloud, int64_t* d_out, bool disable, cudaStream_t st) {
   rsc_ctx* ctx = cloud->ctx;
   const int64_t n_pad = cloud->n_pad;

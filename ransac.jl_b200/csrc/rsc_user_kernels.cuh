@@ -1,0 +1,123 @@
+// rsc_user_kernels.cuh -- the kernels of user-defined shapes, compiled at run time with NVRTC (rsc_user.cu).
+//
+// The library embeds this file as a string and compiles it together with the user's source, which defines
+//
+//   __device__ bool rsc_user_compatible(const double p[7], int outwards, const double k[8],
+//                                       double x, double y, double z, double nx, double ny, double nz);
+//
+// for sm_100a with --fmad=false and no fast-math, so that a NumPy restatement in the same operation order makes
+// the same float64 decisions (DESIGN.md section 8).  The argument structs below are also compiled into the
+// library itself (nvcc): one definition, one layout on both sides of the cudaLaunchKernel call.  Only plain
+// types appear in them -- NVRTC sees no system header.
+#pragma once
+
+struct RscUserPoints {  // = rsc::PointSet
+  const float* x;
+  const float* y;
+  const float* z;
+  const float* nx;
+  const float* ny;
+  const float* nz;
+  const unsigned* enabled;  // bit j%32 of word j/32 = pc.isenabled of point j
+  const unsigned* valid;    // 1 for real points, 0 for padding
+  long long n;
+  long long n_pad;  // multiple of 512
+};
+
+struct RscUserCand {  // = rsc_cand (64 bytes)
+  int type;
+  int outwards;
+  double p[7];
+};
+
+struct RscUserScoreArgs {
+  RscUserPoints ps;
+  const RscUserCand* cands;  // [C], one user type
+  int C;
+  int nk;
+  double k[8];
+  int* counts;       // [C], zeroed by the host
+  unsigned* masks;   // nullable: candidate-major [C][words], zeroed by the host
+  long long words;   // ceil(n / 32)
+};
+
+struct RscUserMaskArgs {
+  RscUserPoints ps;
+  RscUserCand cand;
+  int nk;
+  double k[8];
+  unsigned* inl;  // [n_pad / 32] inlier-mask words (enabled points only)
+};
+
+#define RSC_USER_THREADS 256
+#define RSC_USER_TILE 128  // candidate records staged in shared memory per pass
+
+#ifdef __CUDACC_RTC__
+
+__device__ bool rsc_user_compatible(const double p[7], int outwards, const double k[8], double x, double y, double z, double nx,
+                                    double ny, double nz);
+
+// Counts (and masks) of C candidates of one user type: the transposed mapping of the small-batch scorer
+// (rsc_small.cu).  A thread owns a point; the CTA stages a chunk of candidate records in shared memory and reads
+// them as broadcasts; a (candidate, 32 points) group is one ballot, its POPC goes into a shared counter, and each
+// CTA adds one atomic per candidate.  Candidate chunks are spread over gridDim.y.  Every pair is decided once, in
+// float64, on the point's float32 coordinates widened to double.
+extern "C" __global__ void __launch_bounds__(RSC_USER_THREADS) rsc_user_score_kernel(const RscUserScoreArgs a) {
+  __shared__ RscUserCand sc[RSC_USER_TILE];
+  __shared__ int scount[RSC_USER_TILE];
+  __shared__ double sk[8];
+  const int lane = threadIdx.x & 31;
+  if (threadIdx.x < 8) sk[threadIdx.x] = threadIdx.x < a.nk ? a.k[threadIdx.x] : 0.0;
+  const long long ntiles = a.ps.n_pad / RSC_USER_THREADS;
+  for (int c0 = blockIdx.y * RSC_USER_TILE; c0 < a.C; c0 += gridDim.y * RSC_USER_TILE) {
+    const int ct = min(RSC_USER_TILE, a.C - c0);
+    for (int i = threadIdx.x; i < ct; i += RSC_USER_THREADS) {
+      sc[i] = a.cands[c0 + i];
+      scount[i] = 0;
+    }
+    __syncthreads();
+    for (long long t = blockIdx.x; t < ntiles; t += gridDim.x) {
+      const long long p = t * RSC_USER_THREADS + threadIdx.x;
+      const unsigned live = __ldg(a.ps.enabled + (p >> 5)) & __ldg(a.ps.valid + (p >> 5));
+      if (live == 0u) continue;  // warp-uniform: no enabled real point in this group
+      const bool on = (live >> lane) & 1u;
+      const double x = __ldg(a.ps.x + p), y = __ldg(a.ps.y + p), z = __ldg(a.ps.z + p);
+      const double nx = __ldg(a.ps.nx + p), ny = __ldg(a.ps.ny + p), nz = __ldg(a.ps.nz + p);
+      for (int c = 0; c < ct; ++c) {
+        const bool ok = on && rsc_user_compatible(sc[c].p, sc[c].outwards, sk, x, y, z, nx, ny, nz);
+        const unsigned b = __ballot_sync(0xffffffffu, ok);
+        if (lane == 0 && b) {
+          atomicAdd(&scount[c], __popc(b));
+          if (a.masks) a.masks[(long long)(c0 + c) * a.words + (p >> 5)] = b;
+        }
+      }
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < ct; i += RSC_USER_THREADS)
+      if (scount[i]) atomicAdd(a.counts + c0 + i, scount[i]);
+    __syncthreads();
+  }
+}
+
+// The inlier-mask words of one candidate over the whole cloud, enabled points only: what K4's mask kernel writes
+// for a built-in shape (rsc_extract.cu), so that the library's count / scan / compaction follow unchanged.
+extern "C" __global__ void __launch_bounds__(RSC_USER_THREADS) rsc_user_mask_kernel(const RscUserMaskArgs a) {
+  __shared__ RscUserCand sc;
+  __shared__ double sk[8];
+  if (threadIdx.x == 0) sc = a.cand;
+  if (threadIdx.x < 8) sk[threadIdx.x] = threadIdx.x < a.nk ? a.k[threadIdx.x] : 0.0;
+  __syncthreads();
+  const int lane = threadIdx.x & 31;
+  for (long long p = (long long)blockIdx.x * RSC_USER_THREADS + threadIdx.x; p < a.ps.n_pad;
+       p += (long long)gridDim.x * RSC_USER_THREADS) {
+    const unsigned live = __ldg(a.ps.enabled + (p >> 5)) & __ldg(a.ps.valid + (p >> 5));
+    bool ok = false;
+    if ((live >> lane) & 1u)
+      ok = rsc_user_compatible(sc.p, sc.outwards, sk, __ldg(a.ps.x + p), __ldg(a.ps.y + p), __ldg(a.ps.z + p), __ldg(a.ps.nx + p),
+                               __ldg(a.ps.ny + p), __ldg(a.ps.nz + p));
+    const unsigned b = __ballot_sync(0xffffffffu, ok);
+    if (lane == 0) a.inl[p >> 5] = b;
+  }
+}
+
+#endif  // __CUDACC_RTC__

@@ -1,7 +1,8 @@
 """Host-side mirror of the reference's per-shape operator API and candidate bookkeeping:
 `fit`, `scorecandidate(s)`, `refit`, `forcefitshapes`, `IterationCandidates`, `findhighestscore`
 (src/fitting.jl:15-221 and src/shapes/*.jl).  Every built-in shape routes to the CUDA library
-through the C ABI; there is no Python/NumPy implementation of the math here.
+through the C ABI; there is no Python/NumPy implementation of the math here.  User-defined shapes
+with `cuda_source` score and refit on the device too (rsc_user_score, rsc_user_refit_extract).
 """
 from __future__ import annotations
 
@@ -15,7 +16,7 @@ from ._lib import lib
 from .cloud import RANSACCloud
 from .confidence import ConfidenceInterval, estimatescore, estimatescore_f64, isoverlap
 from .params import to_c
-from .shapes import SHAPE_KIND, ExtractedShape, FittedShape, from_cand, pack_cands
+from .shapes import SHAPE_KIND, ExtractedShape, FittedShape, from_cand, on_device, pack_cands, user_cand
 
 
 # ---- fit (fitting.jl:30; plane.jl:33, sphere.jl:87, cylinder.jl:135, cone.jl:123) ------------
@@ -132,14 +133,68 @@ def unpack_mask(row: np.ndarray, M: int) -> np.ndarray:
     return np.unpackbits(row.view(np.uint8), bitorder="little")[:M].astype(bool)
 
 
+def _user_constants(shape_class, params):
+    k = np.ascontiguousarray([float(v) for v in shape_class.device_constants(params)], dtype=np.float64)
+    if len(k) > 8:
+        raise ValueError(f"{shape_class.__name__}.device_constants: at most 8 constants, got {len(k)}")
+    return k
+
+
+def user_score_counts(pc: RANSACCloud, candidates: Sequence[FittedShape], subsetID: int, params, want_masks=False):
+    """Raw device scoring of user-defined shapes of ONE class with `cuda_source` (rsc_user_score, the analogue of
+    `score_counts`): inlier counts (and packed masks) against subset `subsetID` (0-based; -1 = whole cloud)."""
+    Cn = len(candidates)
+    counts = np.zeros(Cn, dtype=np.int32)
+    if Cn == 0:
+        return counts, None
+    cls = type(candidates[0])
+    if not on_device(cls) or any(type(c) is not cls for c in candidates):
+        raise TypeError("user_score_counts: candidates of one user-defined shape class with cuda_source")
+    if subsetID >= 0:
+        pc.upload_subset(subsetID)
+        M = len(pc.subsets[subsetID])
+    else:
+        M = pc.size
+    tid = pc.ctx.user_type(cls)
+    arr = (_lib.rsc_cand * Cn)()
+    for i, c in enumerate(candidates):
+        arr[i] = user_cand(c, tid)
+    k = _user_constants(cls, params)
+    masks = np.zeros((Cn, (M + 31) // 32), dtype=np.uint32) if want_masks else None
+    pc.ctx.check(lib.rsc_user_score(pc.handle, k.ctypes.data, len(k), arr, Cn, subsetID, counts.ctypes.data,
+                                    masks.ctypes.data if want_masks else None))
+    return counts, masks
+
+
+def _builtin_params(params):
+    it = params["iteration"]
+    return dict(params, iteration=dict(it, shape_types=[t for t in it["shape_types"] if t in SHAPE_KIND]))
+
+
 def scorecandidates(pc: RANSACCloud, candidates: Sequence[FittedShape], subsetID: int, params):
-    """scorecandidates!: [(ConfidenceInterval, inpoints)] for all candidates in ONE launch."""
-    counts, masks = score_counts(pc, candidates, subsetID, params, want_masks=True)
+    """scorecandidates!: [(ConfidenceInterval, inpoints)] in input order.  Built-in shapes are scored in ONE
+    launch (rsc_score), each user-defined class with `cuda_source` in one launch of its own (rsc_user_score);
+    any other user-defined shape calls its own `scorecandidate` (docs/src/newprimitive.md:16)."""
     sub = pc.subsets[subsetID]
-    out = []
-    for i in range(len(candidates)):
-        m = unpack_mask(masks[i], len(sub))
-        out.append((estimatescore(len(sub), pc.size, int(counts[i])), sub[m]))
+    out = [None] * len(candidates)
+    groups: dict = {}
+    for i, c in enumerate(candidates):
+        t = type(c)
+        if t in SHAPE_KIND:
+            groups.setdefault(None, []).append(i)
+        elif on_device(t):
+            groups.setdefault(t, []).append(i)
+        else:
+            out[i] = c.scorecandidate(pc, subsetID, params)
+    for cls, idx in groups.items():
+        cs = [candidates[i] for i in idx]
+        if cls is None:
+            counts, masks = score_counts(pc, cs, subsetID, _builtin_params(params), want_masks=True)
+        else:
+            counts, masks = user_score_counts(pc, cs, subsetID, params, want_masks=True)
+        for j, i in enumerate(idx):
+            m = unpack_mask(masks[j], len(sub))
+            out[i] = (estimatescore(len(sub), pc.size, int(counts[j])), sub[m])
     return out
 
 
@@ -164,10 +219,18 @@ def bitmap_filter(s: FittedShape, pc: RANSACCloud, idx, beta: float, eight: bool
 
 # ---- refit (fitting.jl:57; shapes/*.jl refit) + invalidate_indexes! (fitting.jl:197) -----------
 def refit(s: FittedShape, pc: RANSACCloud, params, disable: bool = False) -> ExtractedShape:
-    cand = s.to_cand()
-    cp = to_c(params)
+    """Compatible enabled points of the whole cloud (ascending), optionally disabled: rsc_refit_extract for built-in
+    shapes, rsc_user_refit_extract for user-defined shapes with `cuda_source`."""
     out = np.zeros(pc.size, dtype=np.int64)
     n = C.c_int64()
+    if on_device(type(s)):
+        cand = user_cand(s, pc.ctx.user_type(type(s)))
+        k = _user_constants(type(s), params)
+        pc.ctx.check(lib.rsc_user_refit_extract(pc.handle, k.ctypes.data, len(k), C.byref(cand), out.ctypes.data, C.byref(n),
+                                                int(disable)))
+        return ExtractedShape(s, out[: n.value].copy())
+    cand = s.to_cand()
+    cp = to_c(_builtin_params(params))
     pc.ctx.check(lib.rsc_refit_extract(pc.handle, C.byref(cp), C.byref(cand), out.ctypes.data, C.byref(n), int(disable)))
     return ExtractedShape(s, out[: n.value].copy())
 
@@ -235,8 +298,11 @@ def refine_progressive(pc: RANSACCloud, A: IterationCandidates, params) -> int:
             break
         todo = [i for i in group if A.evaluated[i][0] == lmin]
         dev = [i for i in todo if type(A.shapes[i]) in SHAPE_KIND]
-        counts = dict(zip(dev, score_counts(pc, [A.shapes[i] for i in dev], lmin, params)[0])) if dev else {}
-        for i in todo:  # user-defined shapes score themselves (docs/src/newprimitive.md:16)
+        counts = dict(zip(dev, score_counts(pc, [A.shapes[i] for i in dev], lmin, _builtin_params(params))[0])) if dev else {}
+        for cls in {type(A.shapes[i]) for i in todo if on_device(type(A.shapes[i]))}:  # one launch per user class
+            ui = [i for i in todo if type(A.shapes[i]) is cls]
+            counts.update(zip(ui, user_score_counts(pc, [A.shapes[i] for i in ui], lmin, params)[0]))
+        for i in todo:  # other user-defined shapes score themselves (docs/src/newprimitive.md:16)
             c = counts[i] if i in counts else len(A.shapes[i].scorecandidate(pc, lmin, params)[1])
             ev = A.evaluated[i]
             ev[0], ev[1], ev[2] = ev[0] + 1, ev[1] + int(c), ev[2] + len(pc.subsets[lmin])

@@ -3,7 +3,9 @@
 For the four built-in shape types the whole loop runs inside the CUDA library behind one C-ABI call
 (`rsc_ransac_run`).  If `shape_types` contains a user-defined FittedShape subclass the loop runs
 here and calls that class's own `fit`/`scorecandidate`/`refit` methods -- the reference's plug-in
-contract (docs/src/newprimitive.md:12-18) -- while built-in types still score on the device.
+contract (docs/src/newprimitive.md:12-18) -- while built-in types still score on the device.  A user
+shape with `cuda_source` keeps its own `fit` but scores and refits on the device (rsc_user_score,
+rsc_user_refit_extract).
 """
 from __future__ import annotations
 
@@ -19,7 +21,7 @@ from .cloud import RANSACCloud
 from .confidence import estimatescore_f64, prob
 from .fitting import IterationCandidates, findhighestscore, lsq_refit, refine_progressive, refit, sample_fit, scorecandidates
 from .params import to_c
-from .shapes import SHAPE_KIND, ExtractedShape, from_cand
+from .shapes import SHAPE_KIND, ExtractedShape, from_cand, on_device
 
 
 def _all_builtin(params) -> bool:
@@ -142,8 +144,10 @@ def _ransac_host(pc, params, seed, progressive=False, lsq=False):
             keyed.sort(key=lambda kc: kc[0])  # stable
             cands = [c for _, c in keyed]
         cc[1] += len(cands)
-        b = [c for c in cands if type(c) in SHAPE_KIND]
-        res = dict(zip(map(id, b), scorecandidates(pc, b, 0, bparams))) if b else {}
+        # built-in and device-capable user shapes: one batched call (one launch per class); other user shapes
+        # score themselves
+        b = [c for c in cands if type(c) in SHAPE_KIND or on_device(type(c))]
+        res = dict(zip(map(id, b), scorecandidates(pc, b, 0, params))) if b else {}
         for c in cands:
             sc, ip = res[id(c)] if id(c) in res else c.scorecandidate(pc, 0, params)
             if progressive:
@@ -160,9 +164,10 @@ def _ransac_host(pc, params, seed, progressive=False, lsq=False):
                 shp = scored.shapes[best]
                 if lsq and type(shp) in SHAPE_KIND:
                     shp = lsq_refit(shp, pc, bparams)[0]
-                ex = refit(shp, pc, bparams, disable=True) if type(shp) in SHAPE_KIND else shp.refit(pc, params)
+                dev = type(shp) in SHAPE_KIND or on_device(type(shp))
+                ex = refit(shp, pc, params, disable=True) if dev else shp.refit(pc, params)
                 if ex is not None:  # a user's refit may return nothing: the reference then skips the extraction (iterations.jl:130)
-                    if type(shp) not in SHAPE_KIND:
+                    if not dev:
                         from .fitting import invalidate_indexes
                         invalidate_indexes(pc, ex.inpoints)
                     extracted.append(ex)

@@ -12,12 +12,34 @@ from . import _lib
 
 
 class FittedShape:
-    """Abstract base (fitting.jl:8): user shapes subclass this and plug into the host loop."""
+    """Abstract base (fitting.jl:8): user shapes subclass this and plug into the host loop.
+
+    A user shape may also run its scoring and refit on the device.  It then defines three members:
+    `cuda_source` (class attribute: CUDA C defining `rsc_user_compatible`, include/rsc.h), `device_record(self)`
+    -> (p, outwards) with at most 7 floats, and the staticmethod `device_constants(params)` -> at most 8 floats
+    (thresholds such as eps and cos(alpha), computed on the host).  Its `fit` stays on the host."""
 
     kind = -1
+    cuda_source = None
 
     def to_cand(self) -> _lib.rsc_cand:  # pragma: no cover - abstract
         raise NotImplementedError
+
+
+def on_device(shape_class) -> bool:
+    """True for a user-defined shape class that brings device source (`cuda_source`)."""
+    return shape_class not in SHAPE_KIND and getattr(shape_class, "cuda_source", None) is not None
+
+
+def user_cand(s: FittedShape, type_id: int) -> _lib.rsc_cand:
+    """The rsc_cand of a device-capable user shape: its `device_record` under the compiled type id."""
+    p, outwards = s.device_record()
+    p = [float(v) for v in p]
+    if len(p) > 7:
+        raise ValueError(f"{type(s).__name__}.device_record: at most 7 parameters, got {len(p)}")
+    c = _lib.rsc_cand(type=int(type_id), outwards=int(bool(outwards)))
+    c.p[:] = p + [0.0] * (7 - len(p))
+    return c
 
 
 def _v3(x):
