@@ -355,7 +355,8 @@ void rsc_run_destroy(rsc_run* run);
  * coordinates and normal widened to double.  The library gates every point on its enabled bit itself.
  * libnvrtc.so.12 (dlopen-ed on first use) compiles the source with the library's kernel template for sm_100a,
  * --fmad=false and no fast-math: float64 + - * / sqrt round to nearest, so a host restatement in the same
- * operation order makes the same decisions (DESIGN.md section 8).  Fitting stays with the caller.  Not for
+ * operation order makes the same decisions (DESIGN.md section 8).  Fitting stays with the caller unless the
+ * source also defines rsc_user_fit (below).  Not for
  * sharded or ranged clouds (RSC_E_STATE).  The source is passed as bytes + length. */
 #define RSC_USER_TYPE0 16
 /* compile only, no device needed: RSC_OK or RSC_E_ARG (RSC_E_STATE: NVRTC cannot be loaded); NVRTC's log
@@ -373,6 +374,38 @@ int32_t rsc_user_score(rsc_cloud* cloud, const double* k, int32_t nk, const rsc_
  * the uploaded subsets) */
 int32_t rsc_user_refit_extract(rsc_cloud* cloud, const double* k, int32_t nk, const rsc_cand* cand,
                                int64_t* out_idx, int64_t* out_n, int32_t disable);
+
+/* ---- user shapes inside the sampler and the device loop ------------------------------------------
+ * A user source that also defines
+ *   __device__ bool rsc_user_fit(int np, const double P[8][3], const double N[8][3], const double k[8],
+ *                                double p[7], int* outwards);
+ * fits on the device: np = drawN (3..8), P / N the minimal set's points and normals in draw order (float32
+ * widened to double), k the type's constants.  It returns true when the set yields a candidate, whose record
+ * is then (type id, *outwards, p); p and *outwards are zeroed before the call.  At most one candidate per
+ * (set, type), like every built-in fit.  Sources without rsc_user_fit compile as before and cannot be used
+ * in a fit order.  The library looks for the token `rsc_user_fit` anywhere in the source, comments included:
+ * a scoring-only source must not mention it, or its compile fails for want of the definition. */
+#define RSC_MAX_ORDER 8 /* positions of a fit order: the 4 built-ins plus up to 4 user types */
+/* one entry of the fit order: a built-in kind (RSC_PLANE..RSC_CONE; k ignored, eps/alpha from rsc_params) or a
+ * compiled user type id (>= RSC_USER_TYPE0) with its nk <= 8 constants.  The calls below take the order as
+ * `const void* order` pointing at rsc_shape_slot[norder] (an rsc_shape_slot array converts implicitly). */
+typedef struct rsc_shape_slot {
+  int32_t type;
+  int32_t nk;
+  double k[8];
+} rsc_shape_slot; /* 72 bytes */
+/* rsc_sample_fit with a mixed fit order (replaces params->shape_types): the same Philox sets, candidates
+ * merged in (set, position in order) order.  norder = 0 only draws (out_idx).  Each type at most once,
+ * norder <= 8, every user type compiled on the cloud's context with a fit (else RSC_E_ARG). */
+int32_t rsc_sample_fit_user(rsc_cloud* cloud, const rsc_params* params, const void* order, int32_t norder,
+                            uint64_t seed, uint64_t set0, int32_t S, rsc_cand* out, int32_t* out_set,
+                            int64_t* out_idx, int32_t* out_n);
+/* rsc_ransac_run with a mixed fit order: the device loop scores, refits and invalidates user candidates with
+ * their compiled kernels.  Built-ins only: exactly rsc_ransac_run with that shape_types.  RSC_E_STATE on
+ * sharded or ranged clouds, with RSC_SAMPLER_OCTREE / RSC_SCORE_PROGRESSIVE / RSC_REFIT_LSQ /
+ * RSC_EXTRACT_BITMAP, and with RSC_LOOP_HOSTWALK set. */
+int32_t rsc_ransac_run_user(rsc_cloud* cloud, const rsc_params* params, const void* order, int32_t norder,
+                            uint64_t seed, rsc_run** out);
 
 #ifdef __cplusplus
 }

@@ -57,6 +57,14 @@ struct RscParams          # 160 bytes
     lw_period::UInt32         # RSC_SAMPLER_OCTREE: refresh period of the level weights (0/1 = every iteration)
 end
 
+struct RscShapeSlot        # 72 bytes: one position of a fit order (a built-in kind or a compiled user type id)
+    type::Int32
+    nk::Int32
+    k::NTuple{8,Float64}
+end
+RscShapeSlot(type::Integer, k::Vector{Float64}=Float64[]) =
+    RscShapeSlot(Int32(type), Int32(length(k)), ntuple(i -> i <= length(k) ? k[i] : 0.0, 8))
+
 const KIND = Dict{Any,Int32}(FittedPlane => 0, FittedSphere => 1, FittedCylinder => 2, FittedCone => 3)
 const S_SYM = Dict(:lengthC => Int32(0), :allcand => Int32(1), :nofminset => Int32(2))
 
@@ -77,7 +85,7 @@ end
 "Flatten the nested NamedTuple of `ransacparameters` (utilities.jl:332-433) into the C POD."
 function toparams(params)
     it = params.iteration
-    types = Int32[KIND[t] for t in it.shape_types]
+    types = Int32[KIND[t] for t in it.shape_types if haskey(KIND, t)]   # (user types travel in a fit order)
     st = ntuple(i -> i <= length(types) ? types[i] : Int32(0), 4)
     g(name, f, d) = haskey(params, name) ? Float64(getfield(getfield(params, name), f)) : d
     eps = (g(:plane, :ϵ, 0.3), g(:sphere, :ϵ, 0.3), g(:cylinder, :ϵ, 0.3), g(:cone, :ϵ, 0.3))
@@ -319,6 +327,59 @@ function user_refit_extract(dc::DeviceCloud, rec::RscCand, k::Vector{Float64}; d
     resize!(out, n[])
     disable && pull_enabled!(dc)
     out .+ 1
+end
+
+"""
+    sample_fit_user(dc, params, order, seed, set0, S) -> (records, sets, idx)
+
+`samplepointcloud4!` + `forcefitshapes!` for a fit order of built-in kinds and compiled user types that define
+`rsc_user_fit` (`order::Vector{RscShapeSlot}`, at most 8, each type once): the sets `rsc_sample_fit` draws, the
+candidates as `RscCand` records in (set, position in the order) order, their 1-based sets, and the drawn indices
+(drawN x S, 1-based; a column starting with 0 is a failed sample).  An empty order only draws: the sampler of a
+Julia plug-in host loop whose shapes still fit in Julia.
+"""
+function sample_fit_user(dc::DeviceCloud, params, order::Vector{RscShapeSlot}, seed::Integer, set0::Integer, S::Integer)
+    prm = Ref(toparams(params))
+    cap = max(S * length(order), 1)
+    out = Vector{RscCand}(undef, cap)
+    out_set = Vector{Int32}(undef, cap)
+    idx = Matrix{Int64}(undef, prm[].drawN, S)
+    n = Ref{Int32}(0)
+    check(ccall(fn(:rsc_sample_fit_user), Int32,
+                (Ptr{Cvoid}, Ref{RscParams}, Ptr{Cvoid}, Int32, UInt64, UInt64, Int32, Ptr{RscCand}, Ptr{Int32}, Ptr{Int64}, Ref{Int32}),
+                dc.h, prm, order, length(order), seed, set0, S, out, out_set, idx, n))
+    out[1:n[]], out_set[1:n[]] .+ 1, idx .+ 1
+end
+
+"""
+    ransac_user(dc, params, order; seed=1234) -> (records, inlier lists, seconds)
+
+The whole device loop (`rsc_ransac_run_user`) for a fit order of built-in kinds and user types with
+`rsc_user_fit`: the extracted shapes as `RscCand` records (user records under their type ids, for the caller to
+turn back into its own types) and their 1-based inlier lists.  No extension switch; not for sharded or ranged
+clouds.
+"""
+function ransac_user(dc::DeviceCloud, params, order::Vector{RscShapeSlot}; seed::Integer=1234)
+    prm = Ref(toparams(params))
+    run = Ref{Ptr{Cvoid}}(C_NULL)
+    check(ccall(fn(:rsc_ransac_run_user), Int32, (Ptr{Cvoid}, Ref{RscParams}, Ptr{Cvoid}, Int32, UInt64, Ref{Ptr{Cvoid}}),
+                dc.h, prm, order, length(order), seed, run))
+    recs = RscCand[]; lists = Vector{Int}[]
+    try
+        for i in 0:ccall(fn(:rsc_run_nshapes), Int32, (Ptr{Cvoid},), run[])-1
+            c = Ref{RscCand}()
+            n = Ref{Int64}(0)
+            check(ccall(fn(:rsc_run_shape), Int32, (Ptr{Cvoid}, Int32, Ref{RscCand}, Ref{Int64}), run[], i, c, n))
+            idx = Vector{Int64}(undef, n[])
+            n[] > 0 && check(ccall(fn(:rsc_run_inpoints), Int32, (Ptr{Cvoid}, Int32, Ptr{Int64}), run[], i, idx))
+            push!(recs, c[]); push!(lists, idx .+ 1)
+        end
+        secs = ccall(fn(:rsc_run_seconds), Float64, (Ptr{Cvoid},), run[])
+        pull_enabled!(dc)
+        return recs, lists, secs
+    finally
+        ccall(fn(:rsc_run_destroy), Cvoid, (Ptr{Cvoid},), run[])
+    end
 end
 
 # ---- one process per GPU: sharded storage (include/rsc.h "point-range sharding") ---------------------

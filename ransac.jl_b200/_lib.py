@@ -26,6 +26,15 @@ class rsc_cand(C.Structure):
     _fields_ = [("type", C.c_int32), ("outwards", C.c_int32), ("p", C.c_double * 7)]
 
 
+class rsc_shape_slot(C.Structure):
+    """one position of a fit order (rsc_sample_fit_user, rsc_ransac_run_user): a built-in kind or a user type id"""
+
+    _fields_ = [("type", C.c_int32), ("nk", C.c_int32), ("k", C.c_double * 8)]
+
+
+RSC_MAX_ORDER = 8
+
+
 class rsc_params(C.Structure):
     _fields_ = [
         ("drawN", C.c_int32),
@@ -131,6 +140,9 @@ SIGNATURES = {
     "rsc_user_shape_compile": (C.c_int32, [_P, _P, C.c_int64, C.POINTER(C.c_int32)]),
     "rsc_user_score": (C.c_int32, [_P, _P, C.c_int32, _P, C.c_int32, C.c_int32, _P, _P]),
     "rsc_user_refit_extract": (C.c_int32, [_P, _P, C.c_int32, C.POINTER(rsc_cand), _P, C.POINTER(C.c_int64), C.c_int32]),
+    "rsc_sample_fit_user": (C.c_int32, [_P, C.POINTER(rsc_params), _P, C.c_int32, C.c_uint64, C.c_uint64, C.c_int32, _P, _P, _P,
+                                        C.POINTER(C.c_int32)]),
+    "rsc_ransac_run_user": (C.c_int32, [_P, C.POINTER(rsc_params), _P, C.c_int32, C.c_uint64, C.POINTER(_P)]),
 }
 
 if not os.path.exists(LIB_PATH):

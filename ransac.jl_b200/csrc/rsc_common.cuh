@@ -284,9 +284,32 @@ struct FitScratch {
   int32_t* level;  // per set: octree level its cell came from (cell sampler only)
   float* gath;     // sharded storage: [S][k][6] coordinates + normals of the drawn points, gathered from their owners
 };
+// a validated fit order of built-in kinds and compiled user types (rsc_shape_slot[], make_fit_order in rsc_user.cu)
+struct FitOrder {
+  int n = 0;
+  bool has_user = false;
+  int32_t type[RSC_MAX_ORDER];
+  int32_t nk[RSC_MAX_ORDER];
+  double k[RSC_MAX_ORDER][8];
+};
+// order: nullptr = params->shape_types (built-ins); else the mixed order, whose user positions are fitted by their
+// compiled rsc_user_fit_kernel into the same dense slots / ballot words
 int32_t fit_enqueue(rsc_ctx* ctx, rsc_cloud* cloud, int mode, const rsc_params* params, int k, const double* dP,
                     const double* dN, const int64_t* d_idx, int S, uint64_t seed, uint64_t set0, cudaStream_t st,
-                    FitScratch* fs, const double* cum = nullptr, int32_t* d_seg = nullptr, int sets_per_iter = 0, int nb = 0);
+                    FitScratch* fs, const double* cum = nullptr, int32_t* d_seg = nullptr, int sets_per_iter = 0, int nb = 0,
+                    const FitOrder* order = nullptr);
+// user shapes of a fit order (rsc_user.cu).  RSC_E_ARG (reason in rsc_last_error) for a duplicate or unknown type,
+// a user type without a compiled fit, norder outside 0..RSC_MAX_ORDER or nk outside 0..8
+int32_t make_fit_order(rsc_ctx* ctx, const rsc_shape_slot* order, int32_t norder, FitOrder* fo, const char* who);
+// K1: the fit kernel of user position `pos` over the S sets of `idx` (cloud coordinates)
+int32_t user_fit_enqueue(rsc_ctx* ctx, const FitOrder& fo, int pos, const rsc_cloud* cloud, const int64_t* idx, int S, int np,
+                         rsc_cand* dense, uint32_t* okmask, cudaStream_t st);
+// K2 / K5: for every user type of the order, ADD the counts of its records among d_cands[0..min(*d_count, c_cap))
+// (d_count nullable: c_cap candidates) on `ps` to ce (and cv, nullable); other records are left as they are
+int32_t user_score_enqueue(rsc_ctx* ctx, const FitOrder& fo, const PointSet& ps, const rsc_cand* d_cands, int c_cap,
+                           const unsigned long long* d_count, int32_t* cv, int32_t* ce, cudaStream_t st);
+// K4 for a user candidate: the inlier-mask words + their count / scan (what refit_mask_enqueue does for a built-in)
+int32_t user_refit_mask_enqueue(rsc_cloud* cloud, const FitOrder& fo, const rsc_cand& cand, cudaStream_t st);
 int64_t count_mask_bits(rsc_ctx* ctx, const uint32_t* words, int64_t nwords);
 // device -> (pageable) host through page-locked staging and worker threads; synchronises `st`
 int32_t staged_d2h(rsc_ctx* ctx, void* h_dst, const void* d_src, size_t bytes, cudaStream_t st);
@@ -299,9 +322,10 @@ int32_t shard_clear_enabled(rsc_cloud* cloud, const uint32_t* inl_local, const i
                             int32_t* d_extra_out, cudaStream_t st);
 // the two loops behind rsc_ransac_run (rsc_loop.cu: reference behaviour, decisions on the device;
 // rsc_run.cu: the extension switches, host-walked)
-int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed, rsc_run* run);
+// order (nullable): a mixed fit order in place of p->shape_types (rsc_ransac_run_user)
+int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed, rsc_run* run, const FitOrder* order = nullptr);
 void loop_scratch_free(rsc_ctx* ctx);
-int32_t fit_reserve(rsc_ctx* ctx, const rsc_params* params, int S);
+int32_t fit_reserve(rsc_ctx* ctx, const rsc_params* params, int S, int ntypes = -1);
 // exclusive scan of n uint32 counts into 64-bit offsets (+ total) on `st` (rsc_fit.cu)
 int32_t scan_u32(rsc_ctx* ctx, const uint32_t* counts, int n, unsigned long long* offsets, unsigned long long* total,
                  cudaStream_t st);

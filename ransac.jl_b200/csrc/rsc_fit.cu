@@ -41,7 +41,7 @@ struct FitParams {
   double eps[RSC_NTYPES], cosa[RSC_NTYPES];
   double cos_par;  // cosd(parallelthrdeg)
   double sphere_par, minconeopang, collin;
-  int32_t ntypes, types[RSC_NTYPES];
+  int32_t ntypes, types[RSC_MAX_ORDER];  // the fit order; user types (>= RSC_USER_TYPE0) are fitted by their own kernel
   int32_t k;
 };
 
@@ -556,6 +556,7 @@ __global__ void __launch_bounds__(128) fit_kernel(GatherSrc src, const int64_t* 
   const int fk = KK ? KK : f.k;
   const int s = blockIdx.x * blockDim.x + threadIdx.x;
   const int t = blockIdx.y;
+  if (f.types[t] >= RSC_NTYPES) return;  // a user position (block-uniform): its own fit kernel writes slot and ballot
   const size_t slot = (size_t)s * f.ntypes + t;
   bool ok = false;
   // (a set the sampler could not draw has idx < 0: no candidate)
@@ -659,7 +660,7 @@ __global__ void __launch_bounds__(1024) group_scan_kernel(const uint32_t* __rest
 __global__ void __launch_bounds__(128) compact_kernel(const rsc_cand* __restrict__ dense, const uint32_t* __restrict__ okmask,
                                                       const uint32_t* __restrict__ base, int ntypes, rsc_cand* __restrict__ out,
                                                       int32_t* __restrict__ out_set) {
-  __shared__ uint32_t m[4 * RSC_NTYPES];  // [type][warp]
+  __shared__ uint32_t m[4 * RSC_MAX_ORDER];  // [type][warp]
   const int t = blockIdx.y, lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   if (threadIdx.x < 4 * ntypes) m[threadIdx.x] = okmask[(size_t)blockIdx.x * 4 * ntypes + threadIdx.x];
   __syncthreads();
@@ -915,20 +916,29 @@ int32_t scan_u32(rsc_ctx* ctx, const uint32_t* counts, int n, unsigned long long
 // Enqueue fit (+ sampling) for S sets; leaves compacted candidates in ctx->fitbuf (FitScratch.out),
 // their count in FitScratch.total.  No synchronisation.
 // size the scratch for batches of up to S sets once (the device loop grows its batches while it runs)
-int32_t fit_reserve(rsc_ctx* ctx, const rsc_params* params, int S) {
+int32_t fit_reserve(rsc_ctx* ctx, const rsc_params* params, int S, int ntypes) {
   FitScratch fs;
-  return carve(ctx, S, params->n_shape_types, params->drawN, &fs);
+  return carve(ctx, S, ntypes >= 0 ? ntypes : params->n_shape_types, params->drawN, &fs);
 }
 
 // mode 0: explicit coordinates, 1: explicit indices, 2: root-cell sampler (the reference's behaviour,
 // Q1), 3: level-weighted cell sampler on the flattened octree (`cum` = cumulative level weights)
 int32_t fit_enqueue(rsc_ctx* ctx, rsc_cloud* cloud, int mode, const rsc_params* params, int k, const double* dP,
                     const double* dN, const int64_t* d_idx, int S, uint64_t seed, uint64_t set0, cudaStream_t st,
-                    FitScratch* fs, const double* cum, int32_t* d_seg, int sets_per_iter, int nb) {
+                    FitScratch* fs, const double* cum, int32_t* d_seg, int sets_per_iter, int nb, const FitOrder* order) {
   if (d_seg && (sets_per_iter <= 0 || sets_per_iter % 128 || nb < 0 || nb >= 1024)) return fail(ctx, RSC_E_ARG, "fit: segment bounds need sets_per_iter % 128 == 0");
   FitParams f;
-  int32_t rc = make_fit_params(ctx, params, k, &f);
-  if (rc) return rc;
+  int32_t rc;
+  if (order) {  // a mixed order replaces params->shape_types
+    rsc_params pb = *params;
+    pb.n_shape_types = 0;
+    if ((rc = make_fit_params(ctx, &pb, k, &f))) return rc;
+    if (order->has_user && (mode != 2 || !cloud || cloud->is_shard())) return fail(ctx, RSC_E_STATE, "fit: user shapes fit on the root-cell sampler of a whole cloud only");
+    f.ntypes = order->n;
+    for (int t = 0; t < order->n; ++t) f.types[t] = order->type[t];
+  } else if ((rc = make_fit_params(ctx, params, k, &f))) {
+    return rc;
+  }
   if ((rc = carve(ctx, S, f.ntypes, k, fs))) return rc;
   const int slots = S * f.ntypes;
   GatherSrc src{nullptr, 0, dP, dN, nullptr};
@@ -943,7 +953,7 @@ int32_t fit_enqueue(rsc_ctx* ctx, rsc_cloud* cloud, int mode, const rsc_params* 
   if (mode == 2 && (rc = build_select_index(cloud, st, &boff, &nblk, &nen))) return rc;
   CellsView cv;
   if (mode == 3 && (rc = build_cells_index(cloud, st, cum, &cv))) return rc;
-  if (slots > 0) {
+  if (slots > 0 || (order && S > 0)) {  // (an empty order only draws)
     const int64_t* use_idx = d_idx;
     if (mode == 3) {
       sample_cells_kernel<<<(S + 127) / 128, 128, 0, st>>>(S, k, seed, set0, cloud->n, cloud->enabled, cloud->n_pad / 32, cv,
@@ -969,11 +979,20 @@ int32_t fit_enqueue(rsc_ctx* ctx, rsc_cloud* cloud, int mode, const rsc_params* 
       RSC_CUDA(ctx, cudaGetLastError());
       use_idx = fs->idx;
     }
+    if (slots == 0) {
+      RSC_CUDA(ctx, cudaMemsetAsync(fs->total, 0, 8, st));
+      ctx->stats.sets_drawn += S;
+      return RSC_OK;
+    }
     if (k == 3)
       fit_kernel<3><<<dim3((S + 127) / 128, f.ntypes), 128, 0, st>>>(src, use_idx, S, f, fs->dense, fs->okmask);
     else
       fit_kernel<0><<<dim3((S + 127) / 128, f.ntypes), 128, 0, st>>>(src, use_idx, S, f, fs->dense, fs->okmask);
     RSC_CUDA(ctx, cudaGetLastError());
+    if (order)
+      for (int t = 0; t < order->n; ++t)
+        if (order->type[t] >= RSC_NTYPES && (rc = user_fit_enqueue(ctx, *order, t, cloud, use_idx, S, k, fs->dense, fs->okmask, st)))
+          return rc;
     group_scan_kernel<<<1, 1024, 0, st>>>(fs->okmask, (S + 127) / 128, f.ntypes, fs->base, fs->total, d_seg, sets_per_iter, nb);
     RSC_CUDA(ctx, cudaGetLastError());
     compact_kernel<<<dim3((S + 127) / 128, f.ntypes), 128, 0, st>>>(fs->dense, fs->okmask, fs->base, f.ntypes, fs->out, fs->out_set);
@@ -1065,6 +1084,31 @@ int32_t rsc_sample_fit(rsc_cloud* cloud, const rsc_params* params, uint64_t seed
   FitScratch fs;
   int32_t rc = fit_enqueue(ctx, cloud, 2, params, k, nullptr, nullptr, nullptr, S, seed, set0, st, &fs);
   if (rc) return rc;
+  return fit_finish(ctx, fs, S, k, st, out, out_set, out_idx, out_n);
+}
+
+int32_t rsc_sample_fit_user(rsc_cloud* cloud, const rsc_params* params, const void* order, int32_t norder,
+                            uint64_t seed, uint64_t set0, int32_t S, rsc_cand* out, int32_t* out_set, int64_t* out_idx,
+                            int32_t* out_n) {
+  if (!cloud) return RSC_E_ARG;
+  rsc_ctx* ctx = cloud->ctx;
+  if (!params || !out_n || S < 0 || (S > 0 && norder > 0 && !out) || (norder > 0 && !order))
+    return fail(ctx, RSC_E_ARG, "sample_fit_user: null arguments");
+  *out_n = 0;
+  FitOrder fo;
+  int32_t rc = make_fit_order(ctx, static_cast<const rsc_shape_slot*>(order), norder, &fo, "sample_fit_user");
+  if (rc) return rc;
+  if (fo.has_user && (cloud->is_shard() || cloud->range_set))
+    return fail(ctx, RSC_E_STATE, "sample_fit_user: sharded or ranged clouds are not supported");
+  if (S == 0) return RSC_OK;
+  const int k = params->drawN;
+  if (k < 3 || k > kMaxK) return fail(ctx, RSC_E_ARG, "sample_fit_user: drawN must be 3..8");
+  RSC_CUDA(ctx, cudaSetDevice(ctx->device));
+  if (int32_t rcr = cloud_ready(cloud)) return rcr;
+  cudaStream_t st = ctx->stream;
+  FitScratch fs;
+  if ((rc = fit_enqueue(ctx, cloud, 2, params, k, nullptr, nullptr, nullptr, S, seed, set0, st, &fs, nullptr, nullptr, 0, 0, &fo)))
+    return rc;
   return fit_finish(ctx, fs, S, k, st, out, out_set, out_idx, out_n);
 }
 

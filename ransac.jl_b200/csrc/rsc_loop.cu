@@ -172,7 +172,7 @@ __global__ void finish_new_dev_kernel(const rsc_cand* __restrict__ cands, const 
   const int n = (int)min(*total, (unsigned long long)cap);
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     const int t = cands[i].type;
-    const bool honour = (honour_enabled >> t) & 1u;
+    const bool honour = t >= RSC_NTYPES || ((honour_enabled >> t) & 1u);  // user shapes honour the enabled mask
     score[i] = honour ? ce[i] : cv[i];
     flags[i] = (uint8_t)(1u | ((!honour && cv[i] != ce[i]) ? 2u : 0u));
   }
@@ -225,7 +225,7 @@ __global__ void k5_pack_kernel(LoopDev* __restrict__ d, const unsigned long long
   out->tot_global = d->tot_global[0];
 }
 
-int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed, rsc_run* run) {
+int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed, rsc_run* run, const FitOrder* order) {
   rsc_ctx* ctx = cloud->ctx;
   cudaStream_t st = ctx->stream;
   if (!ctx->loop_scratch) ctx->loop_scratch = new LoopScratch();
@@ -248,7 +248,11 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
   const int64_t N = cloud->n_global > 0 ? cloud->n_global : cloud->n;
   const int64_t M = sub.m_global > 0 ? sub.m_global : sub.m;
   const int S = p->minsubsetN;
-  const int maxnew = S * p->n_shape_types;
+  const int ntypes = order ? order->n : p->n_shape_types;
+  const int maxnew = S * ntypes;
+  // user shapes (rsc_ransac_run_user): their fit, score and mask kernels join K1, K2, K4 and K5; such runs never take
+  // the culled scorer, which knows the built-in types only
+  const FitOrder* uo = order && order->has_user ? order : nullptr;
   // this rank's slice of the subset copy: all of it (single GPU, or a shard's local entries) or, on
   // replicated storage, the same fraction of it as the rank's range of the cloud
   PointSet sps = view_subset(&sub);
@@ -329,7 +333,7 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
   RUN_CUDA(cudaMalloc(&run->d_idx, (size_t)(n_enabled_local > 0 ? n_enabled_local : 1) * sizeof(int64_t)));  // a point is extracted at most once
 
   RUN_CUDA(ls.newcnt.ensure((size_t)2 * maxnew * Bmax * 4 + 64));
-  if ((rc = fit_reserve(ctx, p, S * Bmax))) return rc;
+  if ((rc = fit_reserve(ctx, p, S * Bmax, ntypes))) return rc;
   RUN_CUDA(store.reserve((size_t)std::min<int64_t>((int64_t)maxnew * Bmax, 1 << 20), st));
   DecideParams q;
   q.N = N, q.M = M, q.tau = p->tau, q.prob_det = p->prob_det;
@@ -346,7 +350,7 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
     // (segment bounds of the batch's iterations: from the compaction itself when an iteration is whole groups of sets)
     const bool seg_fused = S % 128 == 0;
     if ((rc = fit_enqueue(ctx, cloud, 2, p, p->drawN, nullptr, nullptr, nullptr, S * nb, seed, (uint64_t)(k - 1) * S, st, &fs, nullptr,
-                          seg_fused ? dev->seg : nullptr, S, nb)))
+                          seg_fused ? dev->seg : nullptr, S, nb, order)))
       return rc;
     if (!seg_fused) {
       seg_bounds_kernel<<<1, 96, 0, st>>>(fs.out_set, fs.total, S, nb, dev->seg);
@@ -374,6 +378,7 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
       append_new_kernel<<<std::max(1, std::min(cap_new * 4 / 256, 64)), 256, 0, st>>>(fs.out, fs.total, cap_new, dst);
       RUN_CUDA(cudaGetLastError());
       if ((rc = score_small_enqueue(ctx, cloud, sps, th, dst, cap_new, fs.total, cv, ce, st))) return rc;
+      if (uo && (rc = user_score_enqueue(ctx, *uo, sps, dst, cap_new, fs.total, cv, ce, st))) return rc;
       if (coll && ctx->allreduce(ctx->allreduce_user, cv, (int64_t)2 * cap_new, (void*)st))
         return fail(ctx, RSC_E_NCCL, "ransac_run: all-reduce of the counts failed");
       finish_new_dev_kernel<<<std::max(1, std::min(cap_new / 256, 64)), 256, 0, st>>>(
@@ -417,7 +422,8 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
         int32_t* ce = cv + n_new;
         // (the culled scorer on the subset's Morton view when the batch is large: same counts)
         // the overflow flag rides behind the counts, so that a sharded run decides to repeat collectively
-        if ((rc = loop_score_new(ctx, cloud, sub, sps, !ranged, th, dst, n_new, cv, ce, cv + 2 * n_new, st))) return rc;
+        if ((rc = loop_score_new(ctx, cloud, sub, sps, !ranged && !uo, th, dst, n_new, cv, ce, cv + 2 * n_new, st))) return rc;
+        if (uo && (rc = user_score_enqueue(ctx, *uo, sps, dst, n_new, nullptr, cv, ce, st))) return rc;
         if (coll && ctx->allreduce(ctx->allreduce_user, cv, (int64_t)2 * n_new + 1, (void*)st))
           return fail(ctx, RSC_E_NCCL, "ransac_run: all-reduce of the counts failed");
         finish_new_kernel<<<(n_new + 255) / 256, 256, 0, st>>>(dst, n_new, cv, ce, th.honour_enabled,
@@ -461,7 +467,11 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
       const int64_t swords = sub.m_pad / 32;
       RUN_CUDA(ls.olden.ensure((size_t)swords * 4));
       RUN_CUDA(cudaMemcpyAsync(ls.olden.p, sub.enabled, (size_t)swords * 4, cudaMemcpyDeviceToDevice, st));
-      if ((rc = refit_mask_enqueue(cloud, thr, shape, st))) return rc;
+      if (shape.type >= RSC_USER_TYPE0) {
+        if ((rc = user_refit_mask_enqueue(cloud, *uo, shape, st))) return rc;
+      } else if ((rc = refit_mask_enqueue(cloud, thr, shape, st))) {
+        return rc;
+      }
       if (p->compat_flags & RSC_EXTRACT_BITMAP) {  // extension: only the largest connected component in parameter space
         unsigned long long tot = 0;
         RUN_CUDA(cudaMemcpyAsync(&tot, ctx->misc2.p, 8, cudaMemcpyDeviceToHost, st));
@@ -554,6 +564,9 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
           queue_overflow_kernel<<<1, 1, 0, st>>>(ctx->wl_count.as<uint32_t>(), (uint32_t)ctx->wl_cap, hit + nst);
           RUN_CUDA(cudaGetLastError());
         }
+        // user records: the built-in scorers left their hits at 0 (enabled-gated counts, so the scratch bound holds)
+        if (uo && (rc = user_score_enqueue(ctx, *uo, dps, store.cands[store.cur].as<rsc_cand>(), nst, nullptr, nullptr, hit, st)))
+          return rc;
         if (coll && ctx->allreduce(ctx->allreduce_user, hit, (int64_t)nst + 2, (void*)st))
           return fail(ctx, RSC_E_NCCL, "ransac_run: all-reduce of the K5 hits failed");
         invalidate_kernel<<<(nst + 255) / 256, 256, 0, st>>>(hit, store.flags[store.cur].as<uint8_t>(), nst, rec.best_idx, keep);

@@ -16,7 +16,7 @@ static __global__ void finish_new_kernel(const rsc_cand* __restrict__ cands, int
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const int t = cands[i].type;
-  const bool honour = (honour_enabled >> t) & 1u;
+  const bool honour = t >= RSC_NTYPES || ((honour_enabled >> t) & 1u);  // user shapes honour the enabled mask
   score[i] = honour ? ce[i] : cv[i];
   flags[i] = (uint8_t)(1u | ((!honour && cv[i] != ce[i]) ? 2u : 0u));  // bit0 alive, bit1 tainted
 }

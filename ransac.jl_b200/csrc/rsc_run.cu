@@ -159,6 +159,41 @@ int32_t rsc_cloud_set_range(rsc_cloud* cloud, int64_t lo, int64_t hi) {
   return RSC_OK;
 }
 
+int32_t rsc_ransac_run_user(rsc_cloud* cloud, const rsc_params* p, const void* order, int32_t norder, uint64_t seed,
+                            rsc_run** out) {
+  if (!cloud || !out) return RSC_E_ARG;
+  rsc_ctx* ctx = cloud->ctx;
+  *out = nullptr;
+  if (!p) return fail(ctx, RSC_E_ARG, "ransac_run_user: params is null");
+  FitOrder fo;
+  if (int32_t rc = make_fit_order(ctx, static_cast<const rsc_shape_slot*>(order), norder, &fo, "ransac_run_user")) return rc;
+  if (norder < 1) return fail(ctx, RSC_E_ARG, "ransac_run_user: an empty fit order");
+  if (p->drawN < 3 || p->drawN > 8) return fail(ctx, RSC_E_ARG, "ransac_run_user: drawN must be 3..8");
+  if (p->minsubsetN < 1) return fail(ctx, RSC_E_ARG, "ransac_run_user: nothing to sample/fit");
+  if (p->extract_s < 0 || p->extract_s > 2 || p->terminate_s < 0 || p->terminate_s > 2)
+    return fail(ctx, RSC_E_ARG, "ransac_run_user: extract_s/terminate_s must be RSC_S_*");
+  if (cloud->is_shard() || cloud->range_set) return fail(ctx, RSC_E_STATE, "ransac_run_user: sharded or ranged clouds are not supported");
+  if (p->compat_flags & (RSC_SAMPLER_OCTREE | RSC_SCORE_PROGRESSIVE | RSC_REFIT_LSQ | RSC_EXTRACT_BITMAP))
+    return fail(ctx, RSC_E_STATE, "ransac_run_user: the extension switches are not available with a fit order");
+  if (getenv("RSC_LOOP_HOSTWALK")) return fail(ctx, RSC_E_STATE, "ransac_run_user: runs the device loop only (RSC_LOOP_HOSTWALK is set)");
+  if (cloud->subsets.empty() || !cloud->subsets[0].soa)
+    return fail(ctx, RSC_E_STATE, "ransac_run_user: subset 1 is not uploaded (rsc_cloud_set_subset(cloud, 0, ...))");
+  RSC_CUDA(ctx, cudaSetDevice(ctx->device));
+  if (int32_t rcr = cloud_ready(cloud)) return rcr;
+  const auto t0 = std::chrono::steady_clock::now();
+  rsc_run* run = new rsc_run();
+  run->ctx = ctx;
+  const int32_t rcd = ransac_loop_device(cloud, p, seed, run, &fo);
+  cudaStreamSynchronize(ctx->stream);
+  if (rcd) {
+    delete run;
+    return rcd;
+  }
+  run->seconds = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+  *out = run;
+  return RSC_OK;
+}
+
 int32_t rsc_ransac_run(rsc_cloud* cloud, const rsc_params* p, uint64_t seed, rsc_run** out) {
   if (!cloud || !out) return RSC_E_ARG;
   rsc_ctx* ctx = cloud->ctx;

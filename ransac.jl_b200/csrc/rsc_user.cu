@@ -10,7 +10,9 @@
 //   rsc_user_score          rsc_user_score_kernel: counts (+ masks) over a subset copy or the whole cloud
 //   rsc_user_refit_extract  rsc_user_mask_kernel writes K4's inlier-mask words; the count, scan and compaction of
 //                           rsc_extract.cu follow (ascending lists, cleared enabled bits, refreshed subset copies)
-// Fitting stays on the host.  Sharded and ranged clouds are out of scope (RSC_E_STATE).
+// A source that also defines rsc_user_fit gets rsc_user_fit_kernel (K1 of the sampler and of the device loop,
+// rsc_fit.cu); the device loop (rsc_loop.cu) scores its mixed batches with rsc_user_score_kernel too.
+// Sharded and ranged clouds are out of scope (RSC_E_STATE).
 #include <dlfcn.h>
 #include <nvrtc.h>
 #include <string.h>
@@ -73,9 +75,12 @@ static NvrtcApi* nvrtc_api() {
 
 // Compiles template + user source to a CUBIN.  Returns RSC_OK, RSC_E_ARG (the source does not compile, or defines
 // no rsc_user_compatible) or RSC_E_STATE (NVRTC not available); *log receives NVRTC's log in every case.
-static int32_t user_compile(const char* src, size_t nbytes, std::string* cubin, std::string* log) {
+// *has_fit (nullable): the source defines rsc_user_fit, and the program holds rsc_user_fit_kernel.
+static int32_t user_compile(const char* src, size_t nbytes, std::string* cubin, std::string* log, bool* has_fit = nullptr) {
   log->clear();
   const std::string user(src, nbytes);
+  const bool fit = user.find("rsc_user_fit") != std::string::npos;
+  if (has_fit) *has_fit = fit;
   if (user.find("rsc_user_compatible") == std::string::npos) {
     *log = "user shape source defines no rsc_user_compatible(const double p[7], int outwards, const double k[8], double x, "
            "double y, double z, double nx, double ny, double nz)";
@@ -95,8 +100,9 @@ static int32_t user_compile(const char* src, size_t nbytes, std::string* cubin, 
     return RSC_E_ARG;
   }
   // IEEE float64 + - * / sqrt, no contraction: a host restatement in the same operation order decides alike
-  const char* opts[] = {"--gpu-architecture=sm_100a", "--fmad=false", "--std=c++17", "--ptxas-options=-v"};
-  r = a->CompileProgram(p, (int)(sizeof(opts) / sizeof(opts[0])), opts);
+  const char* opts[] = {"--gpu-architecture=sm_100a", "--fmad=false", "--std=c++17", "--ptxas-options=-v", "-DRSC_USER_HAS_FIT"};
+  const int nopts = (int)(sizeof(opts) / sizeof(opts[0])) - (fit ? 0 : 1);
+  r = a->CompileProgram(p, nopts, opts);
   size_t ls = 0;
   if (a->GetProgramLogSize(p, &ls) == NVRTC_SUCCESS && ls > 1) {
     log->resize(ls);
@@ -120,6 +126,7 @@ struct UserProgram {
   std::string src;
   cudaLibrary_t lib = nullptr;
   cudaKernel_t score = nullptr, mask = nullptr;
+  cudaKernel_t fit = nullptr;  // null: the source defines no rsc_user_fit
 };
 
 struct UserShapes {
@@ -165,6 +172,105 @@ static RscUserPoints to_user_points(const PointSet& ps) {
   return u;
 }
 
+int32_t make_fit_order(rsc_ctx* ctx, const rsc_shape_slot* order, int32_t norder, FitOrder* fo, const char* who) {
+  const std::string w(who);
+  if (norder < 0 || norder > RSC_MAX_ORDER || (norder > 0 && !order)) return fail(ctx, RSC_E_ARG, (w + ": 0 <= norder <= 8").c_str());
+  fo->n = norder;
+  fo->has_user = false;
+  for (int i = 0; i < norder; ++i) {
+    const rsc_shape_slot& sl = order[i];
+    for (int j = 0; j < i; ++j)
+      if (order[j].type == sl.type) return fail(ctx, RSC_E_ARG, (w + ": a type appears twice in the fit order").c_str());
+    fo->type[i] = sl.type;
+    fo->nk[i] = 0;
+    for (int q = 0; q < 8; ++q) fo->k[i][q] = 0.0;
+    if (sl.type >= 0 && sl.type < RSC_NTYPES) continue;  // built-in: eps / alpha come from rsc_params
+    const UserProgram* prog = user_program(ctx, sl.type);
+    if (!prog) return fail(ctx, RSC_E_ARG, (w + ": type " + std::to_string(sl.type) + " is neither built-in nor a compiled user shape of this context").c_str());
+    if (!prog->fit) return fail(ctx, RSC_E_ARG, (w + ": user type " + std::to_string(sl.type) + " has no rsc_user_fit").c_str());
+    if (sl.nk < 0 || sl.nk > 8) return fail(ctx, RSC_E_ARG, (w + ": 0 <= nk <= 8 constants").c_str());
+    fo->nk[i] = sl.nk;
+    for (int q = 0; q < sl.nk; ++q) fo->k[i][q] = sl.k[q];
+    fo->has_user = true;
+  }
+  return RSC_OK;
+}
+
+int32_t user_fit_enqueue(rsc_ctx* ctx, const FitOrder& fo, int pos, const rsc_cloud* cloud, const int64_t* idx, int S, int np,
+                         rsc_cand* dense, uint32_t* okmask, cudaStream_t st) {
+  const UserProgram* prog = user_program(ctx, fo.type[pos]);
+  if (!prog || !prog->fit) return fail(ctx, RSC_E_ARG, "fit: user type without a compiled rsc_user_fit");
+  if (S <= 0) return RSC_OK;
+  RscUserFitArgs a;
+  memset(&a, 0, sizeof(a));
+  a.soa = cloud->soa;
+  a.n_pad = cloud->n_pad;
+  a.idx = reinterpret_cast<const long long*>(idx);
+  a.S = S, a.np = np, a.npos = fo.n, a.pos = pos, a.type = fo.type[pos], a.nk = fo.nk[pos];
+  for (int q = 0; q < 8; ++q) a.k[q] = fo.k[pos][q];
+  a.dense = reinterpret_cast<RscUserCand*>(dense);
+  a.okmask = okmask;
+  void* args[] = {&a};
+  RSC_CUDA(ctx, cudaLaunchKernel((const void*)prog->fit, dim3((unsigned)((S + 127) / 128)), dim3(128), args, 0, st));
+  return RSC_OK;
+}
+
+int32_t user_score_enqueue(rsc_ctx* ctx, const FitOrder& fo, const PointSet& ps, const rsc_cand* d_cands, int c_cap,
+                           const unsigned long long* d_count, int32_t* cv, int32_t* ce, cudaStream_t st) {
+  const int64_t ntiles = ps.n_pad / RSC_USER_THREADS;
+  if (c_cap <= 0 || ntiles <= 0) return RSC_OK;
+  for (int t = 0; t < fo.n; ++t) {
+    if (fo.type[t] < RSC_NTYPES) continue;
+    const UserProgram* prog = user_program(ctx, fo.type[t]);
+    if (!prog) return fail(ctx, RSC_E_ARG, "score: user type is not compiled on this context");
+    RscUserScoreArgs a;
+    memset(&a, 0, sizeof(a));
+    a.ps = to_user_points(ps);
+    a.cands = reinterpret_cast<const RscUserCand*>(d_cands);
+    a.C = c_cap;
+    a.nk = fo.nk[t];
+    for (int q = 0; q < 8; ++q) a.k[q] = fo.k[t][q];
+    a.counts = ce;
+    a.counts2 = cv;
+    a.d_count = d_count;
+    a.type = fo.type[t];
+    const int gx = (int)std::min<int64_t>(ntiles, (int64_t)ctx->sm_count * 8);
+    // (a launch sized by a capacity expects a quarter of it, like the small-batch scorer's)
+    const int chunks = ((d_count ? (c_cap + 3) / 4 : c_cap) + RSC_USER_TILE - 1) / RSC_USER_TILE;
+    const int gy = std::max(1, std::min(chunks, ctx->sm_count * 16 / gx));
+    void* args[] = {&a};
+    RSC_CUDA(ctx, cudaLaunchKernel((const void*)prog->score, dim3((unsigned)gx, (unsigned)gy), dim3(RSC_USER_THREADS), args, 0, st));
+    ctx->stats.score_launches += 1;
+  }
+  return RSC_OK;
+}
+
+int32_t user_refit_mask_enqueue(rsc_cloud* cloud, const FitOrder& fo, const rsc_cand& cand, cudaStream_t st) {
+  rsc_ctx* ctx = cloud->ctx;
+  int pos = -1;
+  for (int t = 0; t < fo.n; ++t)
+    if (fo.type[t] == cand.type) pos = t;
+  const UserProgram* prog = user_program(ctx, cand.type);
+  if (pos < 0 || !prog) return fail(ctx, RSC_E_ARG, "refit: user type is not part of the fit order");
+  uint32_t* inl = nullptr;
+  if (int32_t rc = refit_mask_buffer(cloud, &inl)) return rc;
+  RscUserMaskArgs a;
+  memset(&a, 0, sizeof(a));
+  a.ps = to_user_points(view_cloud(cloud));
+  memcpy(&a.cand, &cand, sizeof(rsc_cand));
+  a.nk = fo.nk[pos];
+  for (int q = 0; q < 8; ++q) a.k[q] = fo.k[pos][q];
+  a.inl = inl;
+  const int64_t nblk = cloud->n_pad / RSC_USER_THREADS;
+  if (nblk > 0) {
+    const unsigned grid = (unsigned)std::min<int64_t>(nblk, (int64_t)ctx->sm_count * 16);
+    void* args[] = {&a};
+    RSC_CUDA(ctx, cudaLaunchKernel((const void*)prog->mask, dim3(grid), dim3(RSC_USER_THREADS), args, 0, st));
+  }
+  ctx->stats.evals += cloud->n;
+  return refit_scan_enqueue(cloud, st);
+}
+
 }  // namespace rsc
 
 using namespace rsc;
@@ -194,14 +300,16 @@ int32_t rsc_user_shape_compile(rsc_ctx* ctx, const void* src, int64_t nbytes, in
       return RSC_OK;
     }
   std::string cubin, log;
-  const int32_t rc = user_compile(key.data(), key.size(), &cubin, &log);
+  bool has_fit = false;
+  const int32_t rc = user_compile(key.data(), key.size(), &cubin, &log, &has_fit);
   if (rc) return fail(ctx, rc, ("user_shape_compile: " + log).c_str());
   RSC_CUDA(ctx, cudaSetDevice(ctx->device));
   UserProgram p;
   p.src = key;
   RSC_CUDA(ctx, cudaLibraryLoadData(&p.lib, cubin.data(), nullptr, nullptr, 0, nullptr, nullptr, 0));
   if (cudaLibraryGetKernel(&p.score, p.lib, "rsc_user_score_kernel") != cudaSuccess ||
-      cudaLibraryGetKernel(&p.mask, p.lib, "rsc_user_mask_kernel") != cudaSuccess) {
+      cudaLibraryGetKernel(&p.mask, p.lib, "rsc_user_mask_kernel") != cudaSuccess ||
+      (has_fit && cudaLibraryGetKernel(&p.fit, p.lib, "rsc_user_fit_kernel") != cudaSuccess)) {
     cudaLibraryUnload(p.lib);
     cudaGetLastError();
     return fail(ctx, RSC_E_CUDA, "user_shape_compile: kernels missing from the compiled program");
@@ -241,6 +349,7 @@ int32_t rsc_user_score(rsc_cloud* cloud, const double* k, int32_t nk, const rsc_
   a.ps = to_user_points(ps);
   a.cands = ctx->cands.as<RscUserCand>();
   a.C = C;
+  a.type = cands[0].type;
   a.nk = nk;
   for (int i = 0; i < nk; ++i) a.k[i] = k[i];
   a.counts = ctx->counts.as<int32_t>();

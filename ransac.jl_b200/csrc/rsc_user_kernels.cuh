@@ -5,6 +5,11 @@
 //   __device__ bool rsc_user_compatible(const double p[7], int outwards, const double k[8],
 //                                       double x, double y, double z, double nx, double ny, double nz);
 //
+// and optionally (then the library compiles with -DRSC_USER_HAS_FIT)
+//
+//   __device__ bool rsc_user_fit(int np, const double P[8][3], const double N[8][3], const double k[8],
+//                                double p[7], int* outwards);
+//
 // for sm_100a with --fmad=false and no fast-math, so that a NumPy restatement in the same operation order makes
 // the same float64 decisions (DESIGN.md section 8).  The argument structs below are also compiled into the
 // library itself (nvcc): one definition, one layout on both sides of the cudaLaunchKernel call.  Only plain
@@ -39,6 +44,22 @@ struct RscUserScoreArgs {
   int* counts;       // [C], zeroed by the host
   unsigned* masks;   // nullable: candidate-major [C][words], zeroed by the host
   long long words;   // ceil(n / 32)
+  const unsigned long long* d_count;  // nullable: number of candidates = min(*d_count, C) (the device loop)
+  int type;                           // only records of this type are scored
+  int* counts2;                       // nullable: receives the same counts as `counts`
+};
+
+struct RscUserFitArgs {
+  const float* soa;      // the cloud: x | y | z | nx | ny | nz rows of n_pad floats
+  long long n_pad;
+  const long long* idx;  // [S][np] drawn indices; a row starting with -1 is a failed sample
+  int S, np;
+  int npos, pos;         // positions in the fit order / this type's position
+  int type;
+  int nk;
+  double k[8];
+  RscUserCand* dense;    // [S][npos]: slot s * npos + pos, as the built-in fit kernel writes
+  unsigned* okmask;      // [(S + 127) / 128][npos][4] ballot words
 };
 
 struct RscUserMaskArgs {
@@ -62,15 +83,18 @@ __device__ bool rsc_user_compatible(const double p[7], int outwards, const doubl
 // them as broadcasts; a (candidate, 32 points) group is one ballot, its POPC goes into a shared counter, and each
 // CTA adds one atomic per candidate.  Candidate chunks are spread over gridDim.y.  Every pair is decided once, in
 // float64, on the point's float32 coordinates widened to double.
+// The device loop passes a mixed batch of built-in and user records whose size may stay on the device (a.d_count):
+// only records of a.type are scored, and their counts are ADDED where the built-in scorer has left zeros.
 extern "C" __global__ void __launch_bounds__(RSC_USER_THREADS) rsc_user_score_kernel(const RscUserScoreArgs a) {
   __shared__ RscUserCand sc[RSC_USER_TILE];
   __shared__ int scount[RSC_USER_TILE];
   __shared__ double sk[8];
   const int lane = threadIdx.x & 31;
   if (threadIdx.x < 8) sk[threadIdx.x] = threadIdx.x < a.nk ? a.k[threadIdx.x] : 0.0;
+  const int C = a.d_count && *a.d_count < (unsigned long long)a.C ? (int)*a.d_count : a.C;
   const long long ntiles = a.ps.n_pad / RSC_USER_THREADS;
-  for (int c0 = blockIdx.y * RSC_USER_TILE; c0 < a.C; c0 += gridDim.y * RSC_USER_TILE) {
-    const int ct = min(RSC_USER_TILE, a.C - c0);
+  for (int c0 = blockIdx.y * RSC_USER_TILE; c0 < C; c0 += gridDim.y * RSC_USER_TILE) {
+    const int ct = min(RSC_USER_TILE, C - c0);
     for (int i = threadIdx.x; i < ct; i += RSC_USER_THREADS) {
       sc[i] = a.cands[c0 + i];
       scount[i] = 0;
@@ -84,6 +108,7 @@ extern "C" __global__ void __launch_bounds__(RSC_USER_THREADS) rsc_user_score_ke
       const double x = __ldg(a.ps.x + p), y = __ldg(a.ps.y + p), z = __ldg(a.ps.z + p);
       const double nx = __ldg(a.ps.nx + p), ny = __ldg(a.ps.ny + p), nz = __ldg(a.ps.nz + p);
       for (int c = 0; c < ct; ++c) {
+        if (sc[c].type != a.type) continue;  // block-uniform: a record of another type in a mixed batch
         const bool ok = on && rsc_user_compatible(sc[c].p, sc[c].outwards, sk, x, y, z, nx, ny, nz);
         const unsigned b = __ballot_sync(0xffffffffu, ok);
         if (lane == 0 && b) {
@@ -94,7 +119,10 @@ extern "C" __global__ void __launch_bounds__(RSC_USER_THREADS) rsc_user_score_ke
     }
     __syncthreads();
     for (int i = threadIdx.x; i < ct; i += RSC_USER_THREADS)
-      if (scount[i]) atomicAdd(a.counts + c0 + i, scount[i]);
+      if (scount[i]) {
+        atomicAdd(a.counts + c0 + i, scount[i]);
+        if (a.counts2) atomicAdd(a.counts2 + c0 + i, scount[i]);
+      }
     __syncthreads();
   }
 }
@@ -119,5 +147,43 @@ extern "C" __global__ void __launch_bounds__(RSC_USER_THREADS) rsc_user_mask_ker
     if (lane == 0) a.inl[p >> 5] = b;
   }
 }
+
+#ifdef RSC_USER_HAS_FIT
+__device__ bool rsc_user_fit(int np, const double P[8][3], const double N[8][3], const double k[8], double p[7], int* outwards);
+
+// K1 for one user type: one thread per minimal set, the shape of the built-in fit kernel (rsc_fit.cu).  The
+// candidate goes to the same dense slot and the set's bit into the same ballot word the built-in fits use, so
+// the library's group scan and compaction emit (set, position in the fit order) order unchanged.
+extern "C" __global__ void __launch_bounds__(128) rsc_user_fit_kernel(const RscUserFitArgs a) {
+  const int s = blockIdx.x * blockDim.x + threadIdx.x;
+  bool ok = false;
+  if (s < a.S && a.idx[(long long)s * a.np] >= 0) {
+    double P[8][3], N[8][3], k[8], p[7];
+    for (int q = 0; q < 8; ++q) {
+      k[q] = q < a.nk ? a.k[q] : 0.0;
+      for (int d = 0; d < 3; ++d) P[q][d] = N[q][d] = 0.0;
+    }
+    for (int q = 0; q < a.np; ++q) {
+      const long long i = a.idx[(long long)s * a.np + q];
+      for (int d = 0; d < 3; ++d) {
+        P[q][d] = (double)__ldg(a.soa + d * a.n_pad + i);
+        N[q][d] = (double)__ldg(a.soa + (3 + d) * a.n_pad + i);
+      }
+    }
+    for (int j = 0; j < 7; ++j) p[j] = 0.0;
+    int outw = 0;
+    ok = rsc_user_fit(a.np, P, N, k, p, &outw);
+    if (ok) {
+      RscUserCand c;
+      c.type = a.type;
+      c.outwards = outw;
+      for (int j = 0; j < 7; ++j) c.p[j] = p[j];
+      a.dense[(long long)s * a.npos + a.pos] = c;
+    }
+  }
+  const unsigned m = __ballot_sync(0xffffffffu, ok);
+  if ((threadIdx.x & 31) == 0) a.okmask[((long long)blockIdx.x * a.npos + a.pos) * 4 + (threadIdx.x >> 5)] = m;
+}
+#endif  // RSC_USER_HAS_FIT
 
 #endif  // __CUDACC_RTC__

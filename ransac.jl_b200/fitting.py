@@ -16,7 +16,7 @@ from ._lib import lib
 from .cloud import RANSACCloud
 from .confidence import ConfidenceInterval, estimatescore, estimatescore_f64, isoverlap
 from .params import to_c
-from .shapes import SHAPE_KIND, ExtractedShape, FittedShape, from_cand, on_device, pack_cands, user_cand
+from .shapes import SHAPE_KIND, ExtractedShape, FittedShape, device_fit, from_cand, on_device, pack_cands, user_cand
 
 
 # ---- fit (fitting.jl:30; plane.jl:33, sphere.jl:87, cylinder.jl:135, cone.jl:123) ------------
@@ -69,6 +69,49 @@ def sample_fit(pc: RANSACCloud, params, seed: int, set0: int, S: int):
     out_n = C.c_int32()
     pc.ctx.check(lib.rsc_sample_fit(pc.handle, C.byref(cp), seed, set0, S, out, out_set.ctypes.data, out_idx.ctypes.data, C.byref(out_n)))
     return [from_cand(out[i]) for i in range(out_n.value)], out_set[: out_n.value].copy(), out_idx
+
+
+def fit_order(pc: RANSACCloud, types, params):
+    """rsc_shape_slot[] of a fit order: built-in kinds, and user classes that fit on the device (`device_fit`) under
+    their compiled type ids with their `device_constants`.  Returns (slots, {type id: class})."""
+    if len(types) > _lib.RSC_MAX_ORDER:
+        raise ValueError(f"at most {_lib.RSC_MAX_ORDER} shape types in one fit order")
+    slots = (_lib.rsc_shape_slot * max(len(types), 1))()
+    classes = {}
+    for i, t in enumerate(types):
+        if t in SHAPE_KIND:
+            slots[i].type = SHAPE_KIND[t]
+            continue
+        if not device_fit(t):
+            raise TypeError(f"{t.__name__} does not fit on the device (cuda_source with rsc_user_fit, from_device_record)")
+        k = _user_constants(t, params)
+        slots[i].type = pc.ctx.user_type(t)
+        slots[i].nk = len(k)
+        slots[i].k[: len(k)] = list(k)
+        classes[slots[i].type] = t
+    return slots, classes
+
+
+def shape_from_record(c: _lib.rsc_cand, classes) -> FittedShape:
+    """A built-in rsc_cand, or a user record under a type id of `classes` (fit_order) via `from_device_record`."""
+    if c.type in classes:
+        return classes[c.type].from_device_record(list(c.p), bool(c.outwards))
+    return from_cand(c)
+
+
+def sample_fit_user(pc: RANSACCloud, params, types, seed: int, set0: int, S: int):
+    """sample_fit with a mixed fit order (rsc_sample_fit_user): built-ins and device-fitting user classes in the
+    order `types`; the candidates come back in (set, position) order.  `types = []` only draws the sets."""
+    cp = to_c(_builtin_params(params))
+    slots, classes = fit_order(pc, types, params)
+    cap = max(S * len(types), 1)
+    out = (_lib.rsc_cand * cap)()
+    out_set = np.zeros(cap, dtype=np.int32)
+    out_idx = np.zeros((S, cp.drawN), dtype=np.int64)
+    out_n = C.c_int32()
+    pc.ctx.check(lib.rsc_sample_fit_user(pc.handle, C.byref(cp), slots, len(types), seed, set0, S, out, out_set.ctypes.data,
+                                         out_idx.ctypes.data, C.byref(out_n)))
+    return [shape_from_record(out[i], classes) for i in range(out_n.value)], out_set[: out_n.value].copy(), out_idx
 
 
 def sample_fit_cells(pc: RANSACCloud, params, seed: int, set0: int, S: int, levelweight):

@@ -1,11 +1,12 @@
 """ransac(pc, params, setenabled; reset_rand): mirror of src/iterations.jl:14-162.
 
 For the four built-in shape types the whole loop runs inside the CUDA library behind one C-ABI call
-(`rsc_ransac_run`).  If `shape_types` contains a user-defined FittedShape subclass the loop runs
-here and calls that class's own `fit`/`scorecandidate`/`refit` methods -- the reference's plug-in
-contract (docs/src/newprimitive.md:12-18) -- while built-in types still score on the device.  A user
-shape with `cuda_source` keeps its own `fit` but scores and refits on the device (rsc_user_score,
-rsc_user_refit_extract).
+(`rsc_ransac_run`).  User-defined shapes whose `cuda_source` also fits (`shapes.device_fit`) join that loop
+(`rsc_ransac_run_user`) unless an extension switch is asked for.  Otherwise, if `shape_types` contains a
+user-defined FittedShape subclass, the loop runs here and calls that class's own
+`fit`/`scorecandidate`/`refit` methods -- the reference's plug-in contract (docs/src/newprimitive.md:12-18)
+-- while built-in types still score on the device.  A user shape with `cuda_source` scores and refits on the
+device (rsc_user_score, rsc_user_refit_extract), and fits there too when it can (rsc_sample_fit_user).
 """
 from __future__ import annotations
 
@@ -19,9 +20,10 @@ from . import _lib
 from ._lib import lib
 from .cloud import RANSACCloud
 from .confidence import estimatescore_f64, prob
-from .fitting import IterationCandidates, findhighestscore, lsq_refit, refine_progressive, refit, sample_fit, scorecandidates
+from .fitting import (IterationCandidates, findhighestscore, fit_order, lsq_refit, refine_progressive, refit, sample_fit,
+                      sample_fit_user, scorecandidates, shape_from_record)
 from .params import to_c
-from .shapes import SHAPE_KIND, ExtractedShape, from_cand, on_device
+from .shapes import SHAPE_KIND, ExtractedShape, device_fit, on_device
 
 
 def _all_builtin(params) -> bool:
@@ -53,6 +55,8 @@ def ransac(pc: RANSACCloud, params, setenabled: bool = True, reset_rand: bool = 
         seed = 1234
     if _all_builtin(params):
         return _ransac_device(pc, params, seed, sampler, lsq, progressive, bitmap, lw_period)
+    if _device_order(pc, params["iteration"]["shape_types"]) and sampler == "root" and not progressive and not lsq and bitmap is None:
+        return _ransac_device(pc, params, seed, order=params["iteration"]["shape_types"])
     if bitmap is not None:
         raise ValueError("the bitmap filter is only available in the device loop (built-in shape types)")
     if sampler != "root":
@@ -60,7 +64,20 @@ def ransac(pc: RANSACCloud, params, setenabled: bool = True, reset_rand: bool = 
     return _ransac_host(pc, params, seed, progressive, lsq)
 
 
-def _ransac_device(pc, params, seed, sampler="root", lsq=False, progressive=False, bitmap=None, lw_period=1):
+def _device_order(pc, types) -> bool:
+    """True when rsc_ransac_run_user takes `types`: built-ins and device-fitting user classes only, at most
+    RSC_MAX_ORDER of them, none twice, on a whole (not sharded, not ranged) cloud."""
+    return (all(t in SHAPE_KIND or device_fit(t) for t in types) and len(types) <= _lib.RSC_MAX_ORDER
+            and len(set(types)) == len(types) and not pc.is_shard and not getattr(pc, "ranged", False))
+
+
+def _ransac_device(pc, params, seed, sampler="root", lsq=False, progressive=False, bitmap=None, lw_period=1, order=None):
+    """The device loop: rsc_ransac_run, or rsc_ransac_run_user for a fit order `order` of built-in and device-fitting
+    user classes (no extension switches then)."""
+    classes = {}
+    if order is not None:
+        slots, classes = fit_order(pc, order, params)
+        params = dict(params, iteration=dict(params["iteration"], shape_types=[t for t in order if t in SHAPE_KIND]))
     cp = to_c(params)
     cp.lw_period = max(1, int(lw_period))  # octree sampler: refresh period of the level weights (1 = every iteration)
     if bitmap is not None:
@@ -77,7 +94,10 @@ def _ransac_device(pc, params, seed, sampler="root", lsq=False, progressive=Fals
     elif sampler != "root":
         raise ValueError("sampler must be 'root' or 'octree'")
     run = C.c_void_p()
-    pc.ctx.check(lib.rsc_ransac_run(pc.handle, C.byref(cp), seed, C.byref(run)))
+    if order is not None:
+        pc.ctx.check(lib.rsc_ransac_run_user(pc.handle, C.byref(cp), slots, len(order), seed, C.byref(run)))
+    else:
+        pc.ctx.check(lib.rsc_ransac_run(pc.handle, C.byref(cp), seed, C.byref(run)))
     try:
         out = []
         for i in range(lib.rsc_run_nshapes(run)):
@@ -87,7 +107,7 @@ def _ransac_device(pc, params, seed, sampler="root", lsq=False, progressive=Fals
             idx = np.empty(n.value, dtype=np.int64)  # filled by rsc_run_inpoints (device -> host)
             if n.value:
                 pc.ctx.check(lib.rsc_run_inpoints(run, i, idx.ctypes.data))
-            ex = ExtractedShape(from_cand(cand), idx)
+            ex = ExtractedShape(shape_from_record(cand, classes), idx)
             # sharded storage: `inpoints` is this rank's part of the list (shard.gather_extracted joins them)
             ex.total = int(lib.rsc_run_shape_total(run, i))
             out.append(ex)
@@ -114,7 +134,10 @@ def _ransac_host(pc, params, seed, progressive=False, lsq=False):
     drawN, minsubsetN, prob_det, tau = it["drawN"], it["minsubsetN"], it["prob_det"], it["tau"]
     sidx = {"lengthC": 0, "allcand": 1, "nofminset": 2}
     builtin = [t for t in it["shape_types"] if t in SHAPE_KIND]
-    custom = [t for t in it["shape_types"] if t not in SHAPE_KIND]
+    # built-ins and user shapes that fit on the device: one rsc_sample_fit_user call per iteration; the other user
+    # shapes fit here, on the same drawn sets
+    devfit = [t for t in it["shape_types"] if t in SHAPE_KIND or device_fit(t)]
+    custom = [t for t in it["shape_types"] if t not in devfit]
     bparams = dict(params, iteration=dict(it, shape_types=builtin))
     t0 = time.time()
     scored = IterationCandidates()
@@ -125,10 +148,11 @@ def _ransac_host(pc, params, seed, progressive=False, lsq=False):
     for k in range(1, it["itermax"] + 1):
         if pc.count_enabled() < tau:
             break
-        cands, csets, idx = sample_fit(pc, bparams, seed, (k - 1) * minsubsetN, minsubsetN) if builtin else ([], [], None)
+        if devfit == builtin and builtin:
+            cands, csets, idx = sample_fit(pc, bparams, seed, (k - 1) * minsubsetN, minsubsetN)
+        else:  # device-fitting user types: merged candidates; no device-fitting type at all: the same sets, drawn only
+            cands, csets, idx = sample_fit_user(pc, params, devfit, seed, (k - 1) * minsubsetN, minsubsetN)
         if custom:
-            if idx is None:
-                raise NotImplementedError("user-defined shapes need at least one built-in type for sampling")
             # forcefitshapes! (fitting.jl:165-173) appends per minimal set in shape_types order: merge the device's
             # built-in candidates with the user's by (set, position in shape_types) -- findhighestscore is
             # "first maximum wins", so the order decides ties

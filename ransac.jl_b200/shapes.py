@@ -17,7 +17,10 @@ class FittedShape:
     A user shape may also run its scoring and refit on the device.  It then defines three members:
     `cuda_source` (class attribute: CUDA C defining `rsc_user_compatible`, include/rsc.h), `device_record(self)`
     -> (p, outwards) with at most 7 floats, and the staticmethod `device_constants(params)` -> at most 8 floats
-    (thresholds such as eps and cos(alpha), computed on the host).  Its `fit` stays on the host."""
+    (thresholds such as eps and cos(alpha), computed on the host).  Its `fit` stays on the host unless its
+    `cuda_source` also defines `rsc_user_fit` and the class provides the classmethod `from_device_record(p, outwards)`
+    (the inverse of `device_record`): then it fits on the device too, and a parameter set of such shapes and built-ins
+    runs in the device loop (`device_fit`)."""
 
     kind = -1
     cuda_source = None
@@ -29,6 +32,13 @@ class FittedShape:
 def on_device(shape_class) -> bool:
     """True for a user-defined shape class that brings device source (`cuda_source`)."""
     return shape_class not in SHAPE_KIND and getattr(shape_class, "cuda_source", None) is not None
+
+
+def device_fit(shape_class) -> bool:
+    """True for a user-defined shape class that fits on the device: its `cuda_source` defines `rsc_user_fit` and it
+    turns device records back into instances with `from_device_record(p, outwards)`."""
+    return (on_device(shape_class) and "rsc_user_fit" in shape_class.cuda_source
+            and callable(getattr(shape_class, "from_device_record", None)))
 
 
 def user_cand(s: FittedShape, type_id: int) -> _lib.rsc_cand:

@@ -133,6 +133,7 @@ class ShardedContext:
         if set_range:
             lo, hi = self.range  # an empty range (lo == hi) is a rank that only joins the all-reduces
             pc.ctx.check(lib.rsc_cloud_set_range(pc.handle, lo, hi))
+            pc.ranged = True  # (ransac() keeps such a cloud out of rsc_ransac_run_user)
 
     def close(self):
         if self.comm == "nccl":
