@@ -146,7 +146,8 @@ int32_t rsc_ctx_last_kernel(rsc_ctx* ctx, double* kernel_ms, int64_t* guard_pair
 /* ---- cloud: RANSACCloud (octree.jl:37-59, ctors :78-138) ------------------------------ */
 /* xyz/nrm are AoS (N x 3), bit-compatible with Vector{SVector{3,Float32}}; stored on device as
  * SoA float32.  `_f64` down-converts Vector{SVector{3,Float64}} (the device computes on the float32
- * roundings: decisions are the float64 ones OF THE ROUNDED coordinates).  `_shard` uploads the point
+ * roundings: decisions are the float64 ones OF THE ROUNDED coordinates; `_f64_exact` below keeps the
+ * float64 coordinates too).  `_shard` uploads the point
  * range [global_offset, global_offset+n) of a cloud of n_global points (one shard per GPU/process,
  * sharded storage): global_offset must be a multiple of 2048 and n a multiple of 2048 unless the range
  * ends the cloud; indices the library returns or takes (subsets, inlier lists) are GLOBAL.
@@ -159,6 +160,15 @@ int32_t rsc_cloud_create(rsc_ctx* ctx, const float* xyz, const float* nrm, int64
 int32_t rsc_cloud_create_f64(rsc_ctx* ctx, const double* xyz, const double* nrm, int64_t n, rsc_cloud** out);
 int32_t rsc_cloud_create_shard(rsc_ctx* ctx, const float* xyz, const float* nrm, int64_t n,
                                int64_t global_offset, int64_t n_global, rsc_cloud** out);
+/* Like rsc_cloud_create_f64, but the device also keeps the caller's float64 coordinates: every
+ * decision (scoring, refit/extraction, the loops) is the float64 one of the UNROUNDED points and
+ * every fit runs on them.  +48 B/point of HBM.  Refused later on: rsc_cloud_update, rsc_cloud_set_range.
+ * Not yet available on an exact cloud (RSC_E_STATE): the cell sampler (rsc_sample_fit_cells,
+ * RSC_SAMPLER_OCTREE), RSC_SCORE_PROGRESSIVE, RSC_REFIT_LSQ / rsc_refit_lsq and RSC_EXTRACT_BITMAP /
+ * rsc_bitmap_filter.  rsc_cloud_build_cells quantises the float32 roundings; on an exact cloud its
+ * cells only order the culled scorer (rsc_score_culled), whose counts do not depend on the order. */
+int32_t rsc_cloud_create_f64_exact(rsc_ctx* ctx, const double* xyz, const double* nrm, int64_t n, rsc_cloud** out);
+int32_t rsc_cloud_is_exact(const rsc_cloud* cloud); /* 1 / 0 */
 /* Re-upload new coordinates (same n) into the device buffers of an existing cloud: all points
  * enabled again, subset copies re-gathered, the flattened octree (rsc_cloud_build_cells) dropped.
  * A re-scan of the same scene, no re-allocation. */

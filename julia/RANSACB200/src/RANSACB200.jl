@@ -116,11 +116,13 @@ function context(device::Integer=0)
     CTX[]
 end
 
-"Device twin of a `RANSACCloud`: uploads vertices/normals (float32 SoA on the GPU) and subset 1."
+"""Device twin of a `RANSACCloud`: uploads vertices/normals (float32 SoA on the GPU) and subset 1.
+`exact=true` on a Float64 cloud keeps the Float64 coordinates on the device too (`rsc_cloud_create_f64_exact`,
++48 B/point): every decision and fit is then the Float64 one of the points as given."""
 mutable struct DeviceCloud
     h::Ptr{Cvoid}
     pc::RANSACCloud
-    function DeviceCloud(pc::RANSACCloud)
+    function DeviceCloud(pc::RANSACCloud; exact::Bool=false)
         ctx = context()
         h = Ref{Ptr{Cvoid}}(C_NULL)
         v, n = pc.vertices, pc.normals            # Vector{SVector{3,T}} is bit-compatible with T[3N]
@@ -132,6 +134,9 @@ mutable struct DeviceCloud
         GC.@preserve v n begin
             if eltype(eltype(v)) == Float32
                 check(ccall(fn(:rsc_cloud_create), Int32, (Ptr{Cvoid}, Ptr{Float32}, Ptr{Float32}, Int64, Ref{Ptr{Cvoid}}),
+                            ctx, pointer(v), pointer(n), pc.size, h))
+            elseif exact
+                check(ccall(fn(:rsc_cloud_create_f64_exact), Int32, (Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}, Int64, Ref{Ptr{Cvoid}}),
                             ctx, pointer(v), pointer(n), pc.size, h))
             else
                 check(ccall(fn(:rsc_cloud_create_f64), Int32, (Ptr{Cvoid}, Ptr{Float64}, Ptr{Float64}, Int64, Ref{Ptr{Cvoid}}),

@@ -83,6 +83,8 @@ SIGNATURES = {
     "rsc_ctx_last_kernel": (C.c_int32, [_P, C.POINTER(C.c_double), C.POINTER(C.c_int64)]),
     "rsc_cloud_create": (C.c_int32, [_P, _P, _P, C.c_int64, C.POINTER(_P)]),
     "rsc_cloud_create_f64": (C.c_int32, [_P, _P, _P, C.c_int64, C.POINTER(_P)]),
+    "rsc_cloud_create_f64_exact": (C.c_int32, [_P, _P, _P, C.c_int64, C.POINTER(_P)]),
+    "rsc_cloud_is_exact": (C.c_int32, [_P]),
     "rsc_cloud_create_shard": (C.c_int32, [_P, _P, _P, C.c_int64, C.c_int64, C.c_int64, C.POINTER(_P)]),
     "rsc_cloud_update": (C.c_int32, [_P, _P, _P, C.c_int64]),
     "rsc_cloud_destroy": (None, [_P]),

@@ -30,9 +30,12 @@ def makesubsets(n: int, numofsubsets: int, rng: np.random.Generator) -> List[np.
 
 
 class RANSACCloud:
-    """RANSACCloud(vertices, normals, numofsubsets | subsets; force_eltype=None).
+    """RANSACCloud(vertices, normals, numofsubsets | subsets; force_eltype=None, exact=False).
 
     vertices/normals: (N,3) arrays (float32 or float64; the device copy is float32).
+    exact=True with float64 input keeps the float64 coordinates on the device too
+    (rsc_cloud_create_f64_exact, +48 B/point): every decision and fit is then the float64 one of
+    the caller's unrounded points.  float32 input is exact already.  Not with `shard=`.
     """
 
     def __init__(
@@ -45,7 +48,10 @@ class RANSACCloud:
         seed: int = 1234,
         shard: Optional[tuple] = None,
         ctx: Optional[Context] = None,
+        exact: bool = False,
     ):
+        if exact and shard is not None:
+            raise ValueError("RANSACCloud: exact=True does not support sharded storage (shard=)")
         v = np.asarray(vertices)
         n = np.asarray(normals)
         assert v.shape == n.shape, "Every point must have a normal."
@@ -79,6 +85,8 @@ class RANSACCloud:
             self.is_shard = self.n_global > self.size
         elif self.vertices.dtype == np.float32:
             rc = lib.rsc_cloud_create(self.ctx.h, self.vertices.ctypes.data, self.normals.ctypes.data, self.size, C.byref(self._h))
+        elif exact:
+            rc = lib.rsc_cloud_create_f64_exact(self.ctx.h, self.vertices.ctypes.data, self.normals.ctypes.data, self.size, C.byref(self._h))
         else:
             rc = lib.rsc_cloud_create_f64(self.ctx.h, self.vertices.ctypes.data, self.normals.ctypes.data, self.size, C.byref(self._h))
         self.ctx.check(rc)
@@ -90,6 +98,12 @@ class RANSACCloud:
     @property
     def handle(self):
         return self._h
+
+    @property
+    def exact(self) -> bool:
+        """True when every device decision and fit is the float64 one of the points as given
+        (float32 input, or float64 input with exact=True)."""
+        return self.vertices.dtype == np.float32 or bool(lib.rsc_cloud_is_exact(self._h))
 
     def upload_subset(self, subset_id: int):
         if subset_id in self._uploaded:

@@ -231,6 +231,7 @@ int32_t rsc_score(rsc_cloud* cloud, const rsc_params* params, const rsc_cand* ca
         PointSet sl = ps;
         sl.x += off, sl.y += off, sl.z += off, sl.nx += off, sl.ny += off, sl.nz += off;
         sl.enabled += off / 32, sl.valid += off / 32;
+        if (sl.xyz64) sl.xyz64 += 3 * off, sl.nrm64 += 3 * off;  // (the whole cloud: no map)
         sl.n = cloud->chunk_begin(i + 1) - off;
         sl.n_pad = (i == nchunks - 1) ? cloud->n_pad - off : sl.n;
         RSC_CUDA(ctx, cudaStreamWaitEvent(st, cloud->chunk_ev[i], 0));

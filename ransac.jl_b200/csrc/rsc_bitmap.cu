@@ -352,6 +352,7 @@ extern "C" int32_t rsc_bitmap_filter(rsc_cloud* cloud, const rsc_cand* cand, dou
   if (!cloud) return RSC_E_ARG;
   rsc_ctx* ctx = cloud->ctx;
   if (!cand || !out_n || n < 0 || (n > 0 && (!idx || !out_idx))) return fail(ctx, RSC_E_ARG, "bitmap_filter: null arguments");
+  if (cloud->exact()) return fail(ctx, RSC_E_STATE, "bitmap_filter: the bitmap filter does not support exact clouds yet");
   *out_n = 0;
   if (n == 0) {
     if (info) info[0] = info[1] = info[2] = info[3] = 0;

@@ -281,7 +281,8 @@ static int32_t cloud_upload(rsc_cloud* c, const T* xyz, const T* nrm) {
   fill_valid_kernel<<<(unsigned)((words + 255) / 256), 256, 0, cs>>>(c->valid, c->enabled, n, words);
   RSC_CUDA(ctx, cudaGetLastError());
   const size_t cbytes = (size_t)3 * kChunkPts * sizeof(T);
-  for (int b = 0; b < 2; ++b) RSC_CUDA(ctx, ctx->stage[b].ensure(2 * cbytes));
+  if (!c->xyz64)
+    for (int b = 0; b < 2; ++b) RSC_CUDA(ctx, ctx->stage[b].ensure(2 * cbytes));
   const int nt = staged ? host_copy_threads() : 1;
   if (staged)
     if (int32_t rcs = ensure_hstage(ctx, 2 * cbytes)) return rcs;
@@ -290,6 +291,12 @@ static int32_t cloud_upload(rsc_cloud* c, const T* xyz, const T* nrm) {
     const int64_t cnt = c->chunk_begin(i + 1) - off;
     T* sx = ctx->stage[i & 1].as<T>();
     T* sn = sx + 3 * kChunkPts;
+    if constexpr (sizeof(T) == sizeof(double)) {
+      if (c->xyz64) {  // exact cloud: the chunk lands in the persistent float64 arrays, the transposition reads it there
+        sx = c->xyz64 + 3 * off;
+        sn = c->nrm64 + 3 * off;
+      }
+    }
     if (staged) {
       const size_t half = (size_t)3 * cnt * sizeof(T);
       char* hs = static_cast<char*>(ctx->hstage[i & 1]);
@@ -336,7 +343,7 @@ int32_t cloud_ready(rsc_cloud* c) {
 
 template <class T>
 static int32_t cloud_create_impl(rsc_ctx* ctx, const T* xyz, const T* nrm, int64_t n, int64_t global_offset,
-                                 int64_t n_global, rsc_cloud** out) {
+                                 int64_t n_global, rsc_cloud** out, bool exact = false) {
   if (!ctx || !out) return RSC_E_ARG;
   *out = nullptr;
   if (!xyz || !nrm || n <= 0) return fail(ctx, RSC_E_ARG, "cloud_create: empty cloud or null arrays");
@@ -361,6 +368,11 @@ static int32_t cloud_create_impl(rsc_ctx* ctx, const T* xyz, const T* nrm, int64
     return fail_cuda(ctx, e, "cloud_create: cudaMalloc");
   }
   RSC_CUDA(ctx, cudaMemsetAsync(c->soa, 0, (size_t)6 * c->n_pad * sizeof(float), st));
+  if (exact && ((e = cudaMalloc(&c->xyz64, (size_t)3 * n * sizeof(double))) != cudaSuccess ||
+                (e = cudaMalloc(&c->nrm64, (size_t)3 * n * sizeof(double))) != cudaSuccess)) {
+    rsc_cloud_destroy(c);
+    return fail_cuda(ctx, e, "cloud_create_f64_exact: cudaMalloc");
+  }
   if (shard) {  // replicated whole-cloud enabled mask, all points enabled (like every rank's local mask)
     c->g_words = (n_global + kTile - 1) / kTile * (kTile / 32);
     if ((e = cudaMalloc(&c->g_enabled, (size_t)c->g_words * 4)) != cudaSuccess) {
@@ -393,6 +405,12 @@ int32_t rsc_cloud_create_f64(rsc_ctx* ctx, const double* xyz, const double* nrm,
   return cloud_create_impl<double>(ctx, xyz, nrm, n, 0, n, out);
 }
 
+int32_t rsc_cloud_create_f64_exact(rsc_ctx* ctx, const double* xyz, const double* nrm, int64_t n, rsc_cloud** out) {
+  return cloud_create_impl<double>(ctx, xyz, nrm, n, 0, n, out, true);
+}
+
+int32_t rsc_cloud_is_exact(const rsc_cloud* c) { return c && c->exact() ? 1 : 0; }
+
 int32_t rsc_cloud_create_shard(rsc_ctx* ctx, const float* xyz, const float* nrm, int64_t n, int64_t global_offset,
                                int64_t n_global, rsc_cloud** out) {
   if (global_offset < 0 || n_global < global_offset + n) return fail(ctx, RSC_E_ARG, "cloud_create_shard: bad range");
@@ -401,6 +419,7 @@ int32_t rsc_cloud_create_shard(rsc_ctx* ctx, const float* xyz, const float* nrm,
 
 int32_t rsc_cloud_update(rsc_cloud* c, const float* xyz, const float* nrm, int64_t n) {
   if (!c) return RSC_E_ARG;
+  if (c->exact()) return fail(c->ctx, RSC_E_STATE, "cloud_update: an exact cloud keeps the float64 coordinates it was created from (create a new one)");
   if (!xyz || !nrm || n != c->n) return fail(c->ctx, RSC_E_ARG, "cloud_update: the cloud size cannot change");
   RSC_CUDA(c->ctx, cudaSetDevice(c->ctx->device));
   int32_t rc = cloud_ready(c);  // an earlier upload may still be in flight
@@ -443,6 +462,8 @@ void rsc_cloud_destroy(rsc_cloud* c) {
     s.release_cull_view();
   }
   if (c->soa) cudaFree(c->soa);
+  if (c->xyz64) cudaFree(c->xyz64);
+  if (c->nrm64) cudaFree(c->nrm64);
   if (c->g_enabled) cudaFree(c->g_enabled);
   if (c->enabled) cudaFree(c->enabled);
   if (c->valid) cudaFree(c->valid);
@@ -479,6 +500,8 @@ int32_t rsc_cloud_set_subset(rsc_cloud* c, int32_t subset_id, const int64_t* idx
   }
   s.m = m;
   s.m_global = m_global;
+  s.xyz64 = c->xyz64;
+  s.nrm64 = c->nrm64;
   s.m_pad = (m + kTile - 1) / kTile * kTile;
   if (s.m_pad == 0) s.m_pad = kTile;  // a rank may own no point of the subset: one all-padding tile
   const int64_t words = s.m_pad / 32;

@@ -36,6 +36,11 @@ struct PointSet {
   const uint32_t* valid;    // 1 for real points, 0 for padding
   int64_t n;
   int64_t n_pad;
+  // exact clouds (rsc_cloud_create_f64_exact): the caller's float64 coordinates, AoS [3 n] in the cloud's point
+  // order; real point j of the set is cloud point map[j] (map == nullptr: j).  Null for every other cloud.
+  const double* xyz64 = nullptr;
+  const double* nrm64 = nullptr;
+  const int64_t* map = nullptr;
 };
 
 // per-type thresholds, FP32 for the tiled kernel and FP64 for the exact re-evaluation
@@ -45,6 +50,8 @@ struct Thresh {
   double eps_d[RSC_NTYPES];
   double cosa_d[RSC_NTYPES];
   uint32_t honour_enabled;  // bit t set: type t ANDs pc.isenabled into its inliers (Q4 clears SPHERE)
+  uint32_t exact_in = 0;    // 1: the points are the float32 roundings of float64 ones and every decision is the float64
+                            // one of the unrounded point: the guard bands carry the input-rounding term (kappa_in)
 };
 
 // block table written by the candidate compiler: which slots/type each CTA column covers
@@ -121,6 +128,7 @@ struct rsc_subset {
   uint32_t* enabled = nullptr; // m_pad/32 words
   uint32_t* valid = nullptr;
   int64_t* idx = nullptr;      // m local point indices (device)
+  const double* xyz64 = nullptr, *nrm64 = nullptr;  // the cloud's float64 coordinates (exact clouds; idx maps into them)
   // Morton-ordered view for the culled scorer (rsc_cull.cu), built on first use by subset_cull_view():
   // the same m points in a spatially coherent order + bounding spheres of their 128 / 512-point tiles
   float* csoa = nullptr;       // 6 * m_pad floats
@@ -141,6 +149,7 @@ struct rsc_cells {
   int nlevels = 0;               // 0: not built
   uint32_t* codes = nullptr;     // [n] sorted Morton codes (3 (nlevels-1) bits)
   uint32_t* perm = nullptr;      // [n] sorted position -> point index
+  int64_t* perm64 = nullptr;     // [n] the same, widened: the map of msoa into an exact cloud's float64 coordinates
   uint32_t* inv = nullptr;       // [n] point index -> sorted position
   uint8_t* leafdepth = nullptr;  // [n] by point index: first level whose cell holds <= 8 points
   uint32_t* en_sorted = nullptr; // [n_pad/32] pc.isenabled in Morton order
@@ -161,6 +170,11 @@ struct rsc_cloud {
   float* soa = nullptr;        // 6 * n_pad floats: x | y | z | nx | ny | nz
   uint32_t* enabled = nullptr; // n_pad/32 words
   uint32_t* valid = nullptr;
+  // exact clouds only (rsc_cloud_create_f64_exact): the caller's float64 coordinates in the caller's AoS layout [3 n];
+  // every float64 decision and fit reads them, the float32 SoA above is their rounding
+  double* xyz64 = nullptr;
+  double* nrm64 = nullptr;
+  bool exact() const { return xyz64 != nullptr; }
   float pmax = 0.f;            // max |p| over the cloud (guard-band scale)
   float nmax = 1.f;            // max |n| over the cloud
   // chunked upload in flight: chunk i is usable once chunk_ev[i] has fired on the copy stream
@@ -207,6 +221,8 @@ inline PointSet view_cloud(const rsc_cloud* c) {
   ps.valid = c->valid;
   ps.n = c->n;
   ps.n_pad = c->n_pad;
+  ps.xyz64 = c->xyz64;
+  ps.nrm64 = c->nrm64;
   return ps;
 }
 
@@ -222,6 +238,9 @@ inline PointSet view_subset(const rsc_subset* s) {
   ps.valid = s->valid;
   ps.n = s->m;
   ps.n_pad = s->m_pad;
+  ps.xyz64 = s->xyz64;
+  ps.nrm64 = s->nrm64;
+  if (s->xyz64) ps.map = s->idx;
   return ps;
 }
 

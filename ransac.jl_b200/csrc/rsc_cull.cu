@@ -128,6 +128,11 @@ __global__ void morton_gather_kernel(const float* __restrict__ soa, int64_t n_pa
   for (int f = 0; f < 6; ++f) msoa[f * n_pad + i] = real ? soa[f * n_pad + j] : 0.f;
 }
 
+__global__ void widen_u32_kernel(const uint32_t* __restrict__ in, int64_t n, int64_t* __restrict__ out) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) out[i] = (int64_t)in[i];
+}
+
 // one warp per tile of `tile_pts` points: centre of the bounding box, radius = largest distance of a point to it
 // (rounded up)
 __global__ void __launch_bounds__(256) tile_sphere_kernel(const float* __restrict__ X, const float* __restrict__ Y,
@@ -215,16 +220,15 @@ __device__ __forceinline__ void load_rec(const float* __restrict__ rec, int slot
 }
 
 // the FP64 decision of one in-band pair; out of line so that its registers (and code) do not weigh on the FP32 loop
-__device__ __noinline__ uint32_t cull_exact(const rsc_cand* __restrict__ cp, const Thresh* th, float px, float py, float pz, float nx,
-                                            float ny, float nz) {
+__device__ __noinline__ uint32_t cull_exact(const rsc_cand* __restrict__ cp, const Thresh* th, const PointSet* ps, int64_t j) {
   const rsc_cand c = *cp;
   ex::ConeTrig tr{1.0, 0.0};
   if (c.type == RSC_CONE) {
     tr.ct = cos(-c.p[6] / 2);
     tr.st = sin(-c.p[6] / 2);
   }
-  const ex::V3 p = {(double)px, (double)py, (double)pz};
-  const ex::V3 n = {(double)nx, (double)ny, (double)nz};
+  ex::V3 p, n;
+  ex::point64(*ps, j, &p, &n);
   return ex::compat(c, tr, *th, p, n) ? 1u : 0u;
 }
 
@@ -288,7 +292,7 @@ __device__ __forceinline__ void cull_narrow(const CullArgs& a, const float* __re
           if (ps < a.pcap) {
             a.pairs[ps] = make_uint2((uint32_t)sslot, (uint32_t)j);
           } else {  // queue full or switched off: the reference's float64 decision right here
-            ok = cull_exact(a.cands + a.orig[sslot], &a.th, px, py, pz, nx, ny, nz);
+            ok = cull_exact(a.cands + a.orig[sslot], &a.th, &a.ps, j);
             ++*n_exact;
           }
         }
@@ -459,7 +463,7 @@ __global__ void __launch_bounds__(256) cull_pair_kernel(const __grid_constant__ 
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     const uint2 e = a.pairs[i];
     const int64_t j = (int64_t)e.y;
-    if (cull_exact(a.cands + a.orig[e.x], &a.th, a.ps.x[j], a.ps.y[j], a.ps.z[j], a.ps.nx[j], a.ps.ny[j], a.ps.nz[j])) {
+    if (cull_exact(a.cands + a.orig[e.x], &a.th, &a.ps, j)) {
       const int o = a.orig[e.x];
       atomicAdd(a.cv + o, 1);
       if ((a.ps.enabled[j >> 5] >> (j & 31)) & 1u) atomicAdd(a.ce + o, 1);
@@ -486,6 +490,16 @@ static int32_t cull_prepare(rsc_cloud* cloud, cudaStream_t st) {
     cudaFree(c.msoa);
     c.msoa = nullptr;
     return fail_cuda(ctx, e, "score_culled: cudaMalloc");
+  }
+  if (cloud->exact()) {  // the map of the Morton copy into the float64 coordinates
+    e = cudaMalloc(&c.perm64, (size_t)cloud->n * sizeof(int64_t));
+    if (e != cudaSuccess) {
+      cudaFree(c.msoa), cudaFree(c.tiles);
+      c.msoa = nullptr, c.tiles = nullptr;
+      return fail_cuda(ctx, e, "score_culled: cudaMalloc");
+    }
+    widen_u32_kernel<<<(unsigned)((cloud->n + 255) / 256), 256, 0, st>>>(c.perm, cloud->n, c.perm64);
+    RSC_CUDA(ctx, cudaGetLastError());
   }
   morton_gather_kernel<<<(unsigned)((cloud->n_pad + 255) / 256), 256, 0, st>>>(cloud->soa, cloud->n_pad, c.perm, cloud->n, c.msoa);
   RSC_CUDA(ctx, cudaGetLastError());
@@ -545,9 +559,12 @@ int32_t cull_enqueue(rsc_ctx* ctx, const rsc_cloud* cloud, const PointSet& ps, c
   unsigned long long* ctr = reinterpret_cast<unsigned long long*>(b + o_ctr);
   uint32_t* ctr32 = reinterpret_cast<uint32_t*>(ctr + 2);  // pn, work, hist[5], cursor[5]
   RSC_CUDA(ctx, cudaMemsetAsync(ctr, 0, 96, st));
+  if (cloud->exact() && !ps.xyz64) return fail(ctx, RSC_E_STATE, "score_culled: a point set of an exact cloud lacks its float64 coordinates");
+  Thresh thx = th;
+  thx.exact_in = cloud->exact();
   cull_hist_kernel<<<(C_cap + 255) / 256, 256, 0, st>>>(d_cands, C_cap, d_C, ctr32 + 2);
   RSC_CUDA(ctx, cudaGetLastError());
-  cull_compile_kernel<<<(C_cap + 127) / 128, 128, 0, st>>>(d_cands, C_cap, d_C, th, cloud->pmax, cloud->nmax, ctr32 + 2, ctr32 + 7, d_rec,
+  cull_compile_kernel<<<(C_cap + 127) / 128, 128, 0, st>>>(d_cands, C_cap, d_C, thx, cloud->pmax, cloud->nmax, ctr32 + 2, ctr32 + 7, d_rec,
                                                           d_col, d_orig);
   RSC_CUDA(ctx, cudaGetLastError());
   CullArgs a;
@@ -566,7 +583,7 @@ int32_t cull_enqueue(rsc_ctx* ctx, const rsc_cloud* cloud, const PointSet& ps, c
   a.cands_per_range = per;
   a.nranges = (C_cap + per - 1) / per;
   a.rec = d_rec, a.col = d_col, a.orig = d_orig, a.cands = d_cands, a.d_C = d_C;
-  a.th = th;
+  a.th = thx;
   a.C = C_cap;
   a.cv = cv, a.ce = ce;
   a.stats = d_stats ? d_stats : ctr;
@@ -622,6 +639,7 @@ int32_t loop_score_new(rsc_ctx* ctx, rsc_cloud* cloud, rsc_subset& sub, const Po
   cps.nx = sub.csoa + 3 * sub.m_pad, cps.ny = sub.csoa + 4 * sub.m_pad, cps.nz = sub.csoa + 5 * sub.m_pad;
   cps.enabled = sub.cen, cps.valid = nullptr;
   cps.n = sub.m, cps.n_pad = sub.m_pad;
+  cps.xyz64 = sub.xyz64, cps.nrm64 = sub.nrm64, cps.map = sub.cidx;
   if (int32_t rc = cull_enqueue(ctx, cloud, cps, reinterpret_cast<const float4*>(sub.ctiles), th, d_cands, n_new, nullptr, cv, ce, nullptr, st))
     return rc;
   if (d_ovf) RSC_CUDA(ctx, cudaMemsetAsync(d_ovf, 0, 4, st));  // nothing can overflow: pairs beyond the queue are decided inline
@@ -663,6 +681,7 @@ static int32_t score_culled_impl(rsc_cloud* cloud, const rsc_params* params, con
     ps.nx = m + 3 * cloud->n_pad, ps.ny = m + 4 * cloud->n_pad, ps.nz = m + 5 * cloud->n_pad;
     ps.enabled = cloud->cells.en_sorted, ps.valid = nullptr;
     ps.n = cloud->n, ps.n_pad = cloud->n_pad;
+    ps.xyz64 = cloud->xyz64, ps.nrm64 = cloud->nrm64, ps.map = cloud->cells.perm64;
     tiles = reinterpret_cast<const float4*>(cloud->cells.tiles);
   } else {
     if ((size_t)subset_id >= cloud->subsets.size() || !cloud->subsets[subset_id].soa)
@@ -673,6 +692,7 @@ static int32_t score_culled_impl(rsc_cloud* cloud, const rsc_params* params, con
     ps.nx = sub.csoa + 3 * sub.m_pad, ps.ny = sub.csoa + 4 * sub.m_pad, ps.nz = sub.csoa + 5 * sub.m_pad;
     ps.enabled = sub.cen, ps.valid = nullptr;
     ps.n = sub.m, ps.n_pad = sub.m_pad;
+    ps.xyz64 = sub.xyz64, ps.nrm64 = sub.nrm64, ps.map = sub.cidx;
     tiles = reinterpret_cast<const float4*>(sub.ctiles);
   }
   const Thresh th = make_thresh(params);

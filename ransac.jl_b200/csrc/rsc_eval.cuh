@@ -34,6 +34,14 @@ __host__ __device__ constexpr float kappa(int type) {
   return type == RSC_PLANE ? 8.f : type == RSC_SPHERE ? 16.f : type == RSC_CYLINDER ? 16.f : 20.f;  // both cone forms: 20
 }
 
+// Input-rounding term of an exact cloud (DESIGN.md section 4): the float32 point is the rounding of the caller's
+// float64 one, |dp| <= (u/2) pmax and |dn| <= (u/2) nmax, which moves the margin the kernel evaluates by at most
+// (u/2) L (plane), (3/2) u L (sphere, cylinder) or (1 + 1/sqrt 2) u L (both cone forms).  Like kappa, kappa_in
+// is twice that bound in units of u L.
+__host__ __device__ constexpr float kappa_in(int type) {
+  return type == RSC_PLANE ? 1.f : type == RSC_SPHERE ? 3.f : type == RSC_CYLINDER ? 3.f : 4.f;
+}
+
 // column type of a candidate: its public type, except cones wider than 120 degrees (cos(opang/2) < 1/2)
 __host__ __device__ inline int col_type(const rsc_cand& c) {
   if (c.type != RSC_CONE) return c.type;
@@ -523,7 +531,7 @@ __device__ inline void compile_record(const rsc_cand& c, int col, const Thresh& 
       break;
     }
   }
-  double b = (double)kappa(c.type) * u * L;
+  double b = (double)(th.exact_in ? kappa(c.type) + kappa_in(c.type) : kappa(c.type)) * u * L;
   r[kBandField] = (float)(b * 1.0000002);  // round the band up, never down
 }
 

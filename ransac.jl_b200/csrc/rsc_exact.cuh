@@ -32,6 +32,19 @@ __device__ __forceinline__ V3 cross(V3 a, V3 b) {
           sub(mul(a.x, b.y), mul(a.y, b.x))};
 }
 
+// The float64 coordinates of point j of a set: on an exact cloud the caller's own, else the float32 ones widened
+// (which is what the reference sees for a Float32 cloud).  Padding points (j >= n) are zero either way.
+__device__ __forceinline__ void point64(const PointSet& ps, int64_t j, V3* p, V3* n) {
+  if (ps.xyz64 && j < ps.n) {
+    const int64_t i = 3 * (ps.map ? ps.map[j] : j);
+    *p = V3{ps.xyz64[i], ps.xyz64[i + 1], ps.xyz64[i + 2]};
+    *n = V3{ps.nrm64[i], ps.nrm64[i + 1], ps.nrm64[i + 2]};
+  } else {
+    *p = V3{(double)ps.x[j], (double)ps.y[j], (double)ps.z[j]};
+    *n = V3{(double)ps.nx[j], (double)ps.ny[j], (double)ps.nz[j]};
+  }
+}
+
 // cos/sin of -opang/2 for the cone's Rodrigues matrix
 struct ConeTrig {
   double ct, st;

@@ -102,9 +102,9 @@ __global__ void __launch_bounds__(256) extract_fix_kernel(const __grid_constant_
   const uint32_t n = *a.qn;
   const int type = a.cand.type;  // public type: thresholds
   auto decide = [&](uint32_t pt) {
-    const bool ok = ex::compat(a.cand, a.trig, a.th,
-                               ex::V3{(double)a.ps.x[pt], (double)a.ps.y[pt], (double)a.ps.z[pt]},
-                               ex::V3{(double)a.ps.nx[pt], (double)a.ps.ny[pt], (double)a.ps.nz[pt]});
+    ex::V3 P, N;
+    ex::point64(a.ps, pt, &P, &N);
+    const bool ok = ex::compat(a.cand, a.trig, a.th, P, N);
     const uint32_t bit = 1u << (pt & 31);
     if (ok)
       atomicOr(a.inl + (pt >> 5), bit);
@@ -219,6 +219,7 @@ int32_t refit_mask_enqueue(rsc_cloud* cloud, const Thresh& th, const rsc_cand& c
   ExtractArgs a;
   a.ps = view_cloud(cloud);
   a.th = th;
+  a.th.exact_in = cloud->exact();
   a.cand = cand;
   a.trig.ct = cos(-cand.p[6] / 2);
   a.trig.st = sin(-cand.p[6] / 2);

@@ -412,6 +412,8 @@ struct GatherSrc {
   const double* P;   // explicit coordinates S x k x 3 (used when soa == nullptr)
   const double* N;
   const float* G;    // sharded storage: [S][k][6] float32 x y z nx ny nz gathered from the owning ranks
+  const double* xyz64 = nullptr;  // exact clouds: the float64 coordinates the drawn points are read from instead of soa
+  const double* nrm64 = nullptr;
 };
 
 // sharded storage: every rank writes the bit patterns of the drawn points it owns (zeros for the others);
@@ -567,6 +569,12 @@ __global__ void __launch_bounds__(128) fit_kernel(GatherSrc src, const int64_t* 
       const float* g = src.G + ((size_t)s * fk + q) * 6;
       p[q] = D3{(double)g[0], (double)g[1], (double)g[2]};
       n[q] = D3{(double)g[3], (double)g[4], (double)g[5]};
+    }
+  } else if (src.xyz64) {
+    _Pragma("unroll") for (int q = 0; q < fk; ++q) {
+      const int64_t i = 3 * idx[(size_t)s * fk + q];
+      p[q] = D3{__ldg(src.xyz64 + i), __ldg(src.xyz64 + i + 1), __ldg(src.xyz64 + i + 2)};
+      n[q] = D3{__ldg(src.nrm64 + i), __ldg(src.nrm64 + i + 1), __ldg(src.nrm64 + i + 2)};
     }
   } else if (src.soa) {
     _Pragma("unroll") for (int q = 0; q < fk; ++q) {
@@ -949,7 +957,11 @@ int32_t fit_enqueue(rsc_ctx* ctx, rsc_cloud* cloud, int mode, const rsc_params* 
   if (mode != 0) {
     src.soa = cloud->soa;
     src.n_pad = cloud->n_pad;
+    src.xyz64 = cloud->xyz64;
+    src.nrm64 = cloud->nrm64;
   }
+  if (mode == 3 && cloud->exact())
+    return fail(ctx, RSC_E_STATE, "fit: the cell sampler (octree quantisation) does not support exact clouds yet");
   if (mode == 2 && (rc = build_select_index(cloud, st, &boff, &nblk, &nen))) return rc;
   CellsView cv;
   if (mode == 3 && (rc = build_cells_index(cloud, st, cum, &cv))) return rc;

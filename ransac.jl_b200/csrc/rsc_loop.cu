@@ -190,7 +190,7 @@ __global__ void newly_mask_kernel(uint32_t* __restrict__ old_en, const uint32_t*
 __global__ void newly_gather_capped_kernel(const uint32_t* __restrict__ old_en, const uint32_t* __restrict__ new_en, int64_t words,
                                            const unsigned long long* __restrict__ offs, const unsigned long long* __restrict__ total,
                                            const float* __restrict__ soa, int64_t m_pad, float* __restrict__ out, int64_t cap,
-                                           int32_t* __restrict__ over) {
+                                           int32_t* __restrict__ over, const int64_t* __restrict__ idx, int64_t* __restrict__ out_idx) {
   const int64_t w = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (w == 0) *over = (*total > (unsigned long long)cap) ? 1 : 0;
   if (w >= words) return;
@@ -203,6 +203,7 @@ __global__ void newly_gather_capped_kernel(const uint32_t* __restrict__ old_en, 
     if (o < (unsigned long long)cap) {
 #pragma unroll
       for (int f = 0; f < 6; ++f) out[f * cap + o] = soa[f * m_pad + j];
+      if (out_idx) out_idx[o] = idx[j];  // exact clouds: the scratch set's map into the float64 coordinates
     }
     ++o;
   }
@@ -525,8 +526,13 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
         RUN_CUDA(ls.nscratch.ensure((size_t)6 * cap * 4));
         RUN_CUDA(ls.nvalid.ensure((size_t)(cap / 32) * 4));
         RUN_CUDA(cudaMemsetAsync(ls.nscratch.p, 0, (size_t)6 * cap * 4, st));
-        newly_gather_capped_kernel<<<(unsigned)((sl_words + 255) / 256), 256, 0, st>>>(old_sl, sps.enabled, sl_words, woff, wtot, sps.x,
-                                                                                      sps.y - sps.x, ls.nscratch.as<float>(), cap, d_over);
+        if (sps.map) {  // (entries past the gathered count stay 0: padding lanes may still look their point up)
+          RUN_CUDA(ls.nidx.ensure((size_t)cap * sizeof(int64_t)));
+          RUN_CUDA(cudaMemsetAsync(ls.nidx.p, 0, (size_t)cap * sizeof(int64_t), st));
+        }
+        newly_gather_capped_kernel<<<(unsigned)((sl_words + 255) / 256), 256, 0, st>>>(
+            old_sl, sps.enabled, sl_words, woff, wtot, sps.x, sps.y - sps.x, ls.nscratch.as<float>(), cap, d_over, sps.map,
+            sps.map ? ls.nidx.as<int64_t>() : nullptr);
         RUN_CUDA(cudaGetLastError());
         fill_valid_dev_kernel<<<(unsigned)((cap / 32 + 255) / 256), 256, 0, st>>>(ls.nvalid.as<uint32_t>(), wtot, cap / 32);
         RUN_CUDA(cudaGetLastError());
@@ -534,6 +540,7 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
         dps.x = b, dps.y = b + cap, dps.z = b + 2 * cap, dps.nx = b + 3 * cap, dps.ny = b + 4 * cap, dps.nz = b + 5 * cap;
         dps.enabled = dps.valid = ls.nvalid.as<uint32_t>();
         dps.n = dps.n_pad = cap;
+        if (sps.map) dps.map = ls.nidx.as<int64_t>();
       }
       auto mask_form = [&]() -> cudaError_t {
         newly_mask_kernel<<<(unsigned)((swords + 255) / 256), 256, 0, st>>>(ls.olden.as<uint32_t>(), sub.enabled, swords);

@@ -112,9 +112,11 @@ static __global__ void newly_count_kernel(const uint32_t* __restrict__ old_en, c
 }
 
 // gather the newly disabled subset points into a compact SoA scratch set
+// (exact clouds: idx / out_idx non-null, the cloud index of every gathered point, the map of the scratch set)
 static __global__ void newly_gather_kernel(const uint32_t* __restrict__ old_en, const uint32_t* __restrict__ new_en, int64_t words,
                                     const unsigned long long* __restrict__ offs, const float* __restrict__ soa, int64_t m_pad,
-                                    float* __restrict__ out, int64_t out_pad) {
+                                    float* __restrict__ out, int64_t out_pad, const int64_t* __restrict__ idx,
+                                    int64_t* __restrict__ out_idx) {
   const int64_t w = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (w >= words) return;
   uint32_t bits = old_en[w] & ~new_en[w];
@@ -125,6 +127,7 @@ static __global__ void newly_gather_kernel(const uint32_t* __restrict__ old_en, 
     const int64_t j = w * 32 + b;
 #pragma unroll
     for (int f = 0; f < 6; ++f) out[f * out_pad + o] = soa[f * m_pad + j];
+    if (out_idx) out_idx[o] = idx[j];
     ++o;
   }
 }
@@ -196,7 +199,7 @@ struct Store {
 // device buffers per run cost 10-25 ms of a 40 ms loop)
 struct LoopScratch {
   Store store;
-  DevBuf newcnt, hostio, olden, nscratch, nvalid, nmeta, lvbuf, prog, ntiles;
+  DevBuf newcnt, hostio, olden, nscratch, nidx, nvalid, nmeta, lvbuf, prog, ntiles;
 };
 
 }  // namespace rsc

@@ -347,6 +347,7 @@ extern "C" int32_t rsc_refit_lsq(rsc_cloud* cloud, const rsc_params* params, con
   if (!params || !cand || !out) return fail(ctx, RSC_E_ARG, "refit_lsq: null params/candidate/out");
   if (cand->type < 0 || cand->type >= RSC_NTYPES) return fail(ctx, RSC_E_ARG, "refit_lsq: unknown shape type");
   if (!(band > 0) || !isfinite(band)) return fail(ctx, RSC_E_ARG, "refit_lsq: band must be positive");
+  if (cloud->exact()) return fail(ctx, RSC_E_STATE, "refit_lsq: the least-squares refit does not support exact clouds yet");
   RSC_CUDA(ctx, cudaSetDevice(ctx->device));
   if (int32_t rc = cloud_ready(cloud)) return rc;
   *out = *cand;

@@ -150,6 +150,7 @@ void cells_release(rsc_cloud* cloud) {
   rsc_cells& c = cloud->cells;
   if (c.codes) cudaFree(c.codes);
   if (c.perm) cudaFree(c.perm);
+  if (c.perm64) cudaFree(c.perm64);
   if (c.inv) cudaFree(c.inv);
   if (c.leafdepth) cudaFree(c.leafdepth);
   if (c.en_sorted) cudaFree(c.en_sorted);

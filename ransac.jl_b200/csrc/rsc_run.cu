@@ -111,7 +111,7 @@ void loop_scratch_free(rsc_ctx* ctx) {
   LoopScratch* ls = static_cast<LoopScratch*>(ctx->loop_scratch);
   if (!ls) return;
   ls->store.release();
-  ls->newcnt.release(), ls->hostio.release(), ls->olden.release(), ls->nscratch.release(), ls->nvalid.release(), ls->nmeta.release();
+  ls->newcnt.release(), ls->hostio.release(), ls->olden.release(), ls->nscratch.release(), ls->nidx.release(), ls->nvalid.release(), ls->nmeta.release();
   ls->lvbuf.release(), ls->prog.release(), ls->ntiles.release();
   delete ls;
   ctx->loop_scratch = nullptr;
@@ -150,6 +150,7 @@ int32_t rsc_ctx_set_allreduce(rsc_ctx* ctx, rsc_allreduce_fn fn, void* user) {
 
 int32_t rsc_cloud_set_range(rsc_cloud* cloud, int64_t lo, int64_t hi) {
   if (!cloud) return RSC_E_ARG;
+  if (cloud->exact()) return fail(cloud->ctx, RSC_E_STATE, "set_range: ranged (replicated multi-GPU) runs do not support exact clouds yet");
   // 2048 = points per refit CTA (rsc_extract.cu); lo == hi is an empty rank (clouds smaller than 2048 x ranks)
   if (lo < 0 || hi > cloud->n_pad || lo > hi || (lo % 2048 && lo != cloud->n) || (hi % 2048 && hi != cloud->n_pad && hi != cloud->n))
     return fail(cloud->ctx, RSC_E_ARG, "set_range: range bounds must be multiples of 2048 points (or the cloud size)");
@@ -205,6 +206,9 @@ int32_t rsc_ransac_run(rsc_cloud* cloud, const rsc_params* p, uint64_t seed, rsc
     return fail(ctx, RSC_E_ARG, "ransac_run: extract_s/terminate_s must be RSC_S_*");
   if (cloud->subsets.empty() || !cloud->subsets[0].soa)
     return fail(ctx, RSC_E_STATE, "ransac_run: subset 1 is not uploaded (rsc_cloud_set_subset(cloud, 0, ...))");
+  if (cloud->exact() && (p->compat_flags & (RSC_SAMPLER_OCTREE | RSC_SCORE_PROGRESSIVE | RSC_REFIT_LSQ | RSC_EXTRACT_BITMAP)))
+    return fail(ctx, RSC_E_STATE,
+                "ransac_run: RSC_SAMPLER_OCTREE / RSC_SCORE_PROGRESSIVE / RSC_REFIT_LSQ / RSC_EXTRACT_BITMAP do not support exact clouds yet");
   RSC_CUDA(ctx, cudaSetDevice(ctx->device));
   if (int32_t rcr = cloud_ready(cloud)) return rcr;
   cudaStream_t st = ctx->stream;
@@ -571,8 +575,10 @@ int32_t rsc_ransac_run(rsc_cloud* cloud, const rsc_params* p, uint64_t seed, rsc
             RUN_CUDA(nscratch.ensure((size_t)6 * sp * 4));
             RUN_CUDA(nvalid.ensure((size_t)(sp / 32) * 4));
             RUN_CUDA(cudaMemsetAsync(nscratch.p, 0, (size_t)6 * sp * 4, st));
+            if (cloud->exact()) RUN_CUDA(ls.nidx.ensure((size_t)sp * sizeof(int64_t)));
             newly_gather_kernel<<<(unsigned)((swords + 255) / 256), 256, 0, st>>>(olden.as<uint32_t>(), sub_en, swords, woff, sub_soa,
-                                                                                   sub.m_pad, nscratch.as<float>(), sp);
+                                                                                   sub.m_pad, nscratch.as<float>(), sp, sub.idx,
+                                                                                   cloud->exact() ? ls.nidx.as<int64_t>() : nullptr);
             RUN_CUDA(cudaGetLastError());
             fill_valid_words_kernel<<<(unsigned)((sp / 32 + 255) / 256), 256, 0, st>>>(nvalid.as<uint32_t>(), (int64_t)nnew_dis, sp / 32);
             RUN_CUDA(cudaGetLastError());
@@ -583,6 +589,7 @@ int32_t rsc_ransac_run(rsc_cloud* cloud, const rsc_params* p, uint64_t seed, rsc
             ps.valid = nvalid.as<uint32_t>();
             ps.n = (int64_t)nnew_dis;
             ps.n_pad = sp;
+            if (cloud->exact()) ps.xyz64 = cloud->xyz64, ps.nrm64 = cloud->nrm64, ps.map = ls.nidx.as<int64_t>();
             // replicated on every rank (the scratch set is tiny): no all-reduce needed
             // enabled == valid on the scratch set: the enabled-gated count (kept for every type) is the hit count
             // a large store (cell sampler): most stored candidates are nowhere near the extracted shape -- and the dense

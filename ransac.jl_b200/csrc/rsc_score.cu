@@ -450,8 +450,9 @@ __global__ void __launch_bounds__(256) fixup_pair_kernel(const __grid_constant__
       }
     }
     const uint32_t pt = pr.point;
-    const bool ok = ex::compat(c, tr, a.th, ex::V3{(double)a.ps.x[pt], (double)a.ps.y[pt], (double)a.ps.z[pt]},
-                               ex::V3{(double)a.ps.nx[pt], (double)a.ps.ny[pt], (double)a.ps.nz[pt]});
+    ex::V3 P, N;
+    ex::point64(a.ps, pt, &P, &N);
+    const bool ok = ex::compat(c, tr, a.th, P, N);
     if (ok != used) apply_flip(a, cand, c.type, slot_of[cand], pt, ok);
   }
 }
@@ -742,14 +743,17 @@ int32_t score_enqueue(rsc_ctx* ctx, const rsc_cloud* cloud, const PointSet& ps, 
   RSC_CUDA(ctx, ctx->pairs.ensure(ctx->wl_cap * 8));
   RSC_CUDA(ctx, cudaMemsetAsync(ctx->wl_count.p, 0, 2 * sizeof(uint32_t), st));
 
-  compile_kernel<<<1, 1024, 0, st>>>(d_cands, C, th, L.spcs, cslots, ncols, cloud->pmax, cloud->nmax, d_bounds,
+  if (cloud->exact() && !ps.xyz64) return fail(ctx, RSC_E_STATE, "score: a point set of an exact cloud lacks its float64 coordinates");
+  Thresh thx = th;
+  thx.exact_in = cloud->exact();
+  compile_kernel<<<1, 1024, 0, st>>>(d_cands, C, thx, L.spcs, cslots, ncols, cloud->pmax, cloud->nmax, d_bounds,
                                      ctx->rec.as<float>(), ctx->orig.as<int32_t>(),
                                      ctx->slot_of.as<int32_t>(), ctx->blktab.as<BlockTab>());
   RSC_CUDA(ctx, cudaGetLastError());
 
   ScoreArgs a;
   a.ps = ps;
-  a.th = th;
+  a.th = thx;
   a.rec = ctx->rec.as<float>();
   a.orig = ctx->orig.as<int32_t>();
   a.tab = ctx->blktab.as<BlockTab>();
@@ -899,7 +903,9 @@ __global__ void __launch_bounds__(256) audit_margin_kernel(PointSet ps, Thresh t
 
 int32_t audit_margins(rsc_ctx* ctx, const rsc_cloud* cloud, const PointSet& ps, const Thresh& th, const rsc_cand* d_cands, int32_t C,
                       int64_t p0, int64_t np, float* d_out, float* d_rec, int32_t* d_cols, unsigned long long* d_diffs, cudaStream_t st) {
-  audit_compile_kernel<<<(C + 127) / 128, 128, 0, st>>>(d_cands, C, th, cloud->pmax, cloud->nmax, d_rec, d_cols);
+  Thresh thx = th;
+  thx.exact_in = cloud->exact();
+  audit_compile_kernel<<<(C + 127) / 128, 128, 0, st>>>(d_cands, C, thx, cloud->pmax, cloud->nmax, d_rec, d_cols);
   RSC_CUDA(ctx, cudaGetLastError());
   audit_margin_kernel<<<dim3((unsigned)((np + 255) / 256), (unsigned)C), 256, 0, st>>>(ps, th, d_rec, d_cols, p0, np, d_out, d_diffs);
   RSC_CUDA(ctx, cudaGetLastError());

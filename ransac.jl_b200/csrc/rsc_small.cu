@@ -56,14 +56,15 @@ __global__ void small_compile_kernel(const __grid_constant__ SmallArgs a) {
 }
 
 // the rare path, out of line so that it does not cost the streaming loop registers
-__device__ __noinline__ bool small_exact(const rsc_cand* c, const Thresh& th, float px, float py, float pz, float nx, float ny,
-                                         float nz) {
+__device__ __noinline__ bool small_exact(const rsc_cand* c, const Thresh& th, const PointSet& ps, int64_t p) {
   ex::ConeTrig tr{1.0, 0.0};
   if (c->type == RSC_CONE) {
     tr.ct = cos(-c->p[6] / 2);
     tr.st = sin(-c->p[6] / 2);
   }
-  return ex::compat(*c, tr, th, ex::V3{(double)px, (double)py, (double)pz}, ex::V3{(double)nx, (double)ny, (double)nz});
+  ex::V3 P, N;
+  ex::point64(ps, p, &P, &N);
+  return ex::compat(*c, tr, th, P, N);
 }
 
 __global__ void __launch_bounds__(kSmallThreads) small_score_kernel(const __grid_constant__ SmallArgs a) {
@@ -102,7 +103,7 @@ __global__ void __launch_bounds__(kSmallThreads) small_score_kernel(const __grid
         const int pt = public_type(col);
         const float m = eval_any(col, r, px, py, pz, nx, ny, nz, a.th.eps[pt], a.th.cosa[pt]);
         bool ok = m < 0.f;
-        if (va && !(fabsf(m) > r[kBandField])) ok = small_exact(a.cands + c0 + c, a.th, px, py, pz, nx, ny, nz);
+        if (va && !(fabsf(m) > r[kBandField])) ok = small_exact(a.cands + c0 + c, a.th, a.ps, p);
         const unsigned be = __ballot_sync(0xffffffffu, ok && en);
         const unsigned bv = __ballot_sync(0xffffffffu, ok && va);
         if (lane == 0) {
@@ -127,11 +128,13 @@ int32_t score_small_enqueue(rsc_ctx* ctx, const rsc_cloud* cloud, const PointSet
   RSC_CUDA(ctx, cudaMemsetAsync(d_cv, 0, (size_t)c_cap * 4, st));
   RSC_CUDA(ctx, cudaMemsetAsync(d_ce, 0, (size_t)c_cap * 4, st));
   if (ps.n_pad <= 0) return RSC_OK;
+  if (cloud->exact() && !ps.xyz64) return fail(ctx, RSC_E_STATE, "score: a point set of an exact cloud lacks its float64 coordinates");
   const size_t o_col = ((size_t)c_cap * kRecFields * 4 + 255) / 256 * 256;
   RSC_CUDA(ctx, ctx->smallbuf.ensure(o_col + (size_t)c_cap * 4));
   SmallArgs a;
   a.ps = ps;
   a.th = th;
+  a.th.exact_in = cloud->exact();
   a.cands = d_cands;
   a.d_count = d_count;
   a.c_host = c_cap;

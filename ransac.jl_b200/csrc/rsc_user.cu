@@ -169,6 +169,7 @@ static RscUserPoints to_user_points(const PointSet& ps) {
   RscUserPoints u;
   u.x = ps.x, u.y = ps.y, u.z = ps.z, u.nx = ps.nx, u.ny = ps.ny, u.nz = ps.nz;
   u.enabled = ps.enabled, u.valid = ps.valid, u.n = ps.n, u.n_pad = ps.n_pad;
+  u.xyz64 = ps.xyz64, u.nrm64 = ps.nrm64, u.map = reinterpret_cast<const long long*>(ps.map);
   return u;
 }
 
@@ -205,6 +206,8 @@ int32_t user_fit_enqueue(rsc_ctx* ctx, const FitOrder& fo, int pos, const rsc_cl
   memset(&a, 0, sizeof(a));
   a.soa = cloud->soa;
   a.n_pad = cloud->n_pad;
+  a.xyz64 = cloud->xyz64;
+  a.nrm64 = cloud->nrm64;
   a.idx = reinterpret_cast<const long long*>(idx);
   a.S = S, a.np = np, a.npos = fo.n, a.pos = pos, a.type = fo.type[pos], a.nk = fo.nk[pos];
   for (int q = 0; q < 8; ++q) a.k[q] = fo.k[pos][q];

@@ -27,6 +27,9 @@ struct RscUserPoints {  // = rsc::PointSet
   const unsigned* valid;    // 1 for real points, 0 for padding
   long long n;
   long long n_pad;  // multiple of 512
+  const double* xyz64;    // exact clouds: the caller's float64 coordinates (AoS), point j at 3 * (map ? map[j] : j)
+  const double* nrm64;
+  const long long* map;
 };
 
 struct RscUserCand {  // = rsc_cand (64 bytes)
@@ -52,6 +55,8 @@ struct RscUserScoreArgs {
 struct RscUserFitArgs {
   const float* soa;      // the cloud: x | y | z | nx | ny | nz rows of n_pad floats
   long long n_pad;
+  const double* xyz64;   // exact clouds: the caller's float64 coordinates (AoS [3 n]), read instead of soa
+  const double* nrm64;
   const long long* idx;  // [S][np] drawn indices; a row starting with -1 is a failed sample
   int S, np;
   int npos, pos;         // positions in the fit order / this type's position
@@ -78,11 +83,23 @@ struct RscUserMaskArgs {
 __device__ bool rsc_user_compatible(const double p[7], int outwards, const double k[8], double x, double y, double z, double nx,
                                     double ny, double nz);
 
+// The float64 coordinates of point p of a set: an exact cloud's own, else the float32 ones widened
+__device__ __forceinline__ void rsc_user_point(const RscUserPoints& ps, long long p, double q[6]) {
+  if (ps.xyz64 && p < ps.n) {
+    const long long i = 3 * (ps.map ? ps.map[p] : p);
+    q[0] = ps.xyz64[i], q[1] = ps.xyz64[i + 1], q[2] = ps.xyz64[i + 2];
+    q[3] = ps.nrm64[i], q[4] = ps.nrm64[i + 1], q[5] = ps.nrm64[i + 2];
+  } else {
+    q[0] = __ldg(ps.x + p), q[1] = __ldg(ps.y + p), q[2] = __ldg(ps.z + p);
+    q[3] = __ldg(ps.nx + p), q[4] = __ldg(ps.ny + p), q[5] = __ldg(ps.nz + p);
+  }
+}
+
 // Counts (and masks) of C candidates of one user type: the transposed mapping of the small-batch scorer
 // (rsc_small.cu).  A thread owns a point; the CTA stages a chunk of candidate records in shared memory and reads
 // them as broadcasts; a (candidate, 32 points) group is one ballot, its POPC goes into a shared counter, and each
 // CTA adds one atomic per candidate.  Candidate chunks are spread over gridDim.y.  Every pair is decided once, in
-// float64, on the point's float32 coordinates widened to double.
+// float64, on the point's float32 coordinates widened to double (an exact cloud's float64 coordinates).
 // The device loop passes a mixed batch of built-in and user records whose size may stay on the device (a.d_count):
 // only records of a.type are scored, and their counts are ADDED where the built-in scorer has left zeros.
 extern "C" __global__ void __launch_bounds__(RSC_USER_THREADS) rsc_user_score_kernel(const RscUserScoreArgs a) {
@@ -105,11 +122,11 @@ extern "C" __global__ void __launch_bounds__(RSC_USER_THREADS) rsc_user_score_ke
       const unsigned live = __ldg(a.ps.enabled + (p >> 5)) & __ldg(a.ps.valid + (p >> 5));
       if (live == 0u) continue;  // warp-uniform: no enabled real point in this group
       const bool on = (live >> lane) & 1u;
-      const double x = __ldg(a.ps.x + p), y = __ldg(a.ps.y + p), z = __ldg(a.ps.z + p);
-      const double nx = __ldg(a.ps.nx + p), ny = __ldg(a.ps.ny + p), nz = __ldg(a.ps.nz + p);
+      double q[6];
+      rsc_user_point(a.ps, p, q);
       for (int c = 0; c < ct; ++c) {
         if (sc[c].type != a.type) continue;  // block-uniform: a record of another type in a mixed batch
-        const bool ok = on && rsc_user_compatible(sc[c].p, sc[c].outwards, sk, x, y, z, nx, ny, nz);
+        const bool ok = on && rsc_user_compatible(sc[c].p, sc[c].outwards, sk, q[0], q[1], q[2], q[3], q[4], q[5]);
         const unsigned b = __ballot_sync(0xffffffffu, ok);
         if (lane == 0 && b) {
           atomicAdd(&scount[c], __popc(b));
@@ -140,9 +157,14 @@ extern "C" __global__ void __launch_bounds__(RSC_USER_THREADS) rsc_user_mask_ker
        p += (long long)gridDim.x * RSC_USER_THREADS) {
     const unsigned live = __ldg(a.ps.enabled + (p >> 5)) & __ldg(a.ps.valid + (p >> 5));
     bool ok = false;
-    if ((live >> lane) & 1u)
+    if (((live >> lane) & 1u) && a.ps.xyz64) {  // (a live point is a real one: p < n)
+      const long long i = 3 * (a.ps.map ? a.ps.map[p] : p);
+      ok = rsc_user_compatible(sc.p, sc.outwards, sk, a.ps.xyz64[i], a.ps.xyz64[i + 1], a.ps.xyz64[i + 2], a.ps.nrm64[i],
+                               a.ps.nrm64[i + 1], a.ps.nrm64[i + 2]);
+    } else if ((live >> lane) & 1u) {
       ok = rsc_user_compatible(sc.p, sc.outwards, sk, __ldg(a.ps.x + p), __ldg(a.ps.y + p), __ldg(a.ps.z + p), __ldg(a.ps.nx + p),
                                __ldg(a.ps.ny + p), __ldg(a.ps.nz + p));
+    }
     const unsigned b = __ballot_sync(0xffffffffu, ok);
     if (lane == 0) a.inl[p >> 5] = b;
   }
@@ -166,8 +188,8 @@ extern "C" __global__ void __launch_bounds__(128) rsc_user_fit_kernel(const RscU
     for (int q = 0; q < a.np; ++q) {
       const long long i = a.idx[(long long)s * a.np + q];
       for (int d = 0; d < 3; ++d) {
-        P[q][d] = (double)__ldg(a.soa + d * a.n_pad + i);
-        N[q][d] = (double)__ldg(a.soa + (3 + d) * a.n_pad + i);
+        P[q][d] = a.xyz64 ? a.xyz64[3 * i + d] : (double)__ldg(a.soa + d * a.n_pad + i);
+        N[q][d] = a.xyz64 ? a.nrm64[3 * i + d] : (double)__ldg(a.soa + (3 + d) * a.n_pad + i);
       }
     }
     for (int j = 0; j < 7; ++j) p[j] = 0.0;
