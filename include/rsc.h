@@ -417,6 +417,24 @@ int32_t rsc_sample_fit_user(rsc_cloud* cloud, const rsc_params* params, const vo
 int32_t rsc_ransac_run_user(rsc_cloud* cloud, const rsc_params* params, const void* order, int32_t norder,
                             uint64_t seed, rsc_run** out);
 
+/* ---- normal estimation: oriented PCA normals of the k nearest neighbours (DESIGN.md section 8) ----------
+ * For float32 AoS coordinates xyz[3 n] (the layout rsc_cloud_create takes), N(i) is the k_eff = min(k, finite
+ * points) finite points j smallest in (d2(i, j), j) order, d2 = ((xj-xi)^2 + (yj-yi)^2) + (zj-zi)^2 in float64 of
+ * the float32 values, every operation rounded, no FMA; i itself is included.  The normal is the unit eigenvector of
+ * the smallest eigenvalue of the float64 covariance of N(i) (mean and sums in list order, divided by k_eff), or
+ * (0,0,0) when k_eff < 3, when the middle eigenvalue is <= 2^-40 times the largest (collinear or coincident
+ * neighbours), or when point i has a non-finite coordinate (such points appear in no list).  Sign: with a viewpoint v,
+ * n . (v - p_i) >= 0 (normals face the sensor); without one, the component of largest magnitude is positive (the
+ * first axis on ties).  The normalised float64 vector is rounded to float32 into nrm[3 n], ready for rsc_cloud_create.
+ * 3 <= k <= 32, 1 <= n < 2^31; host in / host out, synchronising.  Device memory: about 60 B per point, plus
+ * 8 n k bytes when nbr is asked for.  Cost: every point of the cells searched around a query is evaluated, so m
+ * coincident points (e.g. the (0,0,0) rows of missing depth) cost O(m^2) distances, and a lone outlier, whose search
+ * covers the whole box, costs n; results stay exact.
+ *   viewpoint: NULL or 3 doubles.  nbr: NULL or n x k int64, row i = N(i) in (d2, index) order, -1 beyond k_eff.
+ *   pairs: NULL or the number of (query, candidate) distances evaluated (for the benchmark). */
+int32_t rsc_estimate_normals(rsc_ctx* ctx, const float* xyz, int64_t n, int32_t k, const double* viewpoint,
+                             float* nrm, int64_t* nbr, int64_t* pairs);
+
 #ifdef __cplusplus
 }
 #endif

@@ -292,6 +292,28 @@ function loop_with_sets(pc::RANSACCloud, params, sets)
     extracted, extracted_at, iterations
 end
 
+# ---- normal estimation (rsc_estimate_normals) ------------------------------------------------------------
+"""
+    estimate_normals(vertices; k=16, viewpoint=nothing) -> Vector{SVector{3,Float32}}
+
+Oriented PCA normals of the `k` (3..32) nearest neighbours of every point, on the device (`rsc_estimate_normals`):
+with a `viewpoint` (the sensor of a single scan) every normal faces it, without one the component of largest
+magnitude is positive.  Non-finite points and collinear or coincident neighbourhoods get zero normals.  For a raw
+scan: `RANSACCloud(V, estimate_normals(V; viewpoint=s), 2)`.
+"""
+function estimate_normals(vertices::Vector{SVector{3,Float32}}; k::Integer=16, viewpoint=nothing)
+    nrm = Vector{SVector{3,Float32}}(undef, length(vertices))
+    vp = viewpoint === nothing ? nothing : Float64[viewpoint[1], viewpoint[2], viewpoint[3]]
+    GC.@preserve vertices nrm vp begin
+        check(ccall(fn(:rsc_estimate_normals), Int32,
+                    (Ptr{Cvoid}, Ptr{Float32}, Int64, Int32, Ptr{Float64}, Ptr{Float32}, Ptr{Int64}, Ptr{Int64}),
+                    context(), Ptr{Float32}(pointer(vertices)), length(vertices), k,
+                    vp === nothing ? Ptr{Float64}(C_NULL) : pointer(vp), Ptr{Float32}(pointer(nrm)),
+                    Ptr{Int64}(C_NULL), Ptr{Int64}(C_NULL)))
+    end
+    nrm
+end
+
 # ---- user-defined shapes on the device (include/rsc.h "user-defined shapes") -----------------------------
 """
     compile_user_shape(src::String) -> type id

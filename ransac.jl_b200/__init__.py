@@ -31,6 +31,7 @@ from .fitting import (
 )
 from .iterations import ransac
 from .jsonyaml import dict2nt, exportJSON, readconfig, toDict
+from .normals import estimate_normals
 from .params import (
     DEFAULT_PARAMETERS,
     DEFAULT_SHAPE_DICT,

@@ -145,6 +145,7 @@ SIGNATURES = {
     "rsc_sample_fit_user": (C.c_int32, [_P, C.POINTER(rsc_params), _P, C.c_int32, C.c_uint64, C.c_uint64, C.c_int32, _P, _P, _P,
                                         C.POINTER(C.c_int32)]),
     "rsc_ransac_run_user": (C.c_int32, [_P, C.POINTER(rsc_params), _P, C.c_int32, C.c_uint64, C.POINTER(_P)]),
+    "rsc_estimate_normals": (C.c_int32, [_P, _P, C.c_int64, C.c_int32, _P, _P, _P, C.POINTER(C.c_int64)]),
 }
 
 if not os.path.exists(LIB_PATH):

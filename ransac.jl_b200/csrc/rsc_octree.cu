@@ -14,30 +14,24 @@
 #include <cub/device/device_radix_sort.cuh>
 
 #include "rsc_common.cuh"
+#include "rsc_morton.cuh"
 
 namespace rsc {
 
-// order-preserving float <-> uint encoding for atomicMin/atomicMax
-__device__ __forceinline__ uint32_t f2ord(float f) {
-  const uint32_t u = __float_as_uint(f);
-  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-__host__ __device__ inline float ord2f(uint32_t o) {
-  const uint32_t u = (o & 0x80000000u) ? (o & 0x7fffffffu) : ~o;
-  float f;
-  memcpy(&f, &u, 4);
-  return f;
-}
-
-__global__ void __launch_bounds__(256) bbox_kernel(const float* __restrict__ soa, int64_t n, int64_t n_pad, uint32_t* __restrict__ mm) {
+__global__ void __launch_bounds__(256) bbox_kernel(const float* __restrict__ soa, int64_t n, int64_t n_pad, uint32_t* __restrict__ mm,
+                                                   bool finite_only) {
   uint32_t lo[3] = {0xffffffffu, 0xffffffffu, 0xffffffffu}, hi[3] = {0u, 0u, 0u};
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const float x = soa[i], y = soa[n_pad + i], z = soa[2 * n_pad + i];
+    if (finite_only && !(isfinite(x) && isfinite(y) && isfinite(z))) continue;
+    const float v[3] = {x, y, z};
 #pragma unroll
     for (int a = 0; a < 3; ++a) {
-      const uint32_t o = f2ord(soa[a * n_pad + i]);
+      const uint32_t o = f2ord(v[a]);
       lo[a] = min(lo[a], o);
       hi[a] = max(hi[a], o);
     }
+  }
 #pragma unroll
   for (int a = 0; a < 3; ++a) {
     lo[a] = __reduce_min_sync(0xffffffffu, lo[a]);
@@ -51,25 +45,13 @@ __global__ void __launch_bounds__(256) bbox_kernel(const float* __restrict__ soa
     }
 }
 
-struct Quant {
-  double lo[3], w[3], scale;
-  int D;
-  uint32_t qmax;
-};
-
 __global__ void __launch_bounds__(256) morton_kernel(const float* __restrict__ soa, int64_t n, int64_t n_pad, Quant q,
                                                      uint32_t* __restrict__ codes, uint32_t* __restrict__ idx) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   uint32_t c[3];
 #pragma unroll
-  for (int a = 0; a < 3; ++a) {
-    // floor((x - lo) / w * 2^D) in float64, exactly as the oracle computes it
-    const double t = __dmul_rn(__ddiv_rn(__dsub_rn((double)soa[a * n_pad + i], q.lo[a]), q.w[a]), q.scale);
-    long long v = (long long)floor(t);
-    v = v < 0 ? 0 : (v > (long long)q.qmax ? (long long)q.qmax : v);
-    c[a] = (uint32_t)v;
-  }
+  for (int a = 0; a < 3; ++a) c[a] = quantise(soa[a * n_pad + i], q, a);
   uint32_t code = 0;
   for (int b = q.D - 1; b >= 0; --b) code = (code << 3) | (((c[0] >> b) & 1u) << 2) | (((c[1] >> b) & 1u) << 1) | ((c[2] >> b) & 1u);
   codes[i] = code;
@@ -211,7 +193,7 @@ int32_t subset_cull_view(rsc_cloud* cloud, rsc_subset& s, cudaStream_t st) {
   if (m > 0) {
     const uint32_t init[6] = {0xffffffffu, 0xffffffffu, 0xffffffffu, 0u, 0u, 0u};
     CV(cudaMemcpyAsync(mm, init, sizeof(init), cudaMemcpyHostToDevice, st));
-    bbox_kernel<<<ctx->sm_count * 8, 256, 0, st>>>(s.soa, m, s.m_pad, mm);
+    bbox_kernel<<<ctx->sm_count * 8, 256, 0, st>>>(s.soa, m, s.m_pad, mm, false);
     CV(cudaGetLastError());
     uint32_t got[6];
     CV(cudaMemcpyAsync(got, mm, sizeof(got), cudaMemcpyDeviceToHost, st));
@@ -287,7 +269,7 @@ int32_t rsc_cloud_build_cells(rsc_cloud* cloud, int32_t nlevels) {
   OCT(cudaMalloc(&mm, 6 * 4));
   const uint32_t init[6] = {0xffffffffu, 0xffffffffu, 0xffffffffu, 0u, 0u, 0u};
   OCT(cudaMemcpyAsync(mm, init, sizeof(init), cudaMemcpyHostToDevice, st));
-  bbox_kernel<<<ctx->sm_count * 8, 256, 0, st>>>(cloud->soa, n, cloud->n_pad, mm);
+  bbox_kernel<<<ctx->sm_count * 8, 256, 0, st>>>(cloud->soa, n, cloud->n_pad, mm, false);
   OCT(cudaGetLastError());
   uint32_t got[6];
   OCT(cudaMemcpyAsync(got, mm, sizeof(got), cudaMemcpyDeviceToHost, st));

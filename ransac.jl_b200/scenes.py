@@ -183,6 +183,88 @@ def scene_mixed(seed: int, n: int, noise_frac=0.01, jitter_deg=2.0, outlier_frac
     return build_scene(rng, prims, n, noise_frac, jitter_deg, outlier_frac)
 
 
+_VIEW_DRAWS = 64  # batches of 2x the wanted points drawn per primitive before scene_view gives up
+
+
+def scene_view(seed: int, n: int, viewpoint=(0.0, 0.0, 150.0), noise_frac: float = 0.002, counts=(3, 2, 2, 1)) -> Scene:
+    """One scan from `viewpoint` with ground-truth oriented normals: primitives from the factories above (spheres,
+    cylinders and cones with outward normals), of which only the points whose analytic normal faces the viewpoint
+    are kept (back-face culling, no occlusion; planes are two-sided), with the normals flipped towards the viewpoint.
+    Area-weighted share of the n points, Gaussian offset along the normal (sigma = noise_frac * primitive size), no
+    outliers, no normal jitter.  ValueError when a primitive barely faces the viewpoint (e.g. one inside a sphere)."""
+    rng = np.random.default_rng(seed)
+    prims = [make_plane(rng) for _ in range(counts[0])]
+    prims += [make_sphere(rng) for _ in range(counts[1])]
+    prims += [make_cylinder(rng) for _ in range(counts[2])]
+    prims += [make_cone(rng) for _ in range(counts[3])]
+    for p in prims:
+        if p.kind != "plane":
+            p.shape.outwards = True
+    vp = np.asarray(viewpoint, np.float64)
+    w = np.array([p.area for p in prims])
+    cnt = np.floor(w / w.sum() * n).astype(int)
+    cnt[0] += n - cnt.sum()
+    P, Nn, Lb = [], [], []
+    for i, (pr, c) in enumerate(zip(prims, cnt)):
+        got_p, got_n, have = [], [], 0
+        for _ in range(_VIEW_DRAWS):
+            if have >= c:
+                break
+            p, nn = sample_primitive(rng, pr, max(2 * int(c), 64))
+            facing = np.einsum("ij,ij->i", nn, vp - p)
+            if pr.kind == "plane":
+                nn = np.where(facing[:, None] < 0, -nn, nn)
+            else:
+                p, nn = p[facing > 0], nn[facing > 0]
+            got_p.append(p), got_n.append(nn)
+            have += len(p)
+        if have < c:
+            raise ValueError(f"scene_view: too little of primitive {i} ({pr.kind}) faces the viewpoint {tuple(vp)}")
+        p, nn = np.concatenate(got_p)[:c], np.concatenate(got_n)[:c]
+        if noise_frac > 0:
+            p = p + nn * rng.normal(scale=noise_frac * pr.size, size=(len(p), 1))
+        P.append(p), Nn.append(nn), Lb.append(np.full(len(p), i, np.int32))
+    perm = rng.permutation(n)
+    P, Nn, Lb = np.concatenate(P)[perm], np.concatenate(Nn)[perm], np.concatenate(Lb)[perm]
+    return Scene(np.ascontiguousarray(P, dtype=np.float32), np.ascontiguousarray(Nn, dtype=np.float32), Lb, prims)
+
+
+def recovered(scene: Scene, shapes, frac: float = 0.5) -> set:
+    """indices of the ground-truth primitives of `scene` found among `shapes` [(kind, inlier indices)]: a shape of the
+    same kind whose inliers are mostly the primitive's points and cover at least `frac` of them"""
+    kinds = {"plane": 0, "sphere": 1, "cylinder": 2, "cone": 3}
+    sizes = np.bincount(scene.labels[scene.labels >= 0], minlength=len(scene.primitives))
+    found = set()
+    for kind, idx in shapes:
+        if len(idx) == 0:
+            continue
+        lab = np.bincount(scene.labels[idx] + 1, minlength=len(scene.primitives) + 1)[1:]
+        i = int(np.argmax(lab))
+        if kinds[scene.primitives[i].kind] == kind and lab[i] >= 0.5 * len(idx) and lab[i] >= frac * sizes[i]:
+            found.add(i)
+    return found
+
+
+SCAN_VIEWPOINT = (30.0, -20.0, 160.0)
+
+
+@dataclass
+class ScanScenario:
+    scene: Scene
+    viewpoint: tuple
+    subsets: int
+    seed: int
+    iteration: dict
+
+
+def scan_scenario() -> ScanScenario:
+    """Normals for a raw scan, end to end: a noisy 40 000-point scene_view from SCAN_VIEWPOINT with 8 primitives, and the
+    ransac() settings run on it.  With the analytic normals the C oracle's loop recovers all 8 primitives (`recovered`),
+    with normals estimated from the coordinates (k = 16, towards the viewpoint) 6 of them."""
+    return ScanScenario(scene_view(21, 40_000, viewpoint=SCAN_VIEWPOINT, noise_frac=0.002), SCAN_VIEWPOINT, 2, 4321,
+                        {"tau": 100, "minsubsetN": 50, "itermax": 200})
+
+
 def scene_c2(n: int = 1 << 20, seed: int = 2) -> Scene:
     return scene_mixed(seed, n)
 
