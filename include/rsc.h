@@ -435,6 +435,31 @@ int32_t rsc_ransac_run_user(rsc_cloud* cloud, const rsc_params* params, const vo
 int32_t rsc_estimate_normals(rsc_ctx* ctx, const float* xyz, int64_t n, int32_t k, const double* viewpoint,
                              float* nrm, int64_t* nbr, int64_t* pairs);
 
+/* ---- normal orientation without a viewpoint: minimum spanning forest of the k-NN graph (DESIGN.md section 8) ---
+ * Makes the signs of the normals consistent over each connected piece of the cloud, for clouds with no single sensor
+ * position (CAD or mesh samples, merged scans, photogrammetry, files with arbitrary signs).  Deterministic; the
+ * definition, restated in oracle/orient_oracle.py orient_mst:
+ *   1. point i is a vertex when its float32 coordinates are finite and its normal is finite with (x^2 + y^2) + z^2 > 0
+ *      in float64; every other point is returned unchanged (a zero normal stays zero, a NaN normal is copied);
+ *   2. u_i = n_i / sqrt((x^2 + y^2) + z^2) in float64 of the float32 values, every operation rounded, no FMA;
+ *   3. the undirected edges are {i, j}, i != j, j in N(i) (the k-NN lists of rsc_estimate_normals, same k), both
+ *      vertices; the symmetric union, duplicates merged;
+ *   4. d(i, j) = (u_i.x u_j.x + u_i.y u_j.y) + u_i.z u_j.z and w = 1 - |d| in float64; edges are ordered by
+ *      (w, lo, hi), lo < hi the two indices, so the minimum spanning forest F is unique;
+ *   5. each tree of F is rooted at its vertex of largest float32 z (lowest index on ties); the root's sign s is +1 when
+ *      u_r.z > 0, -1 when u_r.z < 0, and when u_r.z == 0 the sign that makes its largest-magnitude component positive
+ *      (the first axis on ties);
+ *   6. along a tree edge from parent p to child c, s(c) = s(p) when d(p, c) >= 0, else -s(p);
+ *   7. nrm_out[i] = s(i) * nrm_in[i]: the input float32 normal with its sign bit flipped or not, not renormalised.
+ * nrm_in NULL: the normals are first estimated exactly as rsc_estimate_normals does without a viewpoint, from the
+ * same k-NN search.  nrm_in == nrm_out is allowed.  Each connected component of the graph is oriented on its own.
+ *   edges: NULL or int64[2 n]: F's edges as (lo, hi) pairs in ascending order, stats[1] of them.
+ *   stats: NULL or int64[4]: {vertices, edges of F, trees of F, Boruvka rounds}.
+ * 3 <= k <= 32, 1 <= n < 2^31; host in / host out, synchronising.  Device memory: about (130 + 4 k) B per point plus
+ * 32 B per graph edge (at most n k edges; about 0.6 n k on surface samples). */
+int32_t rsc_orient_normals(rsc_ctx* ctx, const float* xyz, int64_t n, int32_t k, const float* nrm_in, float* nrm_out,
+                           int64_t* edges, int64_t* stats);
+
 #ifdef __cplusplus
 }
 #endif

@@ -314,6 +314,30 @@ function estimate_normals(vertices::Vector{SVector{3,Float32}}; k::Integer=16, v
     nrm
 end
 
+"""
+    orient_normals(vertices; normals=nothing, k=16) -> Vector{SVector{3,Float32}}
+
+Normals with consistent signs for a cloud without one viewpoint (CAD or mesh samples, merged scans, photogrammetry),
+on the device (`rsc_orient_normals`): signs propagate along the minimum spanning forest of the `k`-nearest-neighbour
+graph weighted by 1 - |n_i . n_j|, each tree's highest point getting a positive z component.  `normals` are oriented
+as given (each row negated or not); `nothing` estimates them first as `estimate_normals(vertices; k)` does.  Points
+with a non-finite coordinate or a zero or non-finite normal are returned unchanged.
+`RANSACCloud(V, orient_normals(V), 2)`.
+"""
+function orient_normals(vertices::Vector{SVector{3,Float32}}; normals=nothing, k::Integer=16)
+    nrm = Vector{SVector{3,Float32}}(undef, length(vertices))
+    nin = normals === nothing ? nothing : convert(Vector{SVector{3,Float32}}, normals)
+    nin === nothing || length(nin) == length(vertices) || throw(ArgumentError("normals must match vertices"))
+    GC.@preserve vertices nrm nin begin
+        check(ccall(fn(:rsc_orient_normals), Int32,
+                    (Ptr{Cvoid}, Ptr{Float32}, Int64, Int32, Ptr{Float32}, Ptr{Float32}, Ptr{Int64}, Ptr{Int64}),
+                    context(), Ptr{Float32}(pointer(vertices)), length(vertices), k,
+                    nin === nothing ? Ptr{Float32}(C_NULL) : Ptr{Float32}(pointer(nin)), Ptr{Float32}(pointer(nrm)),
+                    Ptr{Int64}(C_NULL), Ptr{Int64}(C_NULL)))
+    end
+    nrm
+end
+
 # ---- user-defined shapes on the device (include/rsc.h "user-defined shapes") -----------------------------
 """
     compile_user_shape(src::String) -> type id

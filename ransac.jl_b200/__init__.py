@@ -31,7 +31,7 @@ from .fitting import (
 )
 from .iterations import ransac
 from .jsonyaml import dict2nt, exportJSON, readconfig, toDict
-from .normals import estimate_normals
+from .normals import estimate_normals, orient_normals
 from .params import (
     DEFAULT_PARAMETERS,
     DEFAULT_SHAPE_DICT,

@@ -12,14 +12,14 @@
 //     minus a bound on the quantisation's float64 rounding: every point outside the block is then strictly farther
 //     than the k-th.  Otherwise it rescans one level up; level 2 and level 1 cover the whole box.
 // Then, in the same warp: the float64 covariance of N(i) in list order, cyclic Jacobi, the sign rule, and the stores
-// by original index.
+// by original index.  rsc_orient_normals (rsc_orient.cu) runs the same search through knn_prepare / knn_run
+// (rsc_normals.cuh) and keeps the lists on the device as int32.
 #include <cub/device/device_radix_sort.cuh>
 
 #include <climits>
 #include <cmath>
 
-#include "rsc_common.cuh"
-#include "rsc_morton.cuh"
+#include "rsc_normals.cuh"
 
 namespace rsc {
 namespace {
@@ -138,9 +138,13 @@ struct NormalsArgs {
   int has_vp;
   float* nrm;     // [3 n] AoS, by point index
   int64_t* nbr;   // [n k] or null
+  int32_t* lists; // [n k]: the int32 lists of the kLists32 instantiations
   unsigned long long* pairs;
 };
 
+// kPca = false: the lists alone, no covariance and no normal.  kLists32: the lists go to A.lists as int32 (always
+// written) instead of A.nbr.  <true, false> is rsc_estimate_normals' kernel.
+template <bool kPca, bool kLists32>
 __global__ void __launch_bounds__(256, 2) knn_normals_kernel(const NormalsArgs A) {
   const int lane = threadIdx.x & 31;
   const int64_t nwarps = (int64_t)gridDim.x * kWarpsPerBlock;
@@ -152,8 +156,12 @@ __global__ void __launch_bounds__(256, 2) knn_normals_kernel(const NormalsArgs A
   for (int64_t p = (int64_t)blockIdx.x * kWarpsPerBlock + (threadIdx.x >> 5); p < A.n; p += nwarps) {
     const uint32_t i = __ldg(A.perm + p);
     if (p >= A.nf) {  // non-finite point: zero normal, empty row
-      if (lane < 3) A.nrm[3 * (int64_t)i + lane] = 0.f;
-      if (A.nbr && lane < k) A.nbr[(int64_t)i * k + lane] = -1;
+      if (kPca && lane < 3) A.nrm[3 * (int64_t)i + lane] = 0.f;
+      if (kLists32) {
+        if (lane < k) A.lists[(int64_t)i * k + lane] = -1;
+      } else if (A.nbr && lane < k) {
+        A.nbr[(int64_t)i * k + lane] = -1;
+      }
       continue;
     }
     const uint64_t key = __ldg(A.keys + p);
@@ -276,7 +284,12 @@ __global__ void __launch_bounds__(256, 2) knn_normals_kernel(const NormalsArgs A
       bound_j = __shfl_sync(0xffffffffu, lj, k - 1);
       --level;
     }
-    if (A.nbr && lane < k) A.nbr[(int64_t)i * k + lane] = lane < keff ? (int64_t)lj : -1;
+    if (kLists32) {
+      if (lane < k) A.lists[(int64_t)i * k + lane] = lane < keff ? lj : -1;
+      if (!kPca) continue;
+    } else if (A.nbr && lane < k) {
+      A.nbr[(int64_t)i * k + lane] = lane < keff ? (int64_t)lj : -1;
+    }
     // covariance of N(i), summed in list order
     const double px = lane < keff ? (double)A.sx[lp] : 0.0, py = lane < keff ? (double)sy[lp] : 0.0,
                  pz = lane < keff ? (double)sz[lp] : 0.0;
@@ -330,52 +343,29 @@ __global__ void __launch_bounds__(256, 2) knn_normals_kernel(const NormalsArgs A
   if (lane == 0 && A.pairs && pairs) atomicAdd(A.pairs, (unsigned long long)pairs);
 }
 
-// device allocations of one call, released on every return path
-struct Allocs {
-  void* p[10] = {};
-  int np = 0;
-  cudaError_t get(void** out, size_t bytes) {
-    cudaError_t e = cudaMalloc(out, bytes ? bytes : 16);
-    if (e == cudaSuccess) p[np++] = *out;
-    return e;
-  }
-  ~Allocs() {
-    for (int i = 0; i < np; ++i) cudaFree(p[i]);
-  }
-};
-
 }  // namespace
 }  // namespace rsc
 
 using namespace rsc;
 
-extern "C" int32_t rsc_estimate_normals(rsc_ctx* ctx, const float* xyz, int64_t n, int32_t k, const double* viewpoint, float* nrm,
-                                        int64_t* nbr, int64_t* pairs) {
-  if (!ctx) return RSC_E_ARG;
-  if (!xyz || !nrm) return fail(ctx, RSC_E_ARG, "estimate_normals: xyz and nrm must not be NULL");
-  if (k < 3 || k > 32) return fail(ctx, RSC_E_ARG, "estimate_normals: k must be in [3, 32]");
-  if (n < 1 || n >= ((int64_t)1 << 31)) return fail(ctx, RSC_E_ARG, "estimate_normals: n must be in [1, 2^31)");
+int32_t rsc::knn_prepare(rsc_ctx* ctx, const float* xyz, int64_t n, KnnSearch& S) {
   RSC_CUDA(ctx, cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
-  Allocs al;
-  float *d_aos = nullptr, *d_soa = nullptr, *d_nrm = nullptr;
+  Allocs& al = S.al;
   uint64_t* d_keys[2] = {nullptr, nullptr};
   uint32_t* d_idx[2] = {nullptr, nullptr};
   uint32_t* d_mm = nullptr;
-  unsigned long long* d_cnt = nullptr;  // [0] finite points, [1] pairs
-  int64_t* d_nbr = nullptr;
   void* d_tmp = nullptr;
 #define NRM_CUDA(expr) RSC_CUDA(ctx, (expr))
-  NRM_CUDA(al.get((void**)&d_aos, (size_t)n * 12));
-  NRM_CUDA(al.get((void**)&d_soa, (size_t)n * 12));
-  NRM_CUDA(al.get((void**)&d_nrm, (size_t)n * 12));
+  S.n = n;
+  NRM_CUDA(al.get((void**)&S.aos, (size_t)n * 12));
+  NRM_CUDA(al.get((void**)&S.soa, (size_t)n * 12));
   for (int b = 0; b < 2; ++b) {
     NRM_CUDA(al.get((void**)&d_keys[b], (size_t)n * 8));
     NRM_CUDA(al.get((void**)&d_idx[b], (size_t)n * 4));
   }
   NRM_CUDA(al.get((void**)&d_mm, 6 * 4 + 2 * 8));
-  d_cnt = reinterpret_cast<unsigned long long*>(d_mm + 6);
-  if (nbr) NRM_CUDA(al.get((void**)&d_nbr, (size_t)n * k * 8));
+  S.cnt = reinterpret_cast<unsigned long long*>(d_mm + 6);
   cub::DoubleBuffer<uint64_t> kbuf(d_keys[0], d_keys[1]);
   cub::DoubleBuffer<uint32_t> ibuf(d_idx[0], d_idx[1]);
   size_t tmp_bytes = 0;
@@ -383,18 +373,18 @@ extern "C" int32_t rsc_estimate_normals(rsc_ctx* ctx, const float* xyz, int64_t 
   NRM_CUDA(al.get(&d_tmp, tmp_bytes));
 
   const unsigned blocks = (unsigned)((n + 255) / 256);
-  NRM_CUDA(cudaMemcpyAsync(d_aos, xyz, (size_t)n * 12, cudaMemcpyHostToDevice, st));
+  NRM_CUDA(cudaMemcpyAsync(S.aos, xyz, (size_t)n * 12, cudaMemcpyHostToDevice, st));
   const uint32_t init[6] = {0xffffffffu, 0xffffffffu, 0xffffffffu, 0u, 0u, 0u};
   NRM_CUDA(cudaMemcpyAsync(d_mm, init, sizeof(init), cudaMemcpyHostToDevice, st));
-  NRM_CUDA(cudaMemsetAsync(d_cnt, 0, 2 * 8, st));
-  aos_to_soa_kernel<<<blocks, 256, 0, st>>>(d_aos, n, d_soa);
+  NRM_CUDA(cudaMemsetAsync(S.cnt, 0, 2 * 8, st));
+  aos_to_soa_kernel<<<blocks, 256, 0, st>>>(S.aos, n, S.soa);
   NRM_CUDA(cudaGetLastError());
-  bbox_kernel<<<ctx->sm_count * 8, 256, 0, st>>>(d_soa, n, n, d_mm, true);
+  bbox_kernel<<<ctx->sm_count * 8, 256, 0, st>>>(S.soa, n, n, d_mm, true);
   NRM_CUDA(cudaGetLastError());
   uint32_t got[6];
   NRM_CUDA(cudaMemcpyAsync(got, d_mm, sizeof(got), cudaMemcpyDeviceToHost, st));
   NRM_CUDA(cudaStreamSynchronize(st));
-  Quant q;
+  Quant& q = S.q;
   q.D = kKeyBits;
   q.scale = (double)((uint64_t)1 << kKeyBits);
   q.qmax = (1u << kKeyBits) - 1u;
@@ -405,32 +395,63 @@ extern "C" int32_t rsc_estimate_normals(rsc_ctx* ctx, const float* xyz, int64_t 
     if (!(q.w[a] > 0.0)) q.w[a] = 1.0;  // one value on this axis, or no finite point at all
     if (!std::isfinite(q.lo[a])) q.lo[a] = 0.0;
   }
-  keys_kernel<<<blocks, 256, 0, st>>>(d_soa, n, q, d_keys[0], d_idx[0], d_cnt);
+  keys_kernel<<<blocks, 256, 0, st>>>(S.soa, n, q, d_keys[0], d_idx[0], S.cnt);
   NRM_CUDA(cudaGetLastError());
   NRM_CUDA(cub::DeviceRadixSort::SortPairs(d_tmp, tmp_bytes, kbuf, ibuf, (int)n, 0, 64, st));
-  gather_sorted_kernel<<<blocks, 256, 0, st>>>(d_aos, ibuf.Current(), n, d_soa);
+  gather_sorted_kernel<<<blocks, 256, 0, st>>>(S.aos, ibuf.Current(), n, S.soa);
   NRM_CUDA(cudaGetLastError());
   unsigned long long nf = 0;
-  NRM_CUDA(cudaMemcpyAsync(&nf, d_cnt, 8, cudaMemcpyDeviceToHost, st));
+  NRM_CUDA(cudaMemcpyAsync(&nf, S.cnt, 8, cudaMemcpyDeviceToHost, st));
   NRM_CUDA(cudaStreamSynchronize(st));
+  S.nf = (int64_t)nf;
+  S.keys = kbuf.Current();
+  S.perm = ibuf.Current();
+  return RSC_OK;
+}
 
+int32_t rsc::knn_run(rsc_ctx* ctx, const KnnSearch& S, int32_t k, const double* viewpoint, float* d_nrm, int64_t* d_nbr,
+                     int32_t* d_lists) {
   NormalsArgs A;
-  A.keys = kbuf.Current();
-  A.perm = ibuf.Current();
-  A.sx = d_soa;
-  A.n = (int32_t)n, A.nf = (int32_t)nf, A.k = k, A.keff = (int32_t)std::min<unsigned long long>((unsigned long long)k, nf);
-  A.q = q;
+  A.keys = S.keys;
+  A.perm = S.perm;
+  A.sx = S.soa;
+  A.n = (int32_t)S.n, A.nf = (int32_t)S.nf, A.k = k, A.keff = (int32_t)std::min<int64_t>(k, S.nf);
+  A.q = S.q;
   A.has_vp = viewpoint != nullptr;
   for (int a = 0; a < 3; ++a) A.vp[a] = viewpoint ? viewpoint[a] : 0.0;
-  A.nrm = d_nrm, A.nbr = d_nbr, A.pairs = d_cnt + 1;
-  const int64_t want = (n + kWarpsPerBlock - 1) / kWarpsPerBlock;
-  knn_normals_kernel<<<(unsigned)std::min<int64_t>(want, (int64_t)ctx->sm_count * 8), 256, 0, st>>>(A);
+  A.nrm = d_nrm, A.nbr = d_nbr, A.lists = d_lists, A.pairs = S.cnt + 1;
+  const int64_t want = (S.n + kWarpsPerBlock - 1) / kWarpsPerBlock;
+  const unsigned grid = (unsigned)std::min<int64_t>(want, (int64_t)ctx->sm_count * 8);
+  cudaStream_t st = ctx->stream;
+  if (!d_lists)
+    knn_normals_kernel<true, false><<<grid, 256, 0, st>>>(A);
+  else if (d_nrm)
+    knn_normals_kernel<true, true><<<grid, 256, 0, st>>>(A);
+  else
+    knn_normals_kernel<false, true><<<grid, 256, 0, st>>>(A);
   NRM_CUDA(cudaGetLastError());
+  return RSC_OK;
+}
+
+extern "C" int32_t rsc_estimate_normals(rsc_ctx* ctx, const float* xyz, int64_t n, int32_t k, const double* viewpoint, float* nrm,
+                                        int64_t* nbr, int64_t* pairs) {
+  if (!ctx) return RSC_E_ARG;
+  if (!xyz || !nrm) return fail(ctx, RSC_E_ARG, "estimate_normals: xyz and nrm must not be NULL");
+  if (k < 3 || k > 32) return fail(ctx, RSC_E_ARG, "estimate_normals: k must be in [3, 32]");
+  if (n < 1 || n >= ((int64_t)1 << 31)) return fail(ctx, RSC_E_ARG, "estimate_normals: n must be in [1, 2^31)");
+  KnnSearch S;
+  float* d_nrm = nullptr;
+  int64_t* d_nbr = nullptr;
+  if (int32_t rc = knn_prepare(ctx, xyz, n, S)) return rc;
+  NRM_CUDA(S.al.get((void**)&d_nrm, (size_t)n * 12));
+  if (nbr) NRM_CUDA(S.al.get((void**)&d_nbr, (size_t)n * k * 8));
+  if (int32_t rc = knn_run(ctx, S, k, viewpoint, d_nrm, d_nbr, nullptr)) return rc;
+  cudaStream_t st = ctx->stream;
   if (int32_t rc = staged_d2h(ctx, nrm, d_nrm, (size_t)n * 12, st)) return rc;
   if (nbr)
     if (int32_t rc = staged_d2h(ctx, nbr, d_nbr, (size_t)n * k * 8, st)) return rc;
   unsigned long long np = 0;
-  NRM_CUDA(cudaMemcpyAsync(&np, d_cnt + 1, 8, cudaMemcpyDeviceToHost, st));
+  NRM_CUDA(cudaMemcpyAsync(&np, S.cnt + 1, 8, cudaMemcpyDeviceToHost, st));
   NRM_CUDA(cudaStreamSynchronize(st));
 #undef NRM_CUDA
   if (pairs) *pairs = (int64_t)np;
