@@ -244,6 +244,18 @@ inline PointSet view_subset(const rsc_subset* s) {
   return ps;
 }
 
+// the subset's Morton-ordered view (subset_cull_view), as the culled scorer reads it: no valid words (the first m
+// points are the real ones)
+inline PointSet view_subset_morton(const rsc_subset* s) {
+  PointSet ps;
+  ps.x = s->csoa, ps.y = s->csoa + s->m_pad, ps.z = s->csoa + 2 * s->m_pad;
+  ps.nx = s->csoa + 3 * s->m_pad, ps.ny = s->csoa + 4 * s->m_pad, ps.nz = s->csoa + 5 * s->m_pad;
+  ps.enabled = s->cen, ps.valid = nullptr;
+  ps.n = s->m, ps.n_pad = s->m_pad;
+  ps.xyz64 = s->xyz64, ps.nrm64 = s->nrm64, ps.map = s->cidx;
+  return ps;
+}
+
 // error plumbing
 int32_t fail(rsc_ctx* ctx, int32_t code, const char* what);
 int32_t fail_cuda(rsc_ctx* ctx, cudaError_t e, const char* where);
@@ -275,7 +287,8 @@ int32_t refresh_subsets_enabled(rsc_cloud* cloud, cudaStream_t st);
 // culled scorer (rsc_cull.cu) and the Morton view of a subset it runs on (rsc_octree.cu)
 int32_t subset_cull_view(rsc_cloud* cloud, rsc_subset& s, cudaStream_t st);
 size_t cull_sphere_count(int64_t n_pad);  // float4 entries cull_tile_spheres writes (tiles, groups, blocks)
-int32_t cull_tile_spheres(rsc_ctx* ctx, const PointSet& ps, float4* tiles, cudaStream_t st);
+// (d_n, nullable: the number of real points lives on the device, at most ps.n -- the spheres leave the rest out)
+int32_t cull_tile_spheres(rsc_ctx* ctx, const PointSet& ps, float4* tiles, cudaStream_t st, const unsigned long long* d_n = nullptr);
 int32_t cull_enqueue(rsc_ctx* ctx, const rsc_cloud* cloud, const PointSet& ps, const float4* tiles, const Thresh& th,
                      const rsc_cand* d_cands, int C_cap, const int32_t* d_C, int32_t* cv, int32_t* ce, unsigned long long* d_stats,
                      cudaStream_t st);
@@ -339,10 +352,6 @@ int32_t shard_sync_enabled(rsc_cloud* cloud, cudaStream_t st);
 // the ranks too (returned in d_extra_out[0..n_extra), device) -- collective
 int32_t shard_clear_enabled(rsc_cloud* cloud, const uint32_t* inl_local, const int32_t* d_extra_in, int n_extra,
                             int32_t* d_extra_out, cudaStream_t st);
-// the two loops behind rsc_ransac_run (rsc_loop.cu: reference behaviour, decisions on the device;
-// rsc_run.cu: the extension switches, host-walked)
-// order (nullable): a mixed fit order in place of p->shape_types (rsc_ransac_run_user)
-int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed, rsc_run* run, const FitOrder* order = nullptr);
 void loop_scratch_free(rsc_ctx* ctx);
 int32_t fit_reserve(rsc_ctx* ctx, const rsc_params* params, int S, int ntypes = -1);
 // exclusive scan of n uint32 counts into 64-bit offsets (+ total) on `st` (rsc_fit.cu)

@@ -32,7 +32,7 @@
 namespace rsc {
 
 size_t cull_sphere_count(int64_t n_pad);
-int32_t cull_tile_spheres(rsc_ctx* ctx, const PointSet& ps, float4* tiles, cudaStream_t st);
+int32_t cull_tile_spheres(rsc_ctx* ctx, const PointSet& ps, float4* tiles, cudaStream_t st, const unsigned long long* d_n);
 
 constexpr int kCullThreads = 128;
 constexpr int kCullWarps = kCullThreads / 32;
@@ -137,7 +137,8 @@ __global__ void widen_u32_kernel(const uint32_t* __restrict__ in, int64_t n, int
 // (rounded up)
 __global__ void __launch_bounds__(256) tile_sphere_kernel(const float* __restrict__ X, const float* __restrict__ Y,
                                                           const float* __restrict__ Z, int64_t n, int tile_pts, int ntiles,
-                                                          float4* __restrict__ tiles) {
+                                                          float4* __restrict__ tiles, const unsigned long long* __restrict__ d_n) {
+  if (d_n) n = min(n, (int64_t)*d_n);
   const int tile = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   if (tile >= ntiles) return;
@@ -515,16 +516,16 @@ size_t cull_sphere_count(int64_t n_pad) {
   return (size_t)(n_pad / kCullTile + n_pad / kCullGroup + (n_pad / kCullGroup + kCullBlockGroups - 1) / kCullBlockGroups);
 }
 
-int32_t cull_tile_spheres(rsc_ctx* ctx, const PointSet& ps, float4* tiles, cudaStream_t st) {
+int32_t cull_tile_spheres(rsc_ctx* ctx, const PointSet& ps, float4* tiles, cudaStream_t st, const unsigned long long* d_n) {
   const int ntiles = (int)(ps.n_pad / kCullTile), ngroups = (int)(ps.n_pad / kCullGroup);
   const int nblocks = (ngroups + kCullBlockGroups - 1) / kCullBlockGroups;
   if (ntiles == 0) return RSC_OK;
-  tile_sphere_kernel<<<(ntiles + 7) / 8, 256, 0, st>>>(ps.x, ps.y, ps.z, ps.n, kCullTile, ntiles, tiles);
+  tile_sphere_kernel<<<(ntiles + 7) / 8, 256, 0, st>>>(ps.x, ps.y, ps.z, ps.n, kCullTile, ntiles, tiles, d_n);
   RSC_CUDA(ctx, cudaGetLastError());
-  tile_sphere_kernel<<<(ngroups + 7) / 8, 256, 0, st>>>(ps.x, ps.y, ps.z, ps.n, kCullGroup, ngroups, tiles + ntiles);
+  tile_sphere_kernel<<<(ngroups + 7) / 8, 256, 0, st>>>(ps.x, ps.y, ps.z, ps.n, kCullGroup, ngroups, tiles + ntiles, d_n);
   RSC_CUDA(ctx, cudaGetLastError());
   tile_sphere_kernel<<<(nblocks + 7) / 8, 256, 0, st>>>(ps.x, ps.y, ps.z, ps.n, kCullGroup * kCullBlockGroups, nblocks,
-                                                        tiles + ntiles + ngroups);
+                                                        tiles + ntiles + ngroups, d_n);
   RSC_CUDA(ctx, cudaGetLastError());
   return RSC_OK;
 }
@@ -634,13 +635,7 @@ int32_t loop_score_new(rsc_ctx* ctx, rsc_cloud* cloud, rsc_subset& sub, const Po
     return RSC_OK;
   }
   if (int32_t rc = subset_cull_view(cloud, sub, st)) return rc;
-  PointSet cps;
-  cps.x = sub.csoa, cps.y = sub.csoa + sub.m_pad, cps.z = sub.csoa + 2 * sub.m_pad;
-  cps.nx = sub.csoa + 3 * sub.m_pad, cps.ny = sub.csoa + 4 * sub.m_pad, cps.nz = sub.csoa + 5 * sub.m_pad;
-  cps.enabled = sub.cen, cps.valid = nullptr;
-  cps.n = sub.m, cps.n_pad = sub.m_pad;
-  cps.xyz64 = sub.xyz64, cps.nrm64 = sub.nrm64, cps.map = sub.cidx;
-  if (int32_t rc = cull_enqueue(ctx, cloud, cps, reinterpret_cast<const float4*>(sub.ctiles), th, d_cands, n_new, nullptr, cv, ce, nullptr, st))
+  if (int32_t rc = cull_enqueue(ctx, cloud, view_subset_morton(&sub), reinterpret_cast<const float4*>(sub.ctiles), th, d_cands, n_new, nullptr, cv, ce, nullptr, st))
     return rc;
   if (d_ovf) RSC_CUDA(ctx, cudaMemsetAsync(d_ovf, 0, 4, st));  // nothing can overflow: pairs beyond the queue are decided inline
   ctx->stats.score_launches += 1;
@@ -688,11 +683,7 @@ static int32_t score_culled_impl(rsc_cloud* cloud, const rsc_params* params, con
       return fail(ctx, RSC_E_ARG, "score_culled: subset has not been uploaded");
     rsc_subset& sub = cloud->subsets[subset_id];
     if (int32_t rc = subset_cull_view(cloud, sub, st)) return rc;
-    ps.x = sub.csoa, ps.y = sub.csoa + sub.m_pad, ps.z = sub.csoa + 2 * sub.m_pad;
-    ps.nx = sub.csoa + 3 * sub.m_pad, ps.ny = sub.csoa + 4 * sub.m_pad, ps.nz = sub.csoa + 5 * sub.m_pad;
-    ps.enabled = sub.cen, ps.valid = nullptr;
-    ps.n = sub.m, ps.n_pad = sub.m_pad;
-    ps.xyz64 = sub.xyz64, ps.nrm64 = sub.nrm64, ps.map = sub.cidx;
+    ps = view_subset_morton(&sub);
     tiles = reinterpret_cast<const float4*>(sub.ctiles);
   }
   const Thresh th = make_thresh(params);

@@ -1,8 +1,13 @@
-// rsc_loop.cu -- ransac(pc, params) for the built-in shapes with the whole bookkeeping on the device
-// (iterations.jl:35-162): the default loop behind rsc_ransac_run.
+// rsc_loop.cu -- ransac(pc, params) (iterations.jl:35-162): the RANSAC loop behind rsc_ransac_run and
+// rsc_ransac_run_user, with the candidate store, the scoring and the removal of invalid candidates on the device.
 //
-// Per speculative batch of nb iterations (rsc_run.cu explains the batching):
-//   K1  sample + fit                      rsc_fit.cu        -> candidates, per-iteration segment bounds
+// Iterations run in SPECULATIVE BATCHES of nb: as long as nothing is extracted the enabled mask is unchanged,
+// so iterations k..k+nb-1 sample (the same Philox set ids as separate iterations), fit and score together.  The
+// decision then walks the batch with the reference's bookkeeping, iteration by iteration, and cuts it at the
+// first extraction or at termination; the iterations behind the cut are discarded and redone (their sets
+// sampled a stale mask).  Per batch:
+//   K1  sample + fit                      rsc_fit.cu        -> candidates, per-iteration segment bounds (root-cell
+//                                                            sampler; level-weighted cell sampler with RSC_SAMPLER_OCTREE)
 //   K2  score the new candidates on subset 1 (iterations.jl:95), counts all-reduced when sharded
 //   K3  finish_new / argmax / seg_argmax  -> best of the old store, best of every iteration's candidates
 //       decide_kernel                     the reference's bookkeeping, iteration by iteration:
@@ -13,16 +18,21 @@
 //                                         termination test (iterations.jl:151-156) -- it cuts the batch
 //                                         at the first extraction / termination and leaves a 128-byte
 //                                         record (iterations used, extract?, which candidate, its 64-byte
-//                                         shape, counters) that the host reads with ONE synchronisation
+//                                         shape, counters) that the host reads with ONE synchronisation.
+//       With RSC_SCORE_PROGRESSIVE, RSC_SAMPLER_OCTREE or RSC_LOOP_HOSTWALK the host takes that decision instead
+//       (host_decide, rsc_run.cu), from the same segment bounds and keys read with one synchronisation.
 //   on extraction:
 //   K4  refit over the rank's points, ascending inlier indices by stream compaction, enabled bits
 //       cleared (rsc_extract.cu)
-//   K5  removeinvalidshapes!: the stored candidates are re-scored with K2 against the subset-1 copy
-//       under the mask "enabled before the extraction and not after" -- a candidate has a now-disabled
-//       inlier iff that count is non-zero (see rsc_run.cu for the equivalence, Q4 included) -- then
-//       invalidate + order-preserving compaction.  No gather, no intermediate host round trip.
-// Host synchronisations: 2 per batch (the number of new candidates sizes the K2 launch; the decision
-// record) + 1 per extraction (store size, inlier count).
+//   K5  removeinvalidshapes! without stored inlier lists: every stored candidate's subset-1 inliers are enabled
+//       at the time of an extraction (the reference removes any candidate with a disabled inlier at each
+//       extraction, and new candidates only count enabled points), so "has a now-disabled inlier" == "is
+//       compatible with one of the NEWLY disabled subset-1 points".  Those points are gathered into a scratch
+//       point set and the store is re-scored against it, then invalidate + order-preserving compaction.
+//       Spheres, whose reference scorer ignores `isenabled` (Q4), additionally die at the first extraction
+//       after they were scored if they matched any already-disabled point.
+// Host synchronisations: 1 per batch for a small batch (its K2 launch is sized by a prediction), else 2 (the
+// number of new candidates sizes the K2 launch; the decision) + 1 per extraction (store size, inlier count).
 //
 // Multi-GPU, one process per GPU (include/rsc.h "point-range sharding"):
 //   sharded storage  every rank holds its point range only; minimal sets are drawn from the replicated
@@ -43,30 +53,10 @@
 
 namespace rsc {
 
-constexpr int kMaxBatch = 64;
-
 struct DecideParams {
   long long N, M, tau;
   double prob_det;
   int S, drawN, extract_s, terminate_s;
-};
-
-struct BatchRec {  // device -> host, once per batch
-  long long counters[3];
-  int32_t used, extract, terminated, iterations;
-  int32_t best_idx, best_score, store_n, ovf;  // ovf: 1 = a guard-band queue overflowed, 2 = more new candidates than the launch was sized for
-  int32_t n_new, pad;
-  rsc_cand best;
-};
-
-struct LoopDev {  // device-resident scratch + state of one run
-  int64_t oldbest[2];             // arg-max over the store as it was before the batch: index, score
-  long long seg_keys[kMaxBatch];  // per batch iteration: arg-max key over its new candidates
-  int32_t seg[kMaxBatch + 2];     // per batch iteration: first new candidate
-  long long counters[3];          // countcandidates: lengthC, allcand, nofminset (iterations.jl:70)
-  BatchRec rec;
-  unsigned long long kept;        // store size after K5
-  int32_t tot_global[2];          // sharded storage: inliers of the extraction summed over the ranks
 };
 
 struct K5Host {  // what the host reads after an extraction
@@ -166,16 +156,17 @@ __global__ void append_new_kernel(const rsc_cand* __restrict__ src, const unsign
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n * 4; i += gridDim.x * blockDim.x) d[i] = s[i];
 }
 
-__global__ void finish_new_dev_kernel(const rsc_cand* __restrict__ cands, const unsigned long long* __restrict__ total, int cap,
-                                      const int32_t* __restrict__ cv, const int32_t* __restrict__ ce, uint32_t honour_enabled,
-                                      int32_t* __restrict__ score, uint8_t* __restrict__ flags) {
-  const int n = (int)min(*total, (unsigned long long)cap);
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-    const int t = cands[i].type;
-    const bool honour = t >= RSC_NTYPES || ((honour_enabled >> t) & 1u);  // user shapes honour the enabled mask
-    score[i] = honour ? ce[i] : cv[i];
-    flags[i] = (uint8_t)(1u | ((!honour && cv[i] != ce[i]) ? 2u : 0u));
-  }
+// cell sampler, per batch iteration and octree level: number of new candidates and the sum of their scores
+// (fitting.jl:184 adds E(score) per candidate; E is affine in the count, so the host adds the closed form of the sum)
+__global__ void level_stats_kernel(const int32_t* __restrict__ out_set, const int32_t* __restrict__ set_level,
+                                   const int32_t* __restrict__ score, int n, int S, long long (*__restrict__ lv)[22]) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const int l = set_level[out_set[i]] - 1;
+  if (l < 0 || l >= 11) return;
+  long long* row = lv[out_set[i] / S];  // the batch iteration the candidate's minimal set belongs to
+  atomicAdd((unsigned long long*)(row + l), 1ull);
+  atomicAdd((unsigned long long*)(row + 11 + l), (unsigned long long)score[i]);
 }
 
 // K5: mask of the subset points the extraction just disabled, in place: old &= ~new
@@ -226,7 +217,7 @@ __global__ void k5_pack_kernel(LoopDev* __restrict__ d, const unsigned long long
   out->tot_global = d->tot_global[0];
 }
 
-int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed, rsc_run* run, const FitOrder* order) {
+int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed, rsc_run* run, const FitOrder* order, HostWalk* host) {
   rsc_ctx* ctx = cloud->ctx;
   cudaStream_t st = ctx->stream;
   if (!ctx->loop_scratch) ctx->loop_scratch = new LoopScratch();
@@ -246,6 +237,12 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
     return fail(ctx, RSC_E_STATE, "ransac_run: RSC_REFIT_LSQ / RSC_EXTRACT_BITMAP are not available on sharded storage");
   if ((p->compat_flags & RSC_EXTRACT_BITMAP) && !(ctx->bitmap_beta > 0.0))
     return fail(ctx, RSC_E_STATE, "ransac_run: RSC_EXTRACT_BITMAP needs rsc_ctx_set_bitmap(ctx, beta, eight) first");
+  const bool cells = (p->compat_flags & RSC_SAMPLER_OCTREE) != 0;
+  const bool prog = (p->compat_flags & RSC_SCORE_PROGRESSIVE) != 0;
+  // cell sampler: the level weights are refreshed every `lw_period` iterations (params.lw_period; 1 = after every
+  // iteration, the reference's schedule, iterations.jl:148); a batch never crosses a refresh, so the results for a
+  // given period do not depend on the batch size
+  const int lw_period = cells ? std::max(1, (int)p->lw_period) : 1;
   const int64_t N = cloud->n_global > 0 ? cloud->n_global : cloud->n;
   const int64_t M = sub.m_global > 0 ? sub.m_global : sub.m;
   const int S = p->minsubsetN;
@@ -254,18 +251,7 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
   // user shapes (rsc_ransac_run_user): their fit, score and mask kernels join K1, K2, K4 and K5; such runs never take
   // the culled scorer, which knows the built-in types only
   const FitOrder* uo = order && order->has_user ? order : nullptr;
-  // this rank's slice of the subset copy: all of it (single GPU, or a shard's local entries) or, on
-  // replicated storage, the same fraction of it as the rank's range of the cloud
-  PointSet sps = view_subset(&sub);
-  if (ranged && cloud->n_pad > 0) {
-    const int64_t lo = (int64_t)((double)cloud->range_lo / cloud->n_pad * sub.m_pad) / kTile * kTile;
-    const int64_t hi =
-        cloud->range_hi >= cloud->n_pad ? sub.m_pad : (int64_t)((double)cloud->range_hi / cloud->n_pad * sub.m_pad) / kTile * kTile;
-    sps.x += lo, sps.y += lo, sps.z += lo, sps.nx += lo, sps.ny += lo, sps.nz += lo;
-    sps.enabled += lo / 32, sps.valid += lo / 32;
-    sps.n_pad = std::max<int64_t>(0, hi - lo);
-    sps.n = std::max<int64_t>(0, (sub.m < hi ? sub.m : hi) - lo);
-  }
+  const PointSet sps = subset_slice(cloud, sub, ranged);
   const int64_t sps_word0 = sps.enabled - sub.enabled;
   // small-batch scorer (rsc_small.cu) limits: beyond them the tiled kernel is the faster one
   const bool use_small = getenv("RSC_NO_SMALL") == nullptr;
@@ -273,13 +259,18 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
   // points and linear in the candidates, tiled path ~190 us flat at this size -> cross-over near 1e8 evaluations)
   constexpr int kSmallMaxCands = 4096;
   constexpr double kSmallMaxEvals = 1.2e8;
+  // K5 on the subset's Morton view: the culled scorer (0: never, 1: for a large store, 2: always; read per run)
+  const int k5_cull_mode = getenv("RSC_LOOP_CULL") ? atoi(getenv("RSC_LOOP_CULL")) : 1;
   long long rate_seen = -1;  // recent number of new candidates per iteration (-1: no batch yet)
   const int Bmax = getenv("RSC_BATCH") ? std::max(1, std::min(kMaxBatch, atoi(getenv("RSC_BATCH")))) : 16;
   const int Bmin = getenv("RSC_BATCH_MIN") ? std::max(1, std::min(Bmax, atoi(getenv("RSC_BATCH_MIN")))) : std::min(8, Bmax);
-  // Without the two switches the batch sizes follow the run: a batch is cut at the first extraction and the sets drawn
-  // behind the cut are fitted for nothing, so batches should not be much longer than the usual gap between two
-  // extractions (c4: an extraction every ~11 iterations -> 6 rising to 12 measured best (13.7 ms of K1 + K2 against 15.0
-  // at 8..16); c5: every ~17 -> 8..16).  `gap` = smoothed iterations per extraction; results do not depend on any of this.
+  // Unless RSC_BATCH / RSC_BATCH_MIN are set the batch sizes follow the run: a batch is cut at the first extraction and
+  // the sets drawn behind the cut are fitted for nothing, so batches should not be much longer than the usual gap
+  // between two extractions (c4: an extraction every ~11 iterations -> 6 rising to 12 measured best (13.7 ms of K1 + K2
+  // against 15.0 at 8..16); c5: every ~17 -> 8..16).  `gap` = smoothed iterations per extraction; results do not
+  // depend on any of this.  Host-decided runs follow the same policy: on c4 (B200, 1000 W) the cell sampler's loop
+  // (lw_period 16) and progressive scoring's took the same time as under a doubling-to-16 / 8-after-an-extraction
+  // rule, within the run-to-run spread.
   const bool adapt = !getenv("RSC_BATCH") && !getenv("RSC_BATCH_MIN");
   double gap = 16.0;
   int since_extract = 0;
@@ -300,11 +291,14 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
     if (_e != cudaSuccess) return fail_cuda(ctx, _e, #expr); \
   } while (0)
 
-  // pinned mirror of what the host reads (seg bounds, decision record, K5 summary)
+  // pinned mirror of what the host reads (seg bounds, decision record, K5 summary; the device state and the
+  // overflow flag for the host decision)
   struct HostIo {
     int32_t seg[kMaxBatch + 2];
     BatchRec rec;
     K5Host k5;
+    LoopDev dev;
+    int32_t ovf;
   };
   if (ctx->pinned_cap < sizeof(HostIo)) {
     if (ctx->pinned) cudaFreeHost(ctx->pinned);
@@ -340,29 +334,101 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
   q.N = N, q.M = M, q.tau = p->tau, q.prob_det = p->prob_det;
   q.S = S, q.drawN = p->drawN, q.extract_s = p->extract_s, q.terminate_s = p->terminate_s;
   bool terminated = false;
+  std::vector<int32_t> newscore;  // progressive scoring: the new candidates' subset-1 scores, for the host decision
+  std::vector<uint32_t> keep_h;   // progressive scoring: K5's survivors, to compact the host's mirror of the store
 
   for (int k = 1; k <= p->itermax && !terminated;) {
     if (n_enabled < p->tau) break;  // iterations.jl:75
-    const int nb = std::min(B, p->itermax - k + 1);
+    int nb = std::min(B, p->itermax - k + 1);
+    if (cells) nb = std::min(nb, lw_period - (k - 1) % lw_period);  // up to the next refresh of the level weights
     const auto tk0 = now();
     ++run->batches;
     // ---- K1: nb * minsubsetN minimal sets -> candidates (device, compacted in reference order) ----
     FitScratch fs;
+    double cum[11];
+    if (cells) rsc_level_cumsum(run->levelweight, run->nlevels, cum);
     // (segment bounds of the batch's iterations: from the compaction itself when an iteration is whole groups of sets)
     const bool seg_fused = S % 128 == 0;
-    if ((rc = fit_enqueue(ctx, cloud, 2, p, p->drawN, nullptr, nullptr, nullptr, S * nb, seed, (uint64_t)(k - 1) * S, st, &fs, nullptr,
-                          seg_fused ? dev->seg : nullptr, S, nb, order)))
+    if ((rc = fit_enqueue(ctx, cloud, cells ? 3 : 2, p, p->drawN, nullptr, nullptr, nullptr, S * nb, seed, (uint64_t)(k - 1) * S, st, &fs,
+                          cells ? cum : nullptr, seg_fused ? dev->seg : nullptr, S, nb, order)))
       return rc;
     if (!seg_fused) {
       seg_bounds_kernel<<<1, 96, 0, st>>>(fs.out_set, fs.total, S, nb, dev->seg);
       RUN_CUDA(cudaGetLastError());
     }
     const int store_n0 = store.n;
+    // ---- K2 on subset 1 + K3 for `n` new candidates: their number, or (d_total, the sync-free path) the size of a
+    // launch whose true number of candidates stays on the device.  The dense scorer's overflow flag rides behind the
+    // counts, so that a sharded run decides to repeat collectively.  (The cell sampler decides on the host, so its
+    // batches never take the sync-free path: `n` is exact for its level statistics.)
+    auto score_batch = [&](int n, const unsigned long long* d_total) -> int32_t {
+      if (cells) RUN_CUDA(cudaMemsetAsync(dev->lv, 0, (size_t)nb * sizeof(dev->lv[0]), st));  // (an empty batch adds nothing)
+      if (n > 0) {
+        RUN_CUDA(store.reserve((size_t)store_n0 + n, st));
+        RUN_CUDA(ls.newcnt.ensure((size_t)2 * n * 4 + 64));
+        rsc_cand* dst = store.cands[store.cur].as<rsc_cand>() + store_n0;
+        int32_t* cv = ls.newcnt.as<int32_t>();
+        int32_t* ce = cv + n;
+        if (d_total) {
+          append_new_kernel<<<std::max(1, std::min(n * 4 / 256, 64)), 256, 0, st>>>(fs.out, d_total, n, dst);
+          RUN_CUDA(cudaGetLastError());
+          if ((rc = score_small_enqueue(ctx, cloud, sps, th, dst, n, d_total, cv, ce, st))) return rc;
+        } else {
+          RUN_CUDA(cudaMemcpyAsync(dst, fs.out, (size_t)n * sizeof(rsc_cand), cudaMemcpyDeviceToDevice, st));
+          // (the culled scorer on the subset's Morton view when the batch is large: same counts)
+          if ((rc = loop_score_new(ctx, cloud, sub, sps, !ranged && !uo, th, dst, n, cv, ce, cv + 2 * n, st))) return rc;
+        }
+        if (uo && (rc = user_score_enqueue(ctx, *uo, sps, dst, n, d_total, cv, ce, st))) return rc;
+        if (coll && ctx->allreduce(ctx->allreduce_user, cv, (int64_t)2 * n + (d_total ? 0 : 1), (void*)st))
+          return fail(ctx, RSC_E_NCCL, "ransac_run: all-reduce of the counts failed");
+        int32_t* score = store.score[store.cur].as<int32_t>();
+        uint8_t* flags = store.flags[store.cur].as<uint8_t>();
+        finish_new_kernel<<<d_total ? std::max(1, std::min(n / 256, 64)) : (n + 255) / 256, 256, 0, st>>>(
+            dst, fs.total, n, cv, ce, th.honour_enabled, score + store_n0, flags + store_n0);
+        RUN_CUDA(cudaGetLastError());
+        seg_argmax_kernel<<<nb, 256, 0, st>>>(score, flags, dev->seg, store_n0, dev->seg_keys, n);  // never reads past the launch
+        RUN_CUDA(cudaGetLastError());
+        if (cells) {
+          level_stats_kernel<<<(n + 255) / 256, 256, 0, st>>>(fs.out_set, fs.level, score + store_n0, n, S, dev->lv);
+          RUN_CUDA(cudaGetLastError());
+        }
+      } else {
+        RUN_CUDA(cudaMemsetAsync(dev->seg_keys, 0xff, sizeof(dev->seg_keys), st));  // -1: no new candidate
+      }
+      if (store_n0 >= 1)
+        RUN_CUDA(argmax_enqueue(store.score[store.cur].as<int32_t>(), store.flags[store.cur].as<uint8_t>(), store_n0, dev->oldbest,
+                                ctx->sm_count, st));
+      return RSC_OK;
+    };
+    // ---- the decision of the batch -> hio->rec, with one synchronisation: decide_kernel, or the host's ----
+    auto decide = [&](const int32_t* d_ovf, int cap) -> int32_t {
+      if (!host) {
+        decide_kernel<<<1, kMaxBatch, 0, st>>>(dev, d_ovf, store_n0, nb, k, q, store.cands[store.cur].as<rsc_cand>(), cap);
+        RUN_CUDA(cudaGetLastError());
+        RUN_CUDA(cudaMemcpyAsync(&hio->rec, &dev->rec, sizeof(BatchRec), cudaMemcpyDeviceToHost, st));
+        RUN_CUDA(sync());
+        return RSC_OK;
+      }
+      const int n_new = hio->seg[nb];  // (host decisions never take the sync-free path: the bounds are on the host)
+      // (what it reads leads the device state: the arg-maxes, the segment bounds and this batch's level rows)
+      RUN_CUDA(cudaMemcpyAsync(&hio->dev, dev, offsetof(LoopDev, lv) + (cells ? nb : 0) * sizeof(dev->lv[0]), cudaMemcpyDeviceToHost, st));
+      hio->ovf = 0;
+      if (d_ovf) RUN_CUDA(cudaMemcpyAsync(&hio->ovf, d_ovf, 4, cudaMemcpyDeviceToHost, st));
+      if (prog && n_new > 0) {
+        newscore.resize(n_new);
+        RUN_CUDA(cudaMemcpyAsync(newscore.data(), store.score[store.cur].as<int32_t>() + store_n0, (size_t)n_new * 4,
+                                 cudaMemcpyDeviceToHost, st));
+      }
+      RUN_CUDA(sync());
+      hio->rec.ovf = hio->ovf ? 1 : 0;
+      return hio->ovf ? RSC_OK : host_decide(*host, hio->dev, newscore.data(), store_n0, nb, k, &hio->rec);
+    };
     // ---- sync-free path: K2 for a small batch, sized by a PREDICTION of the number of new candidates ----
     // (4 x the largest per-iteration yield seen so far; the true number stays on the device.  If more turn up,
-    // decide_kernel says so and the batch is scored again the classic way.)
+    // decide_kernel says so and the batch is scored again the classic way.)  The host decision needs the keys on
+    // the host, so it always takes the classic path.
     int cap_new = -1;
-    if (use_small && rate_seen >= 0) {
+    if (use_small && !host && rate_seen >= 0) {
       long long want = std::max<long long>(128, 4ll * rate_seen * nb + 64);
       if (const char* e = getenv("RSC_SMALL_CAP")) want = std::max(1, atoi(e));  // test hook: force undersized launches
       const long long cap = std::min<long long>((want + 127) / 128 * 128, (long long)maxnew * nb);
@@ -370,40 +436,12 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
       if (cap <= kSmallMaxCands && (double)(cap / 4) * (double)std::max<int64_t>(sps.n_pad, 1) <= kSmallMaxEvals) cap_new = (int)cap;
     }
     bool scored = false;
-    if (cap_new > 0) {
-      RUN_CUDA(store.reserve((size_t)store_n0 + cap_new, st));
-      RUN_CUDA(ls.newcnt.ensure((size_t)2 * cap_new * 4 + 64));
-      rsc_cand* dst = store.cands[store.cur].as<rsc_cand>() + store_n0;
-      int32_t* cv = ls.newcnt.as<int32_t>();
-      int32_t* ce = cv + cap_new;
-      append_new_kernel<<<std::max(1, std::min(cap_new * 4 / 256, 64)), 256, 0, st>>>(fs.out, fs.total, cap_new, dst);
-      RUN_CUDA(cudaGetLastError());
-      if ((rc = score_small_enqueue(ctx, cloud, sps, th, dst, cap_new, fs.total, cv, ce, st))) return rc;
-      if (uo && (rc = user_score_enqueue(ctx, *uo, sps, dst, cap_new, fs.total, cv, ce, st))) return rc;
-      if (coll && ctx->allreduce(ctx->allreduce_user, cv, (int64_t)2 * cap_new, (void*)st))
-        return fail(ctx, RSC_E_NCCL, "ransac_run: all-reduce of the counts failed");
-      finish_new_dev_kernel<<<std::max(1, std::min(cap_new / 256, 64)), 256, 0, st>>>(
-          dst, fs.total, cap_new, cv, ce, th.honour_enabled, store.score[store.cur].as<int32_t>() + store_n0,
-          store.flags[store.cur].as<uint8_t>() + store_n0);
-      RUN_CUDA(cudaGetLastError());
-      seg_argmax_kernel<<<nb, 256, 0, st>>>(store.score[store.cur].as<int32_t>(), store.flags[store.cur].as<uint8_t>(), dev->seg, store_n0,
-                                             dev->seg_keys, cap_new);  // never reads past the candidates this launch was sized for
-      RUN_CUDA(cudaGetLastError());
-      if (store_n0 >= 1) {
-        RUN_CUDA(argmax_enqueue(store.score[store.cur].as<int32_t>(), store.flags[store.cur].as<uint8_t>(), store_n0, dev->oldbest, ctx->sm_count, st));
-      }
-      decide_kernel<<<1, kMaxBatch, 0, st>>>(dev, nullptr, store_n0, nb, k, q, store.cands[store.cur].as<rsc_cand>(), cap_new);
-      RUN_CUDA(cudaGetLastError());
-      RUN_CUDA(cudaMemcpyAsync(&hio->rec, &dev->rec, sizeof(BatchRec), cudaMemcpyDeviceToHost, st));
-      RUN_CUDA(sync());
-      scored = hio->rec.ovf == 0;
-      if (scored) ctx->stats.evals += (int64_t)hio->rec.n_new * sps.n, ctx->stats.cands_scored += hio->rec.n_new;
-    }
     int n_new = 0;
-    if (scored) {
-      n_new = hio->rec.n_new;
-    } else if (cap_new > 0) {
-      n_new = hio->rec.n_new;  // known from the record of the undersized attempt
+    if (cap_new > 0) {
+      if ((rc = score_batch(cap_new, fs.total)) || (rc = decide(nullptr, cap_new))) return rc;
+      scored = hio->rec.ovf == 0;
+      n_new = hio->rec.n_new;  // (also known from the record of an undersized attempt)
+      if (scored) ctx->stats.evals += (int64_t)n_new * sps.n, ctx->stats.cands_scored += n_new;
     } else {
       RUN_CUDA(cudaMemcpyAsync(hio->seg, dev->seg, (size_t)(nb + 1) * 4, cudaMemcpyDeviceToHost, st));
       RUN_CUDA(sync());
@@ -412,40 +450,9 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
     rate_seen = std::max<long long>((n_new + nb - 1) / nb, rate_seen / 2);  // the yield falls as shapes are extracted: follow it
     const auto tk1 = now();
     t_fit += secs(tk0, tk1);
-    // ---- classic path: K2 (tiled) on subset 1 + K3 (repeated with a larger guard-band queue if that overflowed) ----
+    // ---- classic path: K2 (tiled or culled) + K3, repeated with a larger guard-band queue if that overflowed ----
     for (int attempt = 0; !scored; ++attempt) {
-      const int32_t* d_ovf = nullptr;
-      if (n_new > 0) {
-        RUN_CUDA(store.reserve((size_t)store_n0 + n_new, st));
-        rsc_cand* dst = store.cands[store.cur].as<rsc_cand>() + store_n0;
-        RUN_CUDA(cudaMemcpyAsync(dst, fs.out, (size_t)n_new * sizeof(rsc_cand), cudaMemcpyDeviceToDevice, st));
-        int32_t* cv = ls.newcnt.as<int32_t>();
-        int32_t* ce = cv + n_new;
-        // (the culled scorer on the subset's Morton view when the batch is large: same counts)
-        // the overflow flag rides behind the counts, so that a sharded run decides to repeat collectively
-        if ((rc = loop_score_new(ctx, cloud, sub, sps, !ranged && !uo, th, dst, n_new, cv, ce, cv + 2 * n_new, st))) return rc;
-        if (uo && (rc = user_score_enqueue(ctx, *uo, sps, dst, n_new, nullptr, cv, ce, st))) return rc;
-        if (coll && ctx->allreduce(ctx->allreduce_user, cv, (int64_t)2 * n_new + 1, (void*)st))
-          return fail(ctx, RSC_E_NCCL, "ransac_run: all-reduce of the counts failed");
-        finish_new_kernel<<<(n_new + 255) / 256, 256, 0, st>>>(dst, n_new, cv, ce, th.honour_enabled,
-                                                               store.score[store.cur].as<int32_t>() + store_n0,
-                                                               store.flags[store.cur].as<uint8_t>() + store_n0);
-        RUN_CUDA(cudaGetLastError());
-        seg_argmax_kernel<<<nb, 256, 0, st>>>(store.score[store.cur].as<int32_t>(), store.flags[store.cur].as<uint8_t>(), dev->seg,
-                                               store_n0, dev->seg_keys);
-        RUN_CUDA(cudaGetLastError());
-        d_ovf = cv + 2 * n_new;
-      } else {
-        RUN_CUDA(cudaMemsetAsync(dev->seg_keys, 0xff, sizeof(dev->seg_keys), st));  // -1: no new candidate
-      }
-      if (store_n0 >= 1) {
-        RUN_CUDA(argmax_enqueue(store.score[store.cur].as<int32_t>(), store.flags[store.cur].as<uint8_t>(), store_n0,
-                                          dev->oldbest, ctx->sm_count, st));
-      }
-      decide_kernel<<<1, kMaxBatch, 0, st>>>(dev, d_ovf, store_n0, nb, k, q, store.cands[store.cur].as<rsc_cand>(), -1);
-      RUN_CUDA(cudaGetLastError());
-      RUN_CUDA(cudaMemcpyAsync(&hio->rec, &dev->rec, sizeof(BatchRec), cudaMemcpyDeviceToHost, st));
-      RUN_CUDA(sync());
+      if ((rc = score_batch(n_new, nullptr)) || (rc = decide(n_new > 0 ? ls.newcnt.as<int32_t>() + 2 * n_new : nullptr, -1))) return rc;
       if (!hio->rec.ovf) break;
       if (attempt >= 4) return fail(ctx, RSC_E_STATE, "ransac_run: guard-band queue kept overflowing");
       if ((rc = grow_guard_queue(ctx))) return rc;
@@ -457,6 +464,16 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
     store.n = rec.store_n;
     terminated = rec.terminated != 0;
     if (rec.extract) {
+      // K5's source of the newly disabled points: the subset's Morton view when it has one and the run scores the
+      // whole subset (the points then come out spatially sorted, and the culled scorer can take them: the SET of
+      // points is the same), else this rank's slice.  Its enabled words of before the extraction are kept.
+      const bool view = sub.cen != nullptr && !coll;
+      const PointSet src = view ? view_subset_morton(&sub) : sps;
+      const bool exact = src.xyz64 != nullptr;
+      const int64_t swords = sub.m_pad / 32;
+      RUN_CUDA(ls.olden.ensure((size_t)swords * 4));
+      const uint32_t* old_src = ls.olden.as<uint32_t>() + (view ? 0 : sps_word0);
+      RUN_CUDA(cudaMemcpyAsync(ls.olden.p, view ? sub.cen : sub.enabled, (size_t)swords * 4, cudaMemcpyDeviceToDevice, st));
       // ---- K4: refit over this rank's points, invalidate them ----
       rsc_cand shape = rec.best;
       if (p->compat_flags & RSC_REFIT_LSQ) {  // extension: the paper's least-squares refit within 3 eps
@@ -465,9 +482,6 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
       }
       Thresh thr = th;
       thr.honour_enabled = 0xFu;
-      const int64_t swords = sub.m_pad / 32;
-      RUN_CUDA(ls.olden.ensure((size_t)swords * 4));
-      RUN_CUDA(cudaMemcpyAsync(ls.olden.p, sub.enabled, (size_t)swords * 4, cudaMemcpyDeviceToDevice, st));
       if (shape.type >= RSC_USER_TYPE0) {
         if ((rc = user_refit_mask_enqueue(cloud, *uo, shape, st))) return rc;
       } else if ((rc = refit_mask_enqueue(cloud, thr, shape, st))) {
@@ -495,44 +509,57 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
         if ((rc = shard_clear_enabled(cloud, ctx->idxbuf.as<uint32_t>(), dev->tot_global, 1, dev->tot_global, st))) return rc;
       }
       // ---- K5: drop the best and every candidate compatible with a newly disabled subset point ----
-      // Gathered form: the newly disabled points of this rank's subset slice go into a compact scratch
-      // set.  Their number is only known on the device, but it cannot exceed the candidate's subset
-      // score (every one of them was a compatible, enabled subset point when the candidate was scored;
-      // the enabled set only shrinks), which the host has from the decision record: that sizes the
-      // launch without a round trip.  Masked form (the least-squares refit moves the shape, so the bound
-      // does not hold; also the fallback): score against the whole slice under the mask old & ~new.
+      // Gathered form: the newly disabled points of the source go into a compact scratch set.  Their number is
+      // only known on the device, but it cannot exceed the candidate's subset-1 score in the store (every one of
+      // them was a compatible, enabled subset point when the candidate was scored; the enabled set only shrinks),
+      // which the host has from the decision record: that sizes the launch without a round trip.  Masked form (the
+      // least-squares refit moves the shape, so the bound does not hold; also the fallback): score against the
+      // whole source under the mask old & ~new.
       const int nst = store.n;
       // (the bitmap filter only removes points from the list, so the bound still holds with it)
       bool masked = (p->compat_flags & RSC_REFIT_LSQ) != 0 || getenv("RSC_K5_MASKED") != nullptr;
-      PointSet dps = sps;
+      PointSet dps = src;
+      const float4* tiles = view ? static_cast<const float4*>(sub.ctiles) : nullptr;  // the culled scorer's spheres of dps
       // hit counts [nst] + two flags that ride with them through the all-reduce: guard-band queue overflow,
       // scratch set too small
       RUN_CUDA(ctx->counts.ensure(((size_t)3 * nst + 8) * 4));
       int32_t* hit = ctx->counts.as<int32_t>() + 2 * (size_t)nst;
       int32_t* d_over = hit + nst + 1;
       RUN_CUDA(cudaMemsetAsync(d_over, 0, 4, st));
-      const int64_t sl_words = sps.n_pad / 32;
+      // scratch: [wcnt: sl_words u32][woff: sl_words + 1 u64][keep: nst u32][koff: nst + 1 u64]
+      const int64_t sl_words = src.n_pad / 32;
+      const size_t o_woff = ((size_t)sl_words * 4 + 255) / 256 * 256;
+      const size_t o_keep = o_woff + ((size_t)(sl_words + 1) * 8 + 255) / 256 * 256;
+      const size_t o_koff = o_keep + ((size_t)nst * 4 + 255) / 256 * 256;
+      RUN_CUDA(ls.nmeta.ensure(o_koff + (size_t)(nst + 1) * 8));
+      uint32_t* wcnt = ls.nmeta.as<uint32_t>();
+      unsigned long long* woff = (unsigned long long*)(ls.nmeta.as<char>() + o_woff);
+      unsigned long long* wtot = woff + sl_words;
+      uint32_t* keep = (uint32_t*)(ls.nmeta.as<char>() + o_keep);
+      unsigned long long* koff = (unsigned long long*)(ls.nmeta.as<char>() + o_koff);
+      unsigned long long* ktot = koff + nst;
+      // the culled scorer (built-in types only) on a view-ordered set when the store is large: most stored candidates
+      // are then nowhere near the extracted shape, and the dense path's candidate compiler is ONE CTA (3 ms for a
+      // store of a million candidates, the cell sampler's)
+      auto culled = [&](int64_t npts) {
+        return view && !uo && k5_cull_mode != 0 && (k5_cull_mode == 2 || nst >= 4096 || (double)nst * (double)npts >= 2e8);
+      };
       if (!masked && sl_words > 0) {
         const int64_t cap = ((int64_t)std::max(rec.best_score, 1) + kTile - 1) / kTile * kTile;
-        const size_t o_woff = ((size_t)sl_words * 4 + 255) / 256 * 256;
-        RUN_CUDA(ls.prog.ensure(o_woff + (size_t)(sl_words + 2) * 8 + 64));
-        uint32_t* wcnt = ls.prog.as<uint32_t>();
-        unsigned long long* woff = (unsigned long long*)(ls.prog.as<char>() + o_woff);
-        unsigned long long* wtot = woff + sl_words;
-        const uint32_t* old_sl = ls.olden.as<uint32_t>() + sps_word0;
-        newly_count_kernel<<<(unsigned)((sl_words + 255) / 256), 256, 0, st>>>(old_sl, sps.enabled, sl_words, wcnt);
+        newly_count_kernel<<<(unsigned)((sl_words + 255) / 256), 256, 0, st>>>(old_src, src.enabled, sl_words, wcnt);
         RUN_CUDA(cudaGetLastError());
         if ((rc = scan_u32(ctx, wcnt, (int)sl_words, woff, wtot, st))) return rc;
         RUN_CUDA(ls.nscratch.ensure((size_t)6 * cap * 4));
         RUN_CUDA(ls.nvalid.ensure((size_t)(cap / 32) * 4));
         RUN_CUDA(cudaMemsetAsync(ls.nscratch.p, 0, (size_t)6 * cap * 4, st));
-        if (sps.map) {  // (entries past the gathered count stay 0: padding lanes may still look their point up)
+        if (exact) {  // the scratch set's map into the float64 coordinates, the source's map gathered
+          // (entries past the gathered count stay 0: padding lanes may still look their point up)
           RUN_CUDA(ls.nidx.ensure((size_t)cap * sizeof(int64_t)));
           RUN_CUDA(cudaMemsetAsync(ls.nidx.p, 0, (size_t)cap * sizeof(int64_t), st));
         }
         newly_gather_capped_kernel<<<(unsigned)((sl_words + 255) / 256), 256, 0, st>>>(
-            old_sl, sps.enabled, sl_words, woff, wtot, sps.x, sps.y - sps.x, ls.nscratch.as<float>(), cap, d_over, sps.map,
-            sps.map ? ls.nidx.as<int64_t>() : nullptr);
+            old_src, src.enabled, sl_words, woff, wtot, src.x, src.y - src.x, ls.nscratch.as<float>(), cap, d_over, src.map,
+            exact ? ls.nidx.as<int64_t>() : nullptr);
         RUN_CUDA(cudaGetLastError());
         fill_valid_dev_kernel<<<(unsigned)((cap / 32 + 255) / 256), 256, 0, st>>>(ls.nvalid.as<uint32_t>(), wtot, cap / 32);
         RUN_CUDA(cudaGetLastError());
@@ -540,40 +567,40 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
         dps.x = b, dps.y = b + cap, dps.z = b + 2 * cap, dps.nx = b + 3 * cap, dps.ny = b + 4 * cap, dps.nz = b + 5 * cap;
         dps.enabled = dps.valid = ls.nvalid.as<uint32_t>();
         dps.n = dps.n_pad = cap;
-        if (sps.map) dps.map = ls.nidx.as<int64_t>();
+        dps.map = exact ? ls.nidx.as<int64_t>() : nullptr;
+        if (culled(cap)) {  // spheres of the gathered points only: the zero padding stays out of them
+          RUN_CUDA(ls.ntiles.ensure(cull_sphere_count(cap) * sizeof(float4)));
+          if ((rc = cull_tile_spheres(ctx, dps, ls.ntiles.as<float4>(), st, wtot))) return rc;
+          tiles = ls.ntiles.as<float4>();
+        }
       }
       auto mask_form = [&]() -> cudaError_t {
-        newly_mask_kernel<<<(unsigned)((swords + 255) / 256), 256, 0, st>>>(ls.olden.as<uint32_t>(), sub.enabled, swords);
-        dps = sps;
-        dps.enabled = ls.olden.as<uint32_t>() + sps_word0;
+        newly_mask_kernel<<<(unsigned)((swords + 255) / 256), 256, 0, st>>>(ls.olden.as<uint32_t>(), view ? sub.cen : sub.enabled, swords);
+        dps = src;
+        dps.enabled = dps.valid = old_src;  // (only the enabled-gated counts are read)
+        tiles = view ? static_cast<const float4*>(sub.ctiles) : nullptr;
         masked = true;
         cudaMemsetAsync(d_over, 0, 4, st);
         return cudaGetLastError();
       };
       if (masked) RUN_CUDA(mask_form());
-      const size_t o_koff = ((size_t)nst * 4 + 255) / 256 * 256;
-      RUN_CUDA(ls.nmeta.ensure(o_koff + (size_t)(nst + 1) * 8));
-      uint32_t* keep = ls.nmeta.as<uint32_t>();
-      unsigned long long* koff = (unsigned long long*)(ls.nmeta.as<char>() + o_koff);
-      unsigned long long* ktot = koff + nst;
       int nxt = store.cur ^ 1;
       for (int attempt = 0;; ++attempt) {
         // enabled-gated counts over the newly disabled points = hits
-        if (use_small && nst <= kSmallMaxCands && (double)nst * (double)std::max<int64_t>(dps.n_pad, 1) <= kSmallMaxEvals) {
-          if ((rc = score_small_enqueue(ctx, cloud, dps, th, store.cands[store.cur].as<rsc_cand>(), nst, nullptr,
-                                        ctx->counts.as<int32_t>(), hit, st)))
-            return rc;
+        const rsc_cand* cands = store.cands[store.cur].as<rsc_cand>();
+        if (culled(dps.n)) {
+          if ((rc = cull_enqueue(ctx, cloud, dps, tiles, th, cands, nst, nullptr, ctx->counts.as<int32_t>(), hit, nullptr, st))) return rc;
+          RUN_CUDA(cudaMemsetAsync(hit + nst, 0, 4, st));  // nothing can overflow: pairs beyond the queue are decided inline
+        } else if (use_small && nst <= kSmallMaxCands && (double)nst * (double)std::max<int64_t>(dps.n_pad, 1) <= kSmallMaxEvals) {
+          if ((rc = score_small_enqueue(ctx, cloud, dps, th, cands, nst, nullptr, ctx->counts.as<int32_t>(), hit, st))) return rc;
           RUN_CUDA(cudaMemsetAsync(hit + nst, 0, 4, st));  // no guard-band queue on this path
         } else {
-          if ((rc = score_enqueue(ctx, cloud, dps, th, store.cands[store.cur].as<rsc_cand>(), nst, nullptr, false, st,
-                                  ctx->counts.as<int32_t>(), hit)))
-            return rc;
+          if ((rc = score_enqueue(ctx, cloud, dps, th, cands, nst, nullptr, false, st, ctx->counts.as<int32_t>(), hit))) return rc;
           queue_overflow_kernel<<<1, 1, 0, st>>>(ctx->wl_count.as<uint32_t>(), (uint32_t)ctx->wl_cap, hit + nst);
           RUN_CUDA(cudaGetLastError());
         }
         // user records: the built-in scorers left their hits at 0 (enabled-gated counts, so the scratch bound holds)
-        if (uo && (rc = user_score_enqueue(ctx, *uo, dps, store.cands[store.cur].as<rsc_cand>(), nst, nullptr, nullptr, hit, st)))
-          return rc;
+        if (uo && (rc = user_score_enqueue(ctx, *uo, dps, cands, nst, nullptr, nullptr, hit, st))) return rc;
         if (coll && ctx->allreduce(ctx->allreduce_user, hit, (int64_t)nst + 2, (void*)st))
           return fail(ctx, RSC_E_NCCL, "ransac_run: all-reduce of the K5 hits failed");
         invalidate_kernel<<<(nst + 255) / 256, 256, 0, st>>>(hit, store.flags[store.cur].as<uint8_t>(), nst, rec.best_idx, keep);
@@ -586,6 +613,10 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
         k5_pack_kernel<<<1, 1, 0, st>>>(dev, ktot, hit + nst, d_over, ctx->misc2.as<unsigned long long>(), dk5);
         RUN_CUDA(cudaGetLastError());
         RUN_CUDA(cudaMemcpyAsync(&hio->k5, dk5, sizeof(K5Host), cudaMemcpyDeviceToHost, st));
+        if (host && prog) {
+          keep_h.resize(nst);
+          RUN_CUDA(cudaMemcpyAsync(keep_h.data(), keep, (size_t)nst * 4, cudaMemcpyDeviceToHost, st));
+        }
         RUN_CUDA(sync());
         if (!hio->k5.ovf) break;
         if (hio->k5.ovf & 2) {  // (not expected) more newly disabled points than the bound: masked form
@@ -597,6 +628,7 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
         if (attempt >= 4) return fail(ctx, RSC_E_STATE, "ransac_run: guard-band queue kept overflowing");
         if ((rc = grow_guard_queue(ctx))) return rc;
       }
+      if (host && prog) host_compacted(*host, keep_h);
       const int64_t total_local = (int64_t)hio->k5.total_local;
       const int64_t total = shard ? (int64_t)hio->k5.tot_global : total_local;
       run->shapes.push_back(shape);
@@ -623,7 +655,7 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
   RUN_CUDA(sync());
   if (trace)
     fprintf(stderr,
-            "[rsc_ransac_run/device] iterations %d shapes %zu batches %d syncs %d | sample+fit %.1f ms, score+decide %.1f ms, "
+            "[rsc_ransac_run] iterations %d shapes %zu batches %d syncs %d | sample+fit %.1f ms, score+decide %.1f ms, "
             "refit+invalidate %.1f ms | all-reduces %lld (%.1f MB)\n",
             run->iterations, run->shapes.size(), run->batches, run->syncs, 1e3 * t_fit, 1e3 * t_score, 1e3 * t_extract,
             (long long)ctx->allreduce_calls, ctx->allreduce_bytes / 1e6);

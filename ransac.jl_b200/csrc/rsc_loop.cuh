@@ -1,6 +1,6 @@
-// rsc_loop.cuh -- kernels and device-side structures shared by the two loops behind rsc_ransac_run
-// (rsc_loop.cu: the reference behaviour with the bookkeeping decided on the device; rsc_run.cu: the
-// host-walked loop of the extension switches).  Included by both translation units (static kernels).
+// rsc_loop.cuh -- kernels and structures of the RANSAC loop (rsc_loop.cu) and what the host decision of the
+// extension switches (rsc_run.cu) shares with it: the candidate store, the loop's device state and decision
+// record, the slice of a subset a rank scores, the guard-band queue retry and the run object.
 #pragma once
 #include <vector>
 
@@ -9,16 +9,18 @@
 namespace rsc {
 
 // ---- K3: scores of the freshly scored candidates, arg-max over the store -------------------------
-// score = policy count; tainted = sphere whose count includes a disabled point (Q4)
-static __global__ void finish_new_kernel(const rsc_cand* __restrict__ cands, int n, const int32_t* __restrict__ cv,
-                                  const int32_t* __restrict__ ce, uint32_t honour_enabled, int32_t* __restrict__ score,
-                                  uint8_t* __restrict__ flags) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  const int t = cands[i].type;
-  const bool honour = t >= RSC_NTYPES || ((honour_enabled >> t) & 1u);  // user shapes honour the enabled mask
-  score[i] = honour ? ce[i] : cv[i];
-  flags[i] = (uint8_t)(1u | ((!honour && cv[i] != ce[i]) ? 2u : 0u));  // bit0 alive, bit1 tainted
+// score = policy count; tainted = sphere whose count includes a disabled point (Q4).  The candidates are the
+// first min(*total, cap) of the launch (the sync-free path sizes it by a prediction, the classic one exactly).
+static __global__ void finish_new_kernel(const rsc_cand* __restrict__ cands, const unsigned long long* __restrict__ total, int cap,
+                                         const int32_t* __restrict__ cv, const int32_t* __restrict__ ce, uint32_t honour_enabled,
+                                         int32_t* __restrict__ score, uint8_t* __restrict__ flags) {
+  const int n = (int)min(*total, (unsigned long long)cap);
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    const int t = cands[i].type;
+    const bool honour = t >= RSC_NTYPES || ((honour_enabled >> t) & 1u);  // user shapes honour the enabled mask
+    score[i] = honour ? ce[i] : cv[i];
+    flags[i] = (uint8_t)(1u | ((!honour && cv[i] != ce[i]) ? 2u : 0u));  // bit0 alive, bit1 tainted
+  }
 }
 
 // first index of the maximum score among alive candidates (ties: first wins, Q16)
@@ -111,34 +113,6 @@ static __global__ void newly_count_kernel(const uint32_t* __restrict__ old_en, c
   if (w < words) cnt[w] = __popc(old_en[w] & ~new_en[w]);
 }
 
-// gather the newly disabled subset points into a compact SoA scratch set
-// (exact clouds: idx / out_idx non-null, the cloud index of every gathered point, the map of the scratch set)
-static __global__ void newly_gather_kernel(const uint32_t* __restrict__ old_en, const uint32_t* __restrict__ new_en, int64_t words,
-                                    const unsigned long long* __restrict__ offs, const float* __restrict__ soa, int64_t m_pad,
-                                    float* __restrict__ out, int64_t out_pad, const int64_t* __restrict__ idx,
-                                    int64_t* __restrict__ out_idx) {
-  const int64_t w = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (w >= words) return;
-  uint32_t bits = old_en[w] & ~new_en[w];
-  unsigned long long o = offs[w];
-  while (bits) {
-    const int b = __ffs(bits) - 1;
-    bits &= bits - 1;
-    const int64_t j = w * 32 + b;
-#pragma unroll
-    for (int f = 0; f < 6; ++f) out[f * out_pad + o] = soa[f * m_pad + j];
-    if (out_idx) out_idx[o] = idx[j];
-    ++o;
-  }
-}
-
-static __global__ void fill_valid_words_kernel(uint32_t* __restrict__ valid, int64_t n, int64_t words) {
-  const int64_t w = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (w >= words) return;
-  const int64_t lo = w * 32;
-  valid[w] = lo + 32 <= n ? 0xffffffffu : (lo < n ? (1u << (n - lo)) - 1u : 0u);
-}
-
 // alive &= no newly disabled compatible point; tainted spheres die; keep[] = alive as 0/1 words
 static __global__ void invalidate_kernel(const int32_t* __restrict__ hit, uint8_t* __restrict__ flags, int n, int best,
                                   uint32_t* __restrict__ keep) {
@@ -199,8 +173,55 @@ struct Store {
 // device buffers per run cost 10-25 ms of a 40 ms loop)
 struct LoopScratch {
   Store store;
-  DevBuf newcnt, hostio, olden, nscratch, nidx, nvalid, nmeta, lvbuf, prog, ntiles;
+  DevBuf newcnt, hostio, olden, nscratch, nidx, nvalid, nmeta, prog, ntiles;
 };
+
+constexpr int kMaxBatch = 64;  // most iterations of one speculative batch
+
+struct BatchRec {  // the decision of one batch (decide_kernel's record, or the host's): device -> host, once per batch
+  long long counters[3];
+  int32_t used, extract, terminated, iterations;
+  int32_t best_idx, best_score, store_n, ovf;  // ovf: 1 = a guard-band queue overflowed, 2 = more new candidates than the launch was sized for
+  int32_t n_new, pad;
+  rsc_cand best;
+};
+
+struct LoopDev {  // device-resident scratch + state of one run
+  int64_t oldbest[2];             // arg-max over the store as it was before the batch: index, score
+  long long seg_keys[kMaxBatch];  // per batch iteration: arg-max key over its new candidates
+  int32_t seg[kMaxBatch + 2];     // per batch iteration: first new candidate
+  long long lv[kMaxBatch][22];    // cell sampler, per batch iteration and octree level: new candidates, sum of their scores
+  // (the host decision reads the fields above, up to this batch's rows of lv)
+  long long counters[3];          // countcandidates: lengthC, allcand, nofminset (iterations.jl:70)
+  BatchRec rec;
+  int32_t tot_global[2];          // sharded storage: inliers of the extraction summed over the ranks
+};
+
+// This rank's slice of a subset copy: all of it (single GPU, or a shard's local entries) or, on replicated storage
+// with a point range (`ranged`), the same fraction of it as the rank's range of the cloud.
+inline PointSet subset_slice(const rsc_cloud* cloud, const rsc_subset& sb, bool ranged) {
+  PointSet v = view_subset(&sb);
+  if (!ranged || cloud->n_pad <= 0) return v;
+  const int64_t lo = (int64_t)((double)cloud->range_lo / cloud->n_pad * sb.m_pad) / kTile * kTile;
+  const int64_t hi = cloud->range_hi >= cloud->n_pad ? sb.m_pad : (int64_t)((double)cloud->range_hi / cloud->n_pad * sb.m_pad) / kTile * kTile;
+  v.x += lo, v.y += lo, v.z += lo, v.nx += lo, v.ny += lo, v.nz += lo;
+  v.enabled += lo / 32, v.valid += lo / 32;
+  if (v.map) v.map += lo;
+  v.n_pad = std::max<int64_t>(0, hi - lo);
+  v.n = std::max<int64_t>(0, std::min(sb.m, hi) - lo);
+  return v;
+}
+
+// The host decision of a batch (rsc_run.cu), taken instead of decide_kernel's when RSC_SCORE_PROGRESSIVE,
+// RSC_SAMPLER_OCTREE or RSC_LOOP_HOSTWALK is set.  `d` is the host copy of the device state after K2 + K3,
+// `newscore` the new candidates' subset-1 scores (progressive scoring).  Fills *rec like decide_kernel does.
+struct HostWalk;
+int32_t host_decide(HostWalk& w, const LoopDev& d, const int32_t* newscore, int store_n0, int nb, int k0, BatchRec* rec);
+// after K5: keep[i] = 1 for the store entries that survived (progressive scoring compacts its host mirror with it)
+void host_compacted(HostWalk& w, const std::vector<uint32_t>& keep);
+// the loop behind rsc_ransac_run / rsc_ransac_run_user.  order (nullable): a mixed fit order in place of
+// p->shape_types; host (nullable): the host decision, else decide_kernel's
+int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed, rsc_run* run, const FitOrder* order, HostWalk* host);
 
 }  // namespace rsc
 

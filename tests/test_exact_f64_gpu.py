@@ -240,7 +240,7 @@ def _loop_scene(n, seed):
 
 
 @pytest.mark.parametrize("scene,loop", [("c1", "default"), ("c1", "cull_always"), ("c1", "cull_never"), ("c1", "hostwalk"),
-                                        ("1Mi", "default"), ("1Mi", "cull_always")])
+                                        ("c1", "hostwalk_cull_always"), ("1Mi", "default"), ("1Mi", "cull_always")])
 def test_ransac_on_exact_cloud_equals_c_oracle_on_unrounded_input(R, monkeypatch, scene, loop):
     from tests.test_ransac_gpu import _compare_runs
 
@@ -250,9 +250,11 @@ def test_ransac_on_exact_cloud_equals_c_oracle_on_unrounded_input(R, monkeypatch
     else:
         V, N = _loop_scene(1 << 20, 32)
         nsub, params, seed = 8, R.ransacparameters(iteration={"tau": 3000, "minsubsetN": 256, "itermax": 40}), 99
-    env = {"cull_always": ("RSC_LOOP_CULL", "2"), "cull_never": ("RSC_LOOP_CULL", "0"), "hostwalk": ("RSC_LOOP_HOSTWALK", "1")}
-    if loop in env:
-        monkeypatch.setenv(*env[loop])
+    cull_always, hostwalk = ("RSC_LOOP_CULL", "2"), ("RSC_LOOP_HOSTWALK", "1")
+    env = {"cull_always": [cull_always], "cull_never": [("RSC_LOOP_CULL", "0")], "hostwalk": [hostwalk],
+           "hostwalk_cull_always": [hostwalk, cull_always]}
+    for kv in env.get(loop, []):
+        monkeypatch.setenv(*kv)
     pc = R.RANSACCloud(V, N, nsub, exact=True)
     extracted, _ = R.ransac(pc, params, True, seed=seed)
     want, en, _ = CO.ransac(V, N, pc.subsets[0], oracle_params(params), seed)

@@ -147,3 +147,21 @@ def test_reference_grid_leaf_depth(R):
         _, perm, ld = pc.get_cells()
         assert (ld == 3).all()
         np.testing.assert_array_equal(perm.astype(np.int64), O.MortonOctree(ps, nlevels).perm)
+
+
+def test_cell_sampler_with_empty_batches_matches_oracle(R):
+    """one plane type, one set per iteration: most iterations fit no candidate, so most batches are empty -- their
+    level statistics must add nothing to the level scores"""
+    sc = _scene(20_000, seed=94)
+    subsets = R.makesubsets(len(sc.vertices), 2, np.random.default_rng(1234))
+    params = R.ransacparameters([R.FittedPlane], iteration={"tau": 200, "minsubsetN": 1, "itermax": 300})
+    pc = R.RANSACCloud(sc.vertices, sc.normals, subsets).build_cells(8)
+    extracted, _ = R.ransac(pc, params, True, seed=17, sampler="octree")
+    oc = O.MortonOctree(sc.vertices, 8)
+    opc = O.Cloud(sc.vertices, sc.normals, [s.copy() for s in subsets])
+    tr = O.RansacTrace()
+    want = O.ransac(opc, oracle_params(params), True, seed=17, trace=tr, octree=oc)
+    assert tr.candidates_scored < tr.iterations  # (at most one candidate per iteration: some iterations had none)
+    assert len(extracted) == len(want)
+    np.testing.assert_array_equal(pc.isenabled, opc.isenabled)
+    np.testing.assert_allclose(pc.levelweight, tr.levelweight, rtol=1e-12)
