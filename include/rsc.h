@@ -230,6 +230,27 @@ int32_t rsc_score_dev_masks(rsc_cloud* cloud, const rsc_params* params, const rs
  * margins are nullable. */
 int32_t rsc_debug_margins(rsc_cloud* cloud, const rsc_params* params, const rsc_cand* cands, int32_t C, int64_t point0,
                           int64_t npoints, float* margins, float* bands, int32_t* col_types, int64_t* packed_vs_scalar_diffs);
+/* Test hook for the device loop's small-batch scorer (the one it uses for a batch of new candidates and for
+ * re-scoring a small store after an extraction): the same launch, on the whole cloud (subset_id = -1) or an
+ * uploaded subset.  cv[C] = compatible real points, ce[C] = compatible enabled points, whatever the shape type
+ * (the sphere quirk Q4 picks between them later).  Type ids outside 0..3 compile to no column and count 0.
+ * count >= 0: the number of candidates is read from device memory and C is the capacity, as in the loop's
+ * synchronisation-free path (entries count..C-1 come back 0; count > C scores C). */
+int32_t rsc_debug_score_small(rsc_cloud* cloud, const rsc_params* params, int32_t subset_id, const rsc_cand* cands, int32_t C,
+                              int64_t count, int32_t* cv, int32_t* ce);
+/* Test hook for K5, the device loop's re-scoring of its candidate store after an extraction.  cands[nst] = the
+ * store; the cloud's current enabled mask is the one of before the extraction, new_enabled (packed like
+ * rsc_cloud_set_enabled) the one after, which the cloud keeps.  hit[i] = the number of subset-0 points that were
+ * enabled before and are not after and are compatible with candidate i (all of them counted as enabled).  The
+ * source of those points is subset 0 itself or (form bit 1) its Morton view, built if needed; the form is the
+ * gathered one, in a scratch set sized by `bound` (in the loop: the extracted candidate's subset score), or (form
+ * bit 0) the masked one.  A gathered attempt whose points do not fit is repeated in the masked form, as the loop
+ * does.  The scorer follows RSC_LOOP_CULL and RSC_NO_SMALL like the loop's.  flags[2] (nullable) = the first
+ * attempt's guard-band queue overflow and scratch overflow; survivors[nst] (nullable) = the indices of the candidates
+ * that stay in the store, in order (not `best`, no hit), *n_survivors their number (nullable). */
+int32_t rsc_debug_k5_hits(rsc_cloud* cloud, const rsc_params* params, const rsc_cand* cands, int32_t nst, const uint64_t* new_enabled,
+                          int32_t bound, int32_t form, int32_t best, int32_t* hit, int32_t* flags, int32_t* survivors,
+                          int32_t* n_survivors);
 /* Measurement hook for K4 (HBM bound): average duration (ms) of the refit's compatibility-mask kernel over
  * `reps` back-to-back launches between ONE CUDA-event pair (an event pair around a single ~70 us launch
  * over-reads it by the event latency).  Nothing is extracted or disabled. */

@@ -99,6 +99,9 @@ SIGNATURES = {
     "rsc_score_dev": (C.c_int32, [_P, C.POINTER(rsc_params), _P, C.c_int32, C.c_int32, _P, _P]),
     "rsc_score_dev_masks": (C.c_int32, [_P, C.POINTER(rsc_params), _P, C.c_int32, C.c_int32, _P, _P, _P]),
     "rsc_debug_margins": (C.c_int32, [_P, C.POINTER(rsc_params), _P, C.c_int32, C.c_int64, C.c_int64, _P, _P, _P, C.POINTER(C.c_int64)]),
+    "rsc_debug_score_small": (C.c_int32, [_P, C.POINTER(rsc_params), C.c_int32, _P, C.c_int32, C.c_int64, _P, _P]),
+    "rsc_debug_k5_hits": (C.c_int32, [_P, C.POINTER(rsc_params), _P, C.c_int32, _P, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P,
+                                       C.POINTER(C.c_int32)]),
     "rsc_debug_refit_mask_ms": (C.c_int32, [_P, C.POINTER(rsc_params), C.POINTER(rsc_cand), C.c_int32, C.POINTER(C.c_double), C.POINTER(C.c_int64)]),
     "rsc_estimate_score": (None, [C.c_int64, C.c_int64, C.c_int64, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_double)]),
     "rsc_fit_batch": (C.c_int32, [_P, C.POINTER(rsc_params), _P, C.c_int32, _P, _P, C.POINTER(C.c_int32)]),

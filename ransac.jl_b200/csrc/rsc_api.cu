@@ -377,6 +377,36 @@ int32_t rsc_debug_margins(rsc_cloud* cloud, const rsc_params* params, const rsc_
   return RSC_OK;
 }
 
+// Test hook: the small-batch scorer (rsc_small.cu) as the device loop launches it, on a cloud or a subset.
+int32_t rsc_debug_score_small(rsc_cloud* cloud, const rsc_params* params, int32_t subset_id, const rsc_cand* cands, int32_t C,
+                              int64_t count, int32_t* cv, int32_t* ce) {
+  if (!cloud) return RSC_E_ARG;
+  rsc_ctx* ctx = cloud->ctx;
+  if (C <= 0 || !cands || !cv || !ce) return fail(ctx, RSC_E_ARG, "debug_score_small: bad arguments (C >= 1, non-null buffers)");
+  int32_t rc = check_params(ctx, params);
+  if (rc) return rc;
+  RSC_CUDA(ctx, cudaSetDevice(ctx->device));
+  if ((rc = cloud_ready(cloud))) return rc;
+  PointSet ps;
+  if ((rc = pick_pointset(cloud, subset_id, &ps))) return rc;
+  cudaStream_t st = ctx->stream;
+  // [candidates][cv: C][ce: C][count: u64]
+  const size_t o_cnt = ((size_t)C * sizeof(rsc_cand) + 255) / 256 * 256, o_n = o_cnt + ((size_t)2 * C * 4 + 255) / 256 * 256;
+  RSC_CUDA(ctx, ctx->cullbuf.ensure(o_n + 8));
+  char* b = ctx->cullbuf.as<char>();
+  int32_t* d_cv = (int32_t*)(b + o_cnt);
+  unsigned long long* d_n = (unsigned long long*)(b + o_n);
+  const unsigned long long n = count >= 0 ? (unsigned long long)count : 0ull;
+  RSC_CUDA(ctx, cudaMemcpyAsync(b, cands, (size_t)C * sizeof(rsc_cand), cudaMemcpyHostToDevice, st));
+  RSC_CUDA(ctx, cudaMemcpyAsync(d_n, &n, 8, cudaMemcpyHostToDevice, st));
+  if ((rc = score_small_enqueue(ctx, cloud, ps, make_thresh(params), (const rsc_cand*)b, C, count >= 0 ? d_n : nullptr, d_cv, d_cv + C, st)))
+    return rc;
+  RSC_CUDA(ctx, cudaMemcpyAsync(cv, d_cv, (size_t)C * 4, cudaMemcpyDeviceToHost, st));
+  RSC_CUDA(ctx, cudaMemcpyAsync(ce, d_cv + C, (size_t)C * 4, cudaMemcpyDeviceToHost, st));
+  RSC_CUDA(ctx, cudaStreamSynchronize(st));
+  return RSC_OK;
+}
+
 static inline int64_t wrapmul(int64_t a, int64_t b) { return (int64_t)((uint64_t)a * (uint64_t)b); }
 
 void rsc_estimate_score(int64_t subset_len, int64_t cloud_len, int64_t count, double* out_min, double* out_max,

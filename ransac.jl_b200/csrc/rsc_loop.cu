@@ -217,6 +217,118 @@ __global__ void k5_pack_kernel(LoopDev* __restrict__ d, const unsigned long long
   out->tot_global = d->tot_global[0];
 }
 
+// small-batch scorer (rsc_small.cu) limits: beyond them the tiled kernel is the faster one
+// (measured on c4, profiles/r2h_launches_ransac_c4_summary.json: small kernel ~60 us at ~100 candidates x 312 k
+// points and linear in the candidates, tiled path ~190 us flat at this size -> cross-over near 1e8 evaluations)
+constexpr int kSmallMaxCands = 4096;
+constexpr double kSmallMaxEvals = 1.2e8;
+
+// K5's hits (rsc_loop.cuh).  Gathered form: the newly disabled points of the source go into a compact scratch set.
+// Their number is only known on the device, but it cannot exceed the extracted candidate's subset-1 score in the
+// store (every one of them was a compatible, enabled subset point when the candidate was scored; the enabled set
+// only shrinks), which the host has from the decision record: that sizes the launch without a round trip.  If they
+// do not fit, hit[nst + 1] says so and the caller repeats in the masked form.  Masked form (the least-squares refit
+// moves the shape, so the bound does not hold; also the fallback): score against the whole source under the mask
+// old & ~new.  The hits are enabled-gated counts over those points; with `coll` they are summed over the ranks,
+// together with the two flags.
+int32_t k5_hits(rsc_ctx* ctx, rsc_cloud* cloud, const K5In& in, const Thresh& th, K5Out* out, cudaStream_t st) {
+  if (!ctx->loop_scratch) ctx->loop_scratch = new LoopScratch();
+  LoopScratch& ls = *static_cast<LoopScratch*>(ctx->loop_scratch);
+  const int nst = in.nst;
+  const PointSet& src = in.src;
+  const bool exact = src.xyz64 != nullptr;
+  const uint32_t* old_src = in.olden + in.old_word0;
+  int32_t rc = RSC_OK;
+  PointSet dps = src;
+  const float4* tiles = in.view ? in.view_tiles : nullptr;  // the culled scorer's spheres of dps
+  // hit counts [nst] + two flags that ride with them through the all-reduce: guard-band queue overflow,
+  // scratch set too small
+  RSC_CUDA(ctx, ctx->counts.ensure(((size_t)3 * nst + 8) * 4));
+  int32_t* hit = ctx->counts.as<int32_t>() + 2 * (size_t)nst;
+  int32_t* d_over = hit + nst + 1;
+  RSC_CUDA(ctx, cudaMemsetAsync(d_over, 0, 4, st));
+  // scratch: [wcnt: sl_words u32][woff: sl_words + 1 u64][keep: nst u32][koff: nst + 1 u64]
+  const int64_t sl_words = src.n_pad / 32;
+  const size_t o_woff = ((size_t)sl_words * 4 + 255) / 256 * 256;
+  const size_t o_keep = o_woff + ((size_t)(sl_words + 1) * 8 + 255) / 256 * 256;
+  const size_t o_koff = o_keep + ((size_t)nst * 4 + 255) / 256 * 256;
+  RSC_CUDA(ctx, ls.nmeta.ensure(o_koff + (size_t)(nst + 1) * 8));
+  uint32_t* wcnt = ls.nmeta.as<uint32_t>();
+  unsigned long long* woff = (unsigned long long*)(ls.nmeta.as<char>() + o_woff);
+  unsigned long long* wtot = woff + sl_words;
+  out->hit = hit;
+  out->keep = (uint32_t*)(ls.nmeta.as<char>() + o_keep);
+  out->koff = (unsigned long long*)(ls.nmeta.as<char>() + o_koff);
+  out->ktot = out->koff + nst;
+  // the culled scorer (built-in types only) on a view-ordered set when the store is large: most stored candidates
+  // are then nowhere near the extracted shape, and the dense path's candidate compiler is ONE CTA (3 ms for a
+  // store of a million candidates, the cell sampler's)
+  auto culled = [&](int64_t npts) {
+    return in.view && !in.uo && in.cull_mode != 0 && (in.cull_mode == 2 || nst >= 4096 || (double)nst * (double)npts >= 2e8);
+  };
+  if (in.masked) {
+    newly_mask_kernel<<<(unsigned)((in.swords + 255) / 256), 256, 0, st>>>(in.olden, in.new_en, in.swords);
+    RSC_CUDA(ctx, cudaGetLastError());
+    dps.enabled = dps.valid = old_src;  // (only the enabled-gated counts are read)
+  } else if (sl_words > 0) {
+    const int64_t cap = ((int64_t)std::max(in.bound, 1) + kTile - 1) / kTile * kTile;
+    newly_count_kernel<<<(unsigned)((sl_words + 255) / 256), 256, 0, st>>>(old_src, src.enabled, sl_words, wcnt);
+    RSC_CUDA(ctx, cudaGetLastError());
+    if ((rc = scan_u32(ctx, wcnt, (int)sl_words, woff, wtot, st))) return rc;
+    RSC_CUDA(ctx, ls.nscratch.ensure((size_t)6 * cap * 4));
+    RSC_CUDA(ctx, ls.nvalid.ensure((size_t)(cap / 32) * 4));
+    RSC_CUDA(ctx, cudaMemsetAsync(ls.nscratch.p, 0, (size_t)6 * cap * 4, st));
+    if (exact) {  // the scratch set's map into the float64 coordinates, the source's map gathered
+      // (entries past the gathered count stay 0: padding lanes may still look their point up)
+      RSC_CUDA(ctx, ls.nidx.ensure((size_t)cap * sizeof(int64_t)));
+      RSC_CUDA(ctx, cudaMemsetAsync(ls.nidx.p, 0, (size_t)cap * sizeof(int64_t), st));
+    }
+    newly_gather_capped_kernel<<<(unsigned)((sl_words + 255) / 256), 256, 0, st>>>(
+        old_src, src.enabled, sl_words, woff, wtot, src.x, src.y - src.x, ls.nscratch.as<float>(), cap, d_over, src.map,
+        exact ? ls.nidx.as<int64_t>() : nullptr);
+    RSC_CUDA(ctx, cudaGetLastError());
+    fill_valid_dev_kernel<<<(unsigned)((cap / 32 + 255) / 256), 256, 0, st>>>(ls.nvalid.as<uint32_t>(), wtot, cap / 32);
+    RSC_CUDA(ctx, cudaGetLastError());
+    float* b = ls.nscratch.as<float>();
+    dps.x = b, dps.y = b + cap, dps.z = b + 2 * cap, dps.nx = b + 3 * cap, dps.ny = b + 4 * cap, dps.nz = b + 5 * cap;
+    dps.enabled = dps.valid = ls.nvalid.as<uint32_t>();
+    dps.n = dps.n_pad = cap;
+    dps.map = exact ? ls.nidx.as<int64_t>() : nullptr;
+    if (culled(cap)) {  // spheres of the gathered points only: the zero padding stays out of them
+      RSC_CUDA(ctx, ls.ntiles.ensure(cull_sphere_count(cap) * sizeof(float4)));
+      if ((rc = cull_tile_spheres(ctx, dps, ls.ntiles.as<float4>(), st, wtot))) return rc;
+      tiles = ls.ntiles.as<float4>();
+    }
+  }
+  const rsc_cand* cands = in.cands;
+  if (culled(dps.n)) {
+    if ((rc = cull_enqueue(ctx, cloud, dps, tiles, th, cands, nst, nullptr, ctx->counts.as<int32_t>(), hit, nullptr, st))) return rc;
+    RSC_CUDA(ctx, cudaMemsetAsync(hit + nst, 0, 4, st));  // nothing can overflow: pairs beyond the queue are decided inline
+  } else if (in.use_small && nst <= kSmallMaxCands && (double)nst * (double)std::max<int64_t>(dps.n_pad, 1) <= kSmallMaxEvals) {
+    if ((rc = score_small_enqueue(ctx, cloud, dps, th, cands, nst, nullptr, ctx->counts.as<int32_t>(), hit, st))) return rc;
+    RSC_CUDA(ctx, cudaMemsetAsync(hit + nst, 0, 4, st));  // no guard-band queue on this path
+  } else {
+    if ((rc = score_enqueue(ctx, cloud, dps, th, cands, nst, nullptr, false, st, ctx->counts.as<int32_t>(), hit))) return rc;
+    queue_overflow_kernel<<<1, 1, 0, st>>>(ctx->wl_count.as<uint32_t>(), (uint32_t)ctx->wl_cap, hit + nst);
+    RSC_CUDA(ctx, cudaGetLastError());
+  }
+  // user records: the built-in scorers left their hits at 0 (enabled-gated counts, so the scratch bound holds)
+  if (in.uo && (rc = user_score_enqueue(ctx, *in.uo, dps, cands, nst, nullptr, nullptr, hit, st))) return rc;
+  if (in.coll && ctx->allreduce(ctx->allreduce_user, hit, (int64_t)nst + 2, (void*)st))
+    return fail(ctx, RSC_E_NCCL, "ransac_run: all-reduce of the K5 hits failed");
+  return RSC_OK;
+}
+
+int32_t k5_compact(const K5Out& o, int nst, int best, const rsc_cand* c0, const int32_t* s0, uint8_t* f0, rsc_cand* c1,
+                   int32_t* s1, uint8_t* f1, rsc_ctx* ctx, cudaStream_t st) {
+  invalidate_kernel<<<(nst + 255) / 256, 256, 0, st>>>(o.hit, f0, nst, best, o.keep);
+  RSC_CUDA(ctx, cudaGetLastError());
+  if (int32_t rc = scan_u32(ctx, o.keep, nst, o.koff, o.ktot, st)) return rc;
+  compact_store_kernel<<<(nst + 255) / 256, 256, 0, st>>>(c0, s0, f0, o.keep, o.koff, nst, c1, s1, f1);
+  RSC_CUDA(ctx, cudaGetLastError());
+  return RSC_OK;
+}
+
 int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed, rsc_run* run, const FitOrder* order, HostWalk* host) {
   rsc_ctx* ctx = cloud->ctx;
   cudaStream_t st = ctx->stream;
@@ -253,12 +365,8 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
   const FitOrder* uo = order && order->has_user ? order : nullptr;
   const PointSet sps = subset_slice(cloud, sub, ranged);
   const int64_t sps_word0 = sps.enabled - sub.enabled;
-  // small-batch scorer (rsc_small.cu) limits: beyond them the tiled kernel is the faster one
+  // small-batch scorer (rsc_small.cu), within kSmallMaxCands / kSmallMaxEvals
   const bool use_small = getenv("RSC_NO_SMALL") == nullptr;
-  // (measured on c4, profiles/r2h_launches_ransac_c4_summary.json: small kernel ~60 us at ~100 candidates x 312 k
-  // points and linear in the candidates, tiled path ~190 us flat at this size -> cross-over near 1e8 evaluations)
-  constexpr int kSmallMaxCands = 4096;
-  constexpr double kSmallMaxEvals = 1.2e8;
   // K5 on the subset's Morton view: the culled scorer (0: never, 1: for a large store, 2: always; read per run)
   const int k5_cull_mode = getenv("RSC_LOOP_CULL") ? atoi(getenv("RSC_LOOP_CULL")) : 1;
   long long rate_seen = -1;  // recent number of new candidates per iteration (-1: no batch yet)
@@ -469,10 +577,8 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
       // points is the same), else this rank's slice.  Its enabled words of before the extraction are kept.
       const bool view = sub.cen != nullptr && !coll;
       const PointSet src = view ? view_subset_morton(&sub) : sps;
-      const bool exact = src.xyz64 != nullptr;
       const int64_t swords = sub.m_pad / 32;
       RUN_CUDA(ls.olden.ensure((size_t)swords * 4));
-      const uint32_t* old_src = ls.olden.as<uint32_t>() + (view ? 0 : sps_word0);
       RUN_CUDA(cudaMemcpyAsync(ls.olden.p, view ? sub.cen : sub.enabled, (size_t)swords * 4, cudaMemcpyDeviceToDevice, st));
       // ---- K4: refit over this rank's points, invalidate them ----
       rsc_cand shape = rec.best;
@@ -509,118 +615,36 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
         if ((rc = shard_clear_enabled(cloud, ctx->idxbuf.as<uint32_t>(), dev->tot_global, 1, dev->tot_global, st))) return rc;
       }
       // ---- K5: drop the best and every candidate compatible with a newly disabled subset point ----
-      // Gathered form: the newly disabled points of the source go into a compact scratch set.  Their number is
-      // only known on the device, but it cannot exceed the candidate's subset-1 score in the store (every one of
-      // them was a compatible, enabled subset point when the candidate was scored; the enabled set only shrinks),
-      // which the host has from the decision record: that sizes the launch without a round trip.  Masked form (the
-      // least-squares refit moves the shape, so the bound does not hold; also the fallback): score against the
-      // whole source under the mask old & ~new.
+      // (the bitmap filter only removes points from the list, so the gathered form's bound still holds with it)
       const int nst = store.n;
-      // (the bitmap filter only removes points from the list, so the bound still holds with it)
-      bool masked = (p->compat_flags & RSC_REFIT_LSQ) != 0 || getenv("RSC_K5_MASKED") != nullptr;
-      PointSet dps = src;
-      const float4* tiles = view ? static_cast<const float4*>(sub.ctiles) : nullptr;  // the culled scorer's spheres of dps
-      // hit counts [nst] + two flags that ride with them through the all-reduce: guard-band queue overflow,
-      // scratch set too small
-      RUN_CUDA(ctx->counts.ensure(((size_t)3 * nst + 8) * 4));
-      int32_t* hit = ctx->counts.as<int32_t>() + 2 * (size_t)nst;
-      int32_t* d_over = hit + nst + 1;
-      RUN_CUDA(cudaMemsetAsync(d_over, 0, 4, st));
-      // scratch: [wcnt: sl_words u32][woff: sl_words + 1 u64][keep: nst u32][koff: nst + 1 u64]
-      const int64_t sl_words = src.n_pad / 32;
-      const size_t o_woff = ((size_t)sl_words * 4 + 255) / 256 * 256;
-      const size_t o_keep = o_woff + ((size_t)(sl_words + 1) * 8 + 255) / 256 * 256;
-      const size_t o_koff = o_keep + ((size_t)nst * 4 + 255) / 256 * 256;
-      RUN_CUDA(ls.nmeta.ensure(o_koff + (size_t)(nst + 1) * 8));
-      uint32_t* wcnt = ls.nmeta.as<uint32_t>();
-      unsigned long long* woff = (unsigned long long*)(ls.nmeta.as<char>() + o_woff);
-      unsigned long long* wtot = woff + sl_words;
-      uint32_t* keep = (uint32_t*)(ls.nmeta.as<char>() + o_keep);
-      unsigned long long* koff = (unsigned long long*)(ls.nmeta.as<char>() + o_koff);
-      unsigned long long* ktot = koff + nst;
-      // the culled scorer (built-in types only) on a view-ordered set when the store is large: most stored candidates
-      // are then nowhere near the extracted shape, and the dense path's candidate compiler is ONE CTA (3 ms for a
-      // store of a million candidates, the cell sampler's)
-      auto culled = [&](int64_t npts) {
-        return view && !uo && k5_cull_mode != 0 && (k5_cull_mode == 2 || nst >= 4096 || (double)nst * (double)npts >= 2e8);
-      };
-      if (!masked && sl_words > 0) {
-        const int64_t cap = ((int64_t)std::max(rec.best_score, 1) + kTile - 1) / kTile * kTile;
-        newly_count_kernel<<<(unsigned)((sl_words + 255) / 256), 256, 0, st>>>(old_src, src.enabled, sl_words, wcnt);
-        RUN_CUDA(cudaGetLastError());
-        if ((rc = scan_u32(ctx, wcnt, (int)sl_words, woff, wtot, st))) return rc;
-        RUN_CUDA(ls.nscratch.ensure((size_t)6 * cap * 4));
-        RUN_CUDA(ls.nvalid.ensure((size_t)(cap / 32) * 4));
-        RUN_CUDA(cudaMemsetAsync(ls.nscratch.p, 0, (size_t)6 * cap * 4, st));
-        if (exact) {  // the scratch set's map into the float64 coordinates, the source's map gathered
-          // (entries past the gathered count stay 0: padding lanes may still look their point up)
-          RUN_CUDA(ls.nidx.ensure((size_t)cap * sizeof(int64_t)));
-          RUN_CUDA(cudaMemsetAsync(ls.nidx.p, 0, (size_t)cap * sizeof(int64_t), st));
-        }
-        newly_gather_capped_kernel<<<(unsigned)((sl_words + 255) / 256), 256, 0, st>>>(
-            old_src, src.enabled, sl_words, woff, wtot, src.x, src.y - src.x, ls.nscratch.as<float>(), cap, d_over, src.map,
-            exact ? ls.nidx.as<int64_t>() : nullptr);
-        RUN_CUDA(cudaGetLastError());
-        fill_valid_dev_kernel<<<(unsigned)((cap / 32 + 255) / 256), 256, 0, st>>>(ls.nvalid.as<uint32_t>(), wtot, cap / 32);
-        RUN_CUDA(cudaGetLastError());
-        float* b = ls.nscratch.as<float>();
-        dps.x = b, dps.y = b + cap, dps.z = b + 2 * cap, dps.nx = b + 3 * cap, dps.ny = b + 4 * cap, dps.nz = b + 5 * cap;
-        dps.enabled = dps.valid = ls.nvalid.as<uint32_t>();
-        dps.n = dps.n_pad = cap;
-        dps.map = exact ? ls.nidx.as<int64_t>() : nullptr;
-        if (culled(cap)) {  // spheres of the gathered points only: the zero padding stays out of them
-          RUN_CUDA(ls.ntiles.ensure(cull_sphere_count(cap) * sizeof(float4)));
-          if ((rc = cull_tile_spheres(ctx, dps, ls.ntiles.as<float4>(), st, wtot))) return rc;
-          tiles = ls.ntiles.as<float4>();
-        }
-      }
-      auto mask_form = [&]() -> cudaError_t {
-        newly_mask_kernel<<<(unsigned)((swords + 255) / 256), 256, 0, st>>>(ls.olden.as<uint32_t>(), view ? sub.cen : sub.enabled, swords);
-        dps = src;
-        dps.enabled = dps.valid = old_src;  // (only the enabled-gated counts are read)
-        tiles = view ? static_cast<const float4*>(sub.ctiles) : nullptr;
-        masked = true;
-        cudaMemsetAsync(d_over, 0, 4, st);
-        return cudaGetLastError();
-      };
-      if (masked) RUN_CUDA(mask_form());
+      K5In kin;
+      kin.nst = nst;
+      kin.src = src, kin.view = view, kin.view_tiles = static_cast<const float4*>(sub.ctiles);
+      kin.olden = ls.olden.as<uint32_t>(), kin.old_word0 = view ? 0 : sps_word0;
+      kin.new_en = view ? sub.cen : sub.enabled, kin.swords = swords;
+      kin.bound = rec.best_score;
+      kin.masked = (p->compat_flags & RSC_REFIT_LSQ) != 0 || getenv("RSC_K5_MASKED") != nullptr;
+      kin.cull_mode = k5_cull_mode, kin.use_small = use_small, kin.uo = uo, kin.coll = coll;
+      K5Out ko;
       int nxt = store.cur ^ 1;
       for (int attempt = 0;; ++attempt) {
-        // enabled-gated counts over the newly disabled points = hits
-        const rsc_cand* cands = store.cands[store.cur].as<rsc_cand>();
-        if (culled(dps.n)) {
-          if ((rc = cull_enqueue(ctx, cloud, dps, tiles, th, cands, nst, nullptr, ctx->counts.as<int32_t>(), hit, nullptr, st))) return rc;
-          RUN_CUDA(cudaMemsetAsync(hit + nst, 0, 4, st));  // nothing can overflow: pairs beyond the queue are decided inline
-        } else if (use_small && nst <= kSmallMaxCands && (double)nst * (double)std::max<int64_t>(dps.n_pad, 1) <= kSmallMaxEvals) {
-          if ((rc = score_small_enqueue(ctx, cloud, dps, th, cands, nst, nullptr, ctx->counts.as<int32_t>(), hit, st))) return rc;
-          RUN_CUDA(cudaMemsetAsync(hit + nst, 0, 4, st));  // no guard-band queue on this path
-        } else {
-          if ((rc = score_enqueue(ctx, cloud, dps, th, cands, nst, nullptr, false, st, ctx->counts.as<int32_t>(), hit))) return rc;
-          queue_overflow_kernel<<<1, 1, 0, st>>>(ctx->wl_count.as<uint32_t>(), (uint32_t)ctx->wl_cap, hit + nst);
-          RUN_CUDA(cudaGetLastError());
-        }
-        // user records: the built-in scorers left their hits at 0 (enabled-gated counts, so the scratch bound holds)
-        if (uo && (rc = user_score_enqueue(ctx, *uo, dps, cands, nst, nullptr, nullptr, hit, st))) return rc;
-        if (coll && ctx->allreduce(ctx->allreduce_user, hit, (int64_t)nst + 2, (void*)st))
-          return fail(ctx, RSC_E_NCCL, "ransac_run: all-reduce of the K5 hits failed");
-        invalidate_kernel<<<(nst + 255) / 256, 256, 0, st>>>(hit, store.flags[store.cur].as<uint8_t>(), nst, rec.best_idx, keep);
-        RUN_CUDA(cudaGetLastError());
-        if ((rc = scan_u32(ctx, keep, nst, koff, ktot, st))) return rc;
-        compact_store_kernel<<<(nst + 255) / 256, 256, 0, st>>>(
-            store.cands[store.cur].as<rsc_cand>(), store.score[store.cur].as<int32_t>(), store.flags[store.cur].as<uint8_t>(), keep,
-            koff, nst, store.cands[nxt].as<rsc_cand>(), store.score[nxt].as<int32_t>(), store.flags[nxt].as<uint8_t>());
-        RUN_CUDA(cudaGetLastError());
-        k5_pack_kernel<<<1, 1, 0, st>>>(dev, ktot, hit + nst, d_over, ctx->misc2.as<unsigned long long>(), dk5);
+        kin.cands = store.cands[store.cur].as<rsc_cand>();
+        if ((rc = k5_hits(ctx, cloud, kin, th, &ko, st))) return rc;
+        if ((rc = k5_compact(ko, nst, rec.best_idx, store.cands[store.cur].as<rsc_cand>(), store.score[store.cur].as<int32_t>(),
+                             store.flags[store.cur].as<uint8_t>(), store.cands[nxt].as<rsc_cand>(), store.score[nxt].as<int32_t>(),
+                             store.flags[nxt].as<uint8_t>(), ctx, st)))
+          return rc;
+        k5_pack_kernel<<<1, 1, 0, st>>>(dev, ko.ktot, ko.hit + nst, ko.hit + nst + 1, ctx->misc2.as<unsigned long long>(), dk5);
         RUN_CUDA(cudaGetLastError());
         RUN_CUDA(cudaMemcpyAsync(&hio->k5, dk5, sizeof(K5Host), cudaMemcpyDeviceToHost, st));
         if (host && prog) {
           keep_h.resize(nst);
-          RUN_CUDA(cudaMemcpyAsync(keep_h.data(), keep, (size_t)nst * 4, cudaMemcpyDeviceToHost, st));
+          RUN_CUDA(cudaMemcpyAsync(keep_h.data(), ko.keep, (size_t)nst * 4, cudaMemcpyDeviceToHost, st));
         }
         RUN_CUDA(sync());
         if (!hio->k5.ovf) break;
         if (hio->k5.ovf & 2) {  // (not expected) more newly disabled points than the bound: masked form
-          RUN_CUDA(mask_form());
+          kin.masked = true;
           continue;
         }
         // invalidate_kernel marked flags of this attempt: they only ever go from alive to dead on hits that
@@ -664,3 +688,83 @@ int32_t ransac_loop_device(rsc_cloud* cloud, const rsc_params* p, uint64_t seed,
 }
 
 }  // namespace rsc
+
+// Test hook: K5 on its own (include/rsc.h rsc_debug_k5_hits), through k5_hits and k5_compact as the loop calls them.
+extern "C" int32_t rsc_debug_k5_hits(rsc_cloud* cloud, const rsc_params* params, const rsc_cand* cands, int32_t nst,
+                                     const uint64_t* new_enabled, int32_t bound, int32_t form, int32_t best, int32_t* hit,
+                                     int32_t* flags, int32_t* survivors, int32_t* n_survivors) {
+  using namespace rsc;
+  if (!cloud) return RSC_E_ARG;
+  rsc_ctx* ctx = cloud->ctx;
+  if (nst <= 0 || !cands || !new_enabled || !hit || best < -1 || best >= nst || (form & ~3))
+    return fail(ctx, RSC_E_ARG, "debug_k5_hits: bad arguments (nst >= 1, -1 <= best < nst, form in 0..3)");
+  if (!params) return fail(ctx, RSC_E_ARG, "params is null");
+  RSC_CUDA(ctx, cudaSetDevice(ctx->device));
+  int32_t rc = cloud_ready(cloud);
+  if (rc) return rc;
+  if (cloud->is_shard() || cloud->subsets.empty() || !cloud->subsets[0].soa)
+    return fail(ctx, RSC_E_STATE, "debug_k5_hits: needs subset 0 uploaded (rsc_cloud_set_subset) on an unsharded cloud");
+  cudaStream_t st = ctx->stream;
+  rsc_subset& sub = cloud->subsets[0];
+  const bool view = (form & 2) != 0;
+  if (view && (rc = subset_cull_view(cloud, sub, st))) return rc;
+  if (!ctx->loop_scratch) ctx->loop_scratch = new LoopScratch();
+  LoopScratch& ls = *static_cast<LoopScratch*>(ctx->loop_scratch);
+  const int64_t swords = sub.m_pad / 32;
+  // the store: candidates, scores = their indices (so the compaction reports who survived), all alive
+  RSC_CUDA(ctx, ls.store.reserve((size_t)nst, st));
+  rsc_cand* c0 = ls.store.cands[0].as<rsc_cand>();
+  int32_t* s0 = ls.store.score[0].as<int32_t>();
+  std::vector<int32_t> iota(nst);
+  for (int i = 0; i < nst; ++i) iota[i] = i;
+  RSC_CUDA(ctx, cudaMemcpyAsync(c0, cands, (size_t)nst * sizeof(rsc_cand), cudaMemcpyHostToDevice, st));
+  RSC_CUDA(ctx, cudaMemcpyAsync(s0, iota.data(), (size_t)nst * 4, cudaMemcpyHostToDevice, st));
+  RSC_CUDA(ctx, cudaMemsetAsync(ls.store.flags[0].p, 1, (size_t)nst, st));
+  // the enabled words of before, then the cloud's mask becomes new_enabled (the subset and its view follow)
+  RSC_CUDA(ctx, ls.olden.ensure((size_t)swords * 4));
+  RSC_CUDA(ctx, cudaMemcpyAsync(ls.olden.p, view ? sub.cen : sub.enabled, (size_t)swords * 4, cudaMemcpyDeviceToDevice, st));
+  if ((rc = rsc_cloud_set_enabled(cloud, new_enabled))) return rc;
+  K5In in;
+  in.cands = c0, in.nst = nst;
+  in.src = view ? view_subset_morton(&sub) : subset_slice(cloud, sub, false);
+  in.view = view, in.view_tiles = static_cast<const float4*>(sub.ctiles);
+  in.olden = ls.olden.as<uint32_t>(), in.old_word0 = 0;
+  in.new_en = view ? sub.cen : sub.enabled, in.swords = swords;
+  in.bound = bound;
+  in.masked = (form & 1) != 0;
+  in.cull_mode = getenv("RSC_LOOP_CULL") ? atoi(getenv("RSC_LOOP_CULL")) : 1;
+  in.use_small = getenv("RSC_NO_SMALL") == nullptr;
+  in.uo = nullptr, in.coll = false;
+  const Thresh th = make_thresh(params);
+  K5Out ko;
+  int32_t fl[2] = {0, 0};
+  for (int attempt = 0;; ++attempt) {  // the loop's repeats: the masked form when the scratch set is too small
+    if ((rc = k5_hits(ctx, cloud, in, th, &ko, st))) return rc;
+    int32_t f[2];
+    RSC_CUDA(ctx, cudaMemcpyAsync(f, ko.hit + nst, 8, cudaMemcpyDeviceToHost, st));
+    RSC_CUDA(ctx, cudaStreamSynchronize(st));
+    if (attempt == 0) fl[0] = f[0], fl[1] = f[1];
+    if (f[1] && !in.masked) {
+      in.masked = true;
+      continue;
+    }
+    if (f[0]) {
+      if (attempt >= 4) return fail(ctx, RSC_E_STATE, "debug_k5_hits: guard-band queue kept overflowing");
+      if ((rc = grow_guard_queue(ctx))) return rc;
+      continue;
+    }
+    break;
+  }
+  if ((rc = k5_compact(ko, nst, best, c0, s0, ls.store.flags[0].as<uint8_t>(), ls.store.cands[1].as<rsc_cand>(),
+                       ls.store.score[1].as<int32_t>(), ls.store.flags[1].as<uint8_t>(), ctx, st)))
+    return rc;
+  unsigned long long kept = 0;
+  RSC_CUDA(ctx, cudaMemcpyAsync(hit, ko.hit, (size_t)nst * 4, cudaMemcpyDeviceToHost, st));
+  RSC_CUDA(ctx, cudaMemcpyAsync(&kept, ko.ktot, 8, cudaMemcpyDeviceToHost, st));
+  RSC_CUDA(ctx, cudaStreamSynchronize(st));
+  if (survivors && kept)
+    RSC_CUDA(ctx, cudaMemcpy(survivors, ls.store.score[1].p, (size_t)kept * 4, cudaMemcpyDeviceToHost));
+  if (n_survivors) *n_survivors = (int32_t)kept;
+  if (flags) flags[0] = fl[0], flags[1] = fl[1];
+  return RSC_OK;
+}

@@ -212,6 +212,37 @@ inline PointSet subset_slice(const rsc_cloud* cloud, const rsc_subset& sb, bool 
   return v;
 }
 
+// K5, the re-scoring of the store after an extraction: for each stored candidate, its compatible points among the
+// subset points the extraction just disabled (old & ~new words of the source).
+struct K5In {
+  const rsc_cand* cands;     // the store [nst]
+  int nst;
+  PointSet src;              // the source of the newly disabled points: the subset's Morton view or the rank's slice
+  bool view;                 // src is the Morton view (sub.ctiles are its spheres)
+  const float4* view_tiles;  // sub.ctiles
+  uint32_t* olden;           // the source's whole-subset enabled words before the extraction (the masked form clears
+                             // the still-enabled ones in place: old &= ~new)
+  int64_t old_word0;         // the first word of src within olden
+  const uint32_t* new_en;    // the whole-subset enabled words after the extraction (sub.cen for the view)
+  int64_t swords;            // words of olden / new_en
+  int bound;                 // scratch bound of the gathered form: the extracted candidate's subset-1 score
+  bool masked;               // masked form: score the whole source under old & ~new instead of gathering
+  int cull_mode;             // RSC_LOOP_CULL: 0 never, 1 for a large store, 2 always (view only)
+  bool use_small;            // the small-batch scorer may be taken
+  const FitOrder* uo;        // user shapes (nullable)
+  bool coll;                 // hits summed over the ranks
+};
+struct K5Out {
+  int32_t* hit;              // [nst] hits, then [nst] guard-band queue overflow, [nst + 1] scratch set too small
+  uint32_t* keep;            // [nst] scratch for k5_compact
+  unsigned long long *koff, *ktot;
+};
+int32_t k5_hits(rsc_ctx* ctx, rsc_cloud* cloud, const K5In& in, const Thresh& th, K5Out* out, cudaStream_t st);
+// removeinvalidshapes!: drop the best, every candidate with a hit and the tainted spheres, order-preserving
+// compaction of (cands, score, flags)[0 .. nst) into the *1 arrays; *ktot = survivors
+int32_t k5_compact(const K5Out& o, int nst, int best, const rsc_cand* c0, const int32_t* s0, uint8_t* f0, rsc_cand* c1,
+                       int32_t* s1, uint8_t* f1, rsc_ctx* ctx, cudaStream_t st);
+
 // The host decision of a batch (rsc_run.cu), taken instead of decide_kernel's when RSC_SCORE_PROGRESSIVE,
 // RSC_SAMPLER_OCTREE or RSC_LOOP_HOSTWALK is set.  `d` is the host copy of the device state after K2 + K3,
 // `newscore` the new candidates' subset-1 scores (progressive scoring).  Fills *rec like decide_kernel does.

@@ -6,7 +6,11 @@ the library's own NCCL path is exercised by bench.py / tools/ransac_multi.py on 
     the replicated enabled mask, coordinates are gathered from their owners, inlier lists stay
     distributed -- the joined result equals the C oracle's loop (and so the single-GPU loop);
   * replicated storage with a cloud smaller than 2048 x ranks: one rank's range is empty and it still
-    joins every all-reduce (ADVICE round 1)."""
+    joins every all-reduce (ADVICE round 1);
+  * replicated storage with each extension switch of the loop (progressive scoring, the cell sampler, the
+    least-squares refit, the bitmap filter, the host-walked decision, RSC_LOOP_CULL=2, K5's masked form): every
+    rank scores its slice of the newly disabled points after an extraction and the hits are all-reduced, and the
+    result equals the single-process run of the same configuration."""
 import os
 import sys
 
@@ -31,7 +35,36 @@ def _scene(which):
             {"tau": 400, "minsubsetN": 128, "itermax": 120}, 99)
 
 
-def _worker(rank, world, port, which, layout, q):
+# replicated runs with an extension switch: (environment, ransac() keywords)
+SWITCHES = {
+    "progressive": ({}, {"progressive": True}),
+    "octree_lw1": ({}, {"sampler": "octree", "lw_period": 1}),
+    "octree_lw16": ({}, {"sampler": "octree", "lw_period": 16}),
+    "lsq": ({}, {"lsq": True}),
+    "bitmap": ({}, {"bitmap": (1.5, False)}),
+    "hostwalk": ({"RSC_LOOP_HOSTWALK": "1"}, {}),
+    # (a ranged run never takes the culled scorer, which needs the whole subset's Morton view: this case compares the
+    # dense ranged run with the culled single-process run)
+    "loop_cull2": ({"RSC_LOOP_CULL": "2"}, {}),
+    "k5_masked": ({"RSC_K5_MASKED": "1"}, {}),
+}
+
+
+def _run_switch(R, pc, params, seed, switch):
+    """ransac() under one entry of SWITCHES (its environment is set by the caller); -> (extracted, info)"""
+    _, kw = SWITCHES[switch] if switch else ({}, {})
+    if kw.get("sampler") == "octree":
+        pc.build_cells(8)
+    ex, _ = R.ransac(pc, params, True, seed=seed, **kw)
+    lw = getattr(pc, "levelweight", None)
+    info = {"iterations": pc.last_run_iterations, "refined": pc.last_refined,
+            "levelweight": None if lw is None or not kw.get("sampler") else np.asarray(lw).copy()}
+    return ex, info
+
+
+def _worker(rank, world, port, which, layout, q, switch=None):
+    for k, v in (SWITCHES[switch][0] if switch else {}).items():
+        os.environ[k] = v
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["MASTER_PORT"] = str(port)
     sys.path.insert(0, ROOT)
@@ -53,33 +86,30 @@ def _worker(rank, world, port, which, layout, q):
         local_en = pc.isenabled
         totals = [e.total for e in ex]
         ex = shard.gather_extracted(ex)
+        info = None
         parts = [None] * world
         dist.all_gather_object(parts, local_en)
         enabled = np.concatenate(parts)
     else:
         pc = R.RANSACCloud(sc.vertices, sc.normals, subsets)
         sh = shard.ShardedContext(pc, comm="host")
-        ex, _ = R.ransac(pc, params, True, seed=seed)
+        ex, info = _run_switch(R, pc, params, seed, switch)
         enabled = pc.isenabled
         totals = [e.total for e in ex]
         sh.close()
     if rank == 0:
         q.put(([(e.shape.to_cand().type, bool(e.shape.to_cand().outwards), list(e.shape.to_cand().p), e.inpoints) for e in ex],
-               enabled, totals, pc.last_run_syncs, pc.last_run_batches))
+               enabled, totals, pc.last_run_syncs, pc.last_run_batches, info))
     dist.barrier()
     dist.destroy_process_group()
 
 
-@pytest.mark.parametrize("which,layout", [("c1", "shard"), ("noisy", "shard"), ("tiny", "replicated"), ("noisy", "replicated")])
-def test_two_ranks_one_gpu_match_c_oracle(which, layout):
-    from oracle import c_oracle
-    import ransac_jl_b200 as R
-    from tests.helpers import oracle_params
-
+def _two_ranks(which, layout, switch=None):
+    """runs _worker on two ranks sharing cuda:0; -> rank 0's result"""
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     port = 29600 + os.getpid() % 2000
-    procs = [ctx.Process(target=_worker, args=(rk, 2, port, which, layout, q)) for rk in range(2)]
+    procs = [ctx.Process(target=_worker, args=(rk, 2, port, which, layout, q, switch)) for rk in range(2)]
     for p in procs:
         p.start()
     import queue as _queue
@@ -96,7 +126,14 @@ def test_two_ranks_one_gpu_match_c_oracle(which, layout):
         p.join(120)
         assert p.exitcode == 0
     assert res is not None
-    got, enabled, totals, syncs, batches = res
+    return res
+
+
+def _equal_c_oracle(which, got, enabled, totals):
+    from oracle import c_oracle
+    import ransac_jl_b200 as R
+    from tests.helpers import oracle_params
+
     sc, r, itp, seed = _scene(which)
     subsets = R.makesubsets(len(sc.vertices), r, np.random.default_rng(1234))
     want, en, info = c_oracle.ransac(sc.vertices, sc.normals, subsets[0], oracle_params(R.ransacparameters(iteration=itp)), seed)
@@ -107,8 +144,57 @@ def test_two_ranks_one_gpu_match_c_oracle(which, layout):
         np.testing.assert_array_equal(g[3], w[3])
         assert tot == len(w[3])
     np.testing.assert_array_equal(enabled, en)
+    return want
+
+
+@pytest.mark.parametrize("which,layout", [("c1", "shard"), ("noisy", "shard"), ("tiny", "replicated"), ("noisy", "replicated")])
+def test_two_ranks_one_gpu_match_c_oracle(which, layout):
+    res = _two_ranks(which, layout)
+    got, enabled, totals, syncs, batches, _ = res
+    want = _equal_c_oracle(which, got, enabled, totals)
     # 2 synchronisations per batch + 1 per extraction (+ set-up)
     assert syncs <= 2 * batches + len(want) + 8
+
+
+@pytest.mark.parametrize("which,switch", [("noisy", s) for s in SWITCHES] +
+                         [("tiny", "progressive"), ("tiny", "octree_lw16"), ("tiny", "hostwalk"), ("tiny", "k5_masked")])
+def test_two_ranks_replicated_with_extension_switches(which, switch, monkeypatch):
+    """replicated storage, two ranks with a point range each: every rank scores its slice of the newly disabled
+    subset points after an extraction and the hits are all-reduced.  Shapes (bit for bit), inlier lists, final
+    enabled mask, iterations, progressive refinements and level weights equal the single-process run of the same
+    configuration; the switches that leave the reference's loop as it is also equal the C oracle's loop.  On the
+    tiny scene (1500 points, ranges aligned to 2048) rank 1 owns no point, so its slice of subset 1 is empty."""
+    import ransac_jl_b200 as R
+
+    got, enabled, totals, _, _, info = _two_ranks(which, "replicated", switch)
+    for k, v in SWITCHES[switch][0].items():
+        monkeypatch.setenv(k, v)
+    sc, r, itp, seed = _scene(which)
+    subsets = R.makesubsets(len(sc.vertices), r, np.random.default_rng(1234))
+    pc = R.RANSACCloud(sc.vertices, sc.normals, subsets)
+    want, winfo = _run_switch(R, pc, R.ransacparameters(iteration=itp), seed, switch)
+    assert len(got) == len(want) and len(want) >= 2
+    for g, w, tot in zip(got, want, totals):
+        c = w.shape.to_cand()
+        assert (g[0], g[1]) == (c.type, bool(c.outwards))
+        assert g[2] == list(c.p)  # bit for bit
+        np.testing.assert_array_equal(g[3], w.inpoints)
+        assert tot == len(w.inpoints)
+    np.testing.assert_array_equal(enabled, pc.isenabled)
+    assert info["iterations"] == winfo["iterations"] and info["refined"] == winfo["refined"]
+    if switch == "progressive":
+        assert winfo["refined"] > 0
+    if winfo["levelweight"] is not None:
+        np.testing.assert_array_equal(info["levelweight"], winfo["levelweight"])
+    else:
+        assert info["levelweight"] is None
+    pc.close()
+    # environment-only switches run the reference's loop: the C oracle's too.  The keyword switches (progressive
+    # scoring, the cell sampler, the least-squares refit, the bitmap filter) change the loop itself; the single-process
+    # run they are compared with here is pinned to the NumPy oracle's loop of the same switch by test_progressive.py,
+    # test_octree_gpu.py, test_lsq.py and test_bitmap_gpu.py.
+    if not SWITCHES[switch][1]:
+        _equal_c_oracle(which, got, enabled, totals)
 
 
 def test_library_nccl_communicator_single_rank():
