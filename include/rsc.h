@@ -481,6 +481,36 @@ int32_t rsc_estimate_normals(rsc_ctx* ctx, const float* xyz, int64_t n, int32_t 
 int32_t rsc_orient_normals(rsc_ctx* ctx, const float* xyz, int64_t n, int32_t k, const float* nrm_in, float* nrm_out,
                            int64_t* edges, int64_t* stats);
 
+/* ---- the same two on a cloud sharded by point range over the ranks of the context's communicator ----------------
+ * Collective: every rank calls with its own rows [global_offset, global_offset + n) of a cloud of n_global points
+ * (1 <= n_global < 2^31), the layout rsc_cloud_create_shard takes.  xyz, nrm, nbr, nrm_in and nrm_out hold this rank's
+ * rows; nbr holds global indices.  The ranges must tile [0, n_global) (any order of ranks, no alignment); a rank may be
+ * empty (n = 0, its row pointers may be NULL).  The concatenation of the ranks' outputs in range order is bit for bit
+ * the single call's on the whole cloud: normals and lists, and the sum of the ranks' `pairs` (each rank counts its own
+ * distances).  edges (capacity 2 n_global values) and stats describe the whole forest and are identical on every rank.
+ * Protocol (DESIGN.md section 8):
+ *   1. argument check, two all-reduces (104 B and 4 B): k, n_global, the viewpoint and whether it is given must agree,
+ *      the n must sum to n_global, nbr / nrm_in must be given on all non-empty ranks or on none, and every rank must
+ *      allocate the device buffers of the later steps (between the two all-reduces).  Otherwise every rank returns
+ *      RSC_E_ARG; without a communicator, RSC_E_STATE at once.  After the check a rank leaves early only on a CUDA
+ *      error (a device fault, a failed launch), which can leave the other ranks blocked in the next all-reduce, as in
+ *      every collective of the library;
+ *   2. gather: every rank's rows into a zero-filled n_global record buffer (coordinates + a coverage word: 16 B per
+ *      point; 28 B with nrm_in, whose normals travel along), one all-reduce; overlapping or missing rows: RSC_E_ARG on
+ *      every rank;
+ *   3. every rank sorts the whole cloud as rsc_estimate_normals does and searches one contiguous run of the sorted
+ *      queries; the non-empty ranks share the finite points equally;
+ *   4. the rows (normals 12 B, int64 lists 8 k B / int32 lists 4 k B per point) return to their owners through one
+ *      zero-filled n_global buffer and one all-reduce; orientation then builds the forest on every rank.
+ * All-reduces per call: 4.  Volume: estimation 104 + 4 + (16 + 12) n_global B, plus 8 k n_global with nbr;
+ * orientation 104 + 4 + (28 + 4 k) n_global B.  Device memory per rank: the single call's on n_global points, plus
+ * the record and row buffers (16 + 12 B per point, + 8 k / 4 k).  The search divides over the ranks; the gather, the
+ * sort, the exchanges and orientation's forest are replicated. */
+int32_t rsc_estimate_normals_shard(rsc_ctx* ctx, const float* xyz, int64_t n, int64_t global_offset, int64_t n_global,
+                                   int32_t k, const double* viewpoint, float* nrm, int64_t* nbr, int64_t* pairs);
+int32_t rsc_orient_normals_shard(rsc_ctx* ctx, const float* xyz, int64_t n, int64_t global_offset, int64_t n_global,
+                                 int32_t k, const float* nrm_in, float* nrm_out, int64_t* edges, int64_t* stats);
+
 #ifdef __cplusplus
 }
 #endif

@@ -338,6 +338,56 @@ function orient_normals(vertices::Vector{SVector{3,Float32}}; normals=nothing, k
     nrm
 end
 
+# ---- the same on a cloud sharded by point range (rsc_estimate_normals_shard, rsc_orient_normals_shard) ----------
+"""
+    estimate_normals(vertices, shard::Tuple{Integer,Integer}; k=16, viewpoint=nothing) -> Vector{SVector{3,Float32}}
+    orient_normals(vertices, shard::Tuple{Integer,Integer}; normals=nothing, k=16) -> Vector{SVector{3,Float32}}
+
+Collective over the ranks of the context's communicator (`comm_init`): `shard = (global_offset, n_global)`,
+`vertices` (and `normals`) are this rank's rows of a cloud of `n_global` points, the ranks' ranges tile it (a rank
+may be empty), and the result is this rank's rows of the single call's result on the whole cloud, bit for bit.  The
+rows feed `rsc_cloud_create_shard`.  The shard is a positional argument (Python spells it `shard=(lo, n)`): Julia
+does not dispatch on keywords, and a `shard` keyword would change the signature of the one-GPU methods above.
+"""
+function estimate_normals(vertices::Vector{SVector{3,Float32}}, shard::Tuple{Integer,Integer}; k::Integer=16,
+                          viewpoint=nothing)
+    off, n_global = shard_range(shard, length(vertices))
+    nrm = Vector{SVector{3,Float32}}(undef, length(vertices))
+    vp = viewpoint === nothing ? nothing : Float64[viewpoint[1], viewpoint[2], viewpoint[3]]
+    GC.@preserve vertices nrm vp begin
+        check(ccall(fn(:rsc_estimate_normals_shard), Int32,
+                    (Ptr{Cvoid}, Ptr{Float32}, Int64, Int64, Int64, Int32, Ptr{Float64}, Ptr{Float32}, Ptr{Int64}, Ptr{Int64}),
+                    context(), Ptr{Float32}(pointer(vertices)), length(vertices), off, n_global, k,
+                    vp === nothing ? Ptr{Float64}(C_NULL) : pointer(vp), Ptr{Float32}(pointer(nrm)),
+                    Ptr{Int64}(C_NULL), Ptr{Int64}(C_NULL)))
+    end
+    nrm
+end
+
+function orient_normals(vertices::Vector{SVector{3,Float32}}, shard::Tuple{Integer,Integer}; normals=nothing,
+                        k::Integer=16)
+    off, n_global = shard_range(shard, length(vertices))
+    nrm = Vector{SVector{3,Float32}}(undef, length(vertices))
+    nin = normals === nothing ? nothing : convert(Vector{SVector{3,Float32}}, normals)
+    nin === nothing || length(nin) == length(vertices) || throw(ArgumentError("normals must match vertices"))
+    GC.@preserve vertices nrm nin begin
+        check(ccall(fn(:rsc_orient_normals_shard), Int32,
+                    (Ptr{Cvoid}, Ptr{Float32}, Int64, Int64, Int64, Int32, Ptr{Float32}, Ptr{Float32}, Ptr{Int64}, Ptr{Int64}),
+                    context(), Ptr{Float32}(pointer(vertices)), length(vertices), off, n_global, k,
+                    nin === nothing ? Ptr{Float32}(C_NULL) : Ptr{Float32}(pointer(nin)), Ptr{Float32}(pointer(nrm)),
+                    Ptr{Int64}(C_NULL), Ptr{Int64}(C_NULL)))
+    end
+    nrm
+end
+
+# (global_offset, n_global) of a shard, checked against this rank's n rows before any device work
+function shard_range(shard, n::Integer)
+    off, n_global = Int64(shard[1]), Int64(shard[2])
+    1 <= n_global < 2^31 && 0 <= off && off + n <= n_global ||
+        throw(ArgumentError("shard = ($off, $n_global) does not hold this rank's $n rows inside [0, n_global)"))
+    off, n_global
+end
+
 # ---- user-defined shapes on the device (include/rsc.h "user-defined shapes") -----------------------------
 """
     compile_user_shape(src::String) -> type id

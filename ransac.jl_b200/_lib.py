@@ -150,6 +150,9 @@ SIGNATURES = {
     "rsc_ransac_run_user": (C.c_int32, [_P, C.POINTER(rsc_params), _P, C.c_int32, C.c_uint64, C.POINTER(_P)]),
     "rsc_estimate_normals": (C.c_int32, [_P, _P, C.c_int64, C.c_int32, _P, _P, _P, C.POINTER(C.c_int64)]),
     "rsc_orient_normals": (C.c_int32, [_P, _P, C.c_int64, C.c_int32, _P, _P, _P, _P]),
+    "rsc_estimate_normals_shard": (C.c_int32, [_P, _P, C.c_int64, C.c_int64, C.c_int64, C.c_int32, _P, _P, _P,
+                                               C.POINTER(C.c_int64)]),
+    "rsc_orient_normals_shard": (C.c_int32, [_P, _P, C.c_int64, C.c_int64, C.c_int64, C.c_int32, _P, _P, _P, _P]),
 }
 
 if not os.path.exists(LIB_PATH):

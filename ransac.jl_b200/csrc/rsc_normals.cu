@@ -13,11 +13,18 @@
 //     than the k-th.  Otherwise it rescans one level up; level 2 and level 1 cover the whole box.
 // Then, in the same warp: the float64 covariance of N(i) in list order, cyclic Jacobi, the sign rule, and the stores
 // by original index.  rsc_orient_normals (rsc_orient.cu) runs the same search through knn_prepare / knn_run
-// (rsc_normals.cuh) and keeps the lists on the device as int32.
+// (rsc_normals.cuh) and keeps the lists on the device as int32.  The sharded forms (rsc_*_normals_shard) gather the
+// cloud on every rank, sort it identically there and give each rank a contiguous run of the sorted queries.
 #include <cub/device/device_radix_sort.cuh>
 
+#include <chrono>
 #include <climits>
 #include <cmath>
+#include <cstdio>
+#include <cstdlib>
+#include <cstring>
+#include <functional>
+#include <string>
 
 #include "rsc_normals.cuh"
 
@@ -133,6 +140,7 @@ struct NormalsArgs {
   const uint32_t* perm;  // [n] sorted position -> point index
   const float* sx;       // [3 n] sorted SoA coordinates
   int32_t n, nf, k, keff;
+  int32_t p0, p1;        // the queries: sorted positions [p0, p1)
   Quant q;
   double vp[3];
   int has_vp;
@@ -153,7 +161,7 @@ __global__ void __launch_bounds__(256, 2) knn_normals_kernel(const NormalsArgs A
   const int k = A.k, keff = A.keff;
   long long pairs = 0;
   // positions and candidate counters are 64-bit: p + nwarps and base + 32 may pass 2^31 - 1 for n close to it
-  for (int64_t p = (int64_t)blockIdx.x * kWarpsPerBlock + (threadIdx.x >> 5); p < A.n; p += nwarps) {
+  for (int64_t p = A.p0 + (int64_t)blockIdx.x * kWarpsPerBlock + (threadIdx.x >> 5); p < A.p1; p += nwarps) {
     const uint32_t i = __ldg(A.perm + p);
     if (p >= A.nf) {  // non-finite point: zero normal, empty row
       if (kPca && lane < 3) A.nrm[3 * (int64_t)i + lane] = 0.f;
@@ -343,37 +351,92 @@ __global__ void __launch_bounds__(256, 2) knn_normals_kernel(const NormalsArgs A
   if (lane == 0 && A.pairs && pairs) atomicAdd(A.pairs, (unsigned long long)pairs);
 }
 
+// sharded forms: this rank's rows into the zero-filled all-reduce records of W int32 words by point index -- the
+// coordinate bits, the normal bits when given, and a coverage word: 3 on the range's first row, 1 on the others
+__global__ void __launch_bounds__(256) shard_pack_kernel(const float* __restrict__ xyz, const float* __restrict__ nrm, int64_t n,
+                                                         int64_t off, int W, int32_t* __restrict__ rec) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  int32_t* r = rec + (off + i) * W;
+#pragma unroll
+  for (int a = 0; a < 3; ++a) {
+    r[a] = __float_as_int(xyz[3 * i + a]);
+    if (nrm) r[3 + a] = __float_as_int(nrm[3 * i + a]);
+  }
+  r[W - 1] = i == 0 ? 3 : 1;
+}
+
+// the summed records back to AoS; cnt[0] rows covered by no range or by several, cnt[1] ranges starting before off,
+// cnt[2] ranges (non-empty ones)
+__global__ void __launch_bounds__(256) shard_unpack_kernel(const int32_t* __restrict__ rec, int64_t n, int64_t off, int W,
+                                                           float* __restrict__ aos, float* __restrict__ nrm,
+                                                           unsigned long long* __restrict__ cnt) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  bool bad = false, start = false;
+  if (i < n) {
+    const int32_t* r = rec + i * W;
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+      aos[3 * i + a] = __int_as_float(r[a]);
+      if (nrm) nrm[3 * i + a] = __int_as_float(r[3 + a]);
+    }
+    const int32_t c = r[W - 1];
+    bad = c != 1 && c != 3;
+    start = c == 3;
+  }
+  const int nb = __syncthreads_count(bad), ns = __syncthreads_count(start), nbefore = __syncthreads_count(start && i < off);
+  if (threadIdx.x == 0) {
+    if (nb) atomicAdd(cnt, (unsigned long long)nb);
+    if (nbefore) atomicAdd(cnt + 1, (unsigned long long)nbefore);
+    if (ns) atomicAdd(cnt + 2, (unsigned long long)ns);
+  }
+}
+
 }  // namespace
 }  // namespace rsc
 
 using namespace rsc;
 
+#define NRM_CUDA(expr) RSC_CUDA(ctx, (expr))
+
 int32_t rsc::knn_prepare(rsc_ctx* ctx, const float* xyz, int64_t n, KnnSearch& S) {
   RSC_CUDA(ctx, cudaSetDevice(ctx->device));
-  cudaStream_t st = ctx->stream;
+  if (int32_t rc = knn_reserve(ctx, n, S)) return rc;
+  NRM_CUDA(cudaMemcpyAsync(S.aos, xyz, (size_t)n * 12, cudaMemcpyHostToDevice, ctx->stream));
+  return knn_sort(ctx, S);
+}
+
+int32_t rsc::knn_reserve(rsc_ctx* ctx, int64_t n, KnnSearch& S) {
   Allocs& al = S.al;
-  uint64_t* d_keys[2] = {nullptr, nullptr};
-  uint32_t* d_idx[2] = {nullptr, nullptr};
-  uint32_t* d_mm = nullptr;
-  void* d_tmp = nullptr;
-#define NRM_CUDA(expr) RSC_CUDA(ctx, (expr))
   S.n = n;
   NRM_CUDA(al.get((void**)&S.aos, (size_t)n * 12));
   NRM_CUDA(al.get((void**)&S.soa, (size_t)n * 12));
   for (int b = 0; b < 2; ++b) {
-    NRM_CUDA(al.get((void**)&d_keys[b], (size_t)n * 8));
-    NRM_CUDA(al.get((void**)&d_idx[b], (size_t)n * 4));
+    NRM_CUDA(al.get((void**)&S.keys_buf[b], (size_t)n * 8));
+    NRM_CUDA(al.get((void**)&S.idx_buf[b], (size_t)n * 4));
   }
-  NRM_CUDA(al.get((void**)&d_mm, 6 * 4 + 2 * 8));
-  S.cnt = reinterpret_cast<unsigned long long*>(d_mm + 6);
+  NRM_CUDA(al.get((void**)&S.mm, 6 * 4 + 2 * 8));
+  S.cnt = reinterpret_cast<unsigned long long*>(S.mm + 6);
+  cub::DoubleBuffer<uint64_t> kbuf(S.keys_buf[0], S.keys_buf[1]);
+  cub::DoubleBuffer<uint32_t> ibuf(S.idx_buf[0], S.idx_buf[1]);
+  S.tmp_bytes = 0;
+  NRM_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, S.tmp_bytes, kbuf, ibuf, (int)n, 0, 64, ctx->stream));
+  NRM_CUDA(al.get(&S.tmp, S.tmp_bytes));
+  return RSC_OK;
+}
+
+int32_t rsc::knn_sort(rsc_ctx* ctx, KnnSearch& S) {
+  cudaStream_t st = ctx->stream;
+  const int64_t n = S.n;
+  uint64_t* const* d_keys = S.keys_buf;
+  uint32_t* const* d_idx = S.idx_buf;
+  uint32_t* d_mm = S.mm;
   cub::DoubleBuffer<uint64_t> kbuf(d_keys[0], d_keys[1]);
   cub::DoubleBuffer<uint32_t> ibuf(d_idx[0], d_idx[1]);
-  size_t tmp_bytes = 0;
-  NRM_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, kbuf, ibuf, (int)n, 0, 64, st));
-  NRM_CUDA(al.get(&d_tmp, tmp_bytes));
+  size_t tmp_bytes = S.tmp_bytes;
+  void* d_tmp = S.tmp;
 
   const unsigned blocks = (unsigned)((n + 255) / 256);
-  NRM_CUDA(cudaMemcpyAsync(S.aos, xyz, (size_t)n * 12, cudaMemcpyHostToDevice, st));
   const uint32_t init[6] = {0xffffffffu, 0xffffffffu, 0xffffffffu, 0u, 0u, 0u};
   NRM_CUDA(cudaMemcpyAsync(d_mm, init, sizeof(init), cudaMemcpyHostToDevice, st));
   NRM_CUDA(cudaMemsetAsync(S.cnt, 0, 2 * 8, st));
@@ -410,17 +473,19 @@ int32_t rsc::knn_prepare(rsc_ctx* ctx, const float* xyz, int64_t n, KnnSearch& S
 }
 
 int32_t rsc::knn_run(rsc_ctx* ctx, const KnnSearch& S, int32_t k, const double* viewpoint, float* d_nrm, int64_t* d_nbr,
-                     int32_t* d_lists) {
+                     int32_t* d_lists, int64_t p_begin, int64_t p_end) {
+  if (p_end <= p_begin) return RSC_OK;
   NormalsArgs A;
   A.keys = S.keys;
   A.perm = S.perm;
   A.sx = S.soa;
   A.n = (int32_t)S.n, A.nf = (int32_t)S.nf, A.k = k, A.keff = (int32_t)std::min<int64_t>(k, S.nf);
+  A.p0 = (int32_t)p_begin, A.p1 = (int32_t)p_end;
   A.q = S.q;
   A.has_vp = viewpoint != nullptr;
   for (int a = 0; a < 3; ++a) A.vp[a] = viewpoint ? viewpoint[a] : 0.0;
   A.nrm = d_nrm, A.nbr = d_nbr, A.lists = d_lists, A.pairs = S.cnt + 1;
-  const int64_t want = (S.n + kWarpsPerBlock - 1) / kWarpsPerBlock;
+  const int64_t want = (p_end - p_begin + kWarpsPerBlock - 1) / kWarpsPerBlock;
   const unsigned grid = (unsigned)std::min<int64_t>(want, (int64_t)ctx->sm_count * 8);
   cudaStream_t st = ctx->stream;
   if (!d_lists)
@@ -431,6 +496,132 @@ int32_t rsc::knn_run(rsc_ctx* ctx, const KnnSearch& S, int32_t k, const double* 
     knn_normals_kernel<false, true><<<grid, 256, 0, st>>>(A);
   NRM_CUDA(cudaGetLastError());
   return RSC_OK;
+}
+
+// The check's record: int32 words summed over the ranks.  Every multi-bit value travels as 16-bit pieces, so that a
+// sum over up to 2^15 ranks cannot overflow; a rank compares each sum with R times its own value, R = the sum of the
+// ones.
+namespace {
+constexpr int kRecOne = 0, kRecNonEmpty = 1, kRecN = 2, kRecNGlobal = 6, kRecK = 10, kRecHasVp = 12, kRecOpt = 13,
+              kRecVp = 14, kRecWords = 26;
+
+void put16(int32_t* rec, int at, uint64_t v, int pieces) {
+  for (int p = 0; p < pieces; ++p) rec[at + p] = (int32_t)((v >> (16 * p)) & 0xffffu);
+}
+}  // namespace
+
+int32_t rsc::shard_check(rsc_ctx* ctx, Allocs& al, const char* fn, const char* own, int64_t n, int64_t n_global, int32_t k,
+                         const double* viewpoint, bool opt, const std::function<bool(bool)>& reserve, bool* opt_on) {
+  if (!ctx->allreduce)
+    return fail(ctx, RSC_E_STATE, (std::string(fn) + ": the context has no communicator (rsc_ctx_comm_init / rsc_ctx_set_allreduce)").c_str());
+  RSC_CUDA(ctx, cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  int32_t rec[kRecWords] = {}, sum[kRecWords];
+  rec[kRecOne] = 1;
+  rec[kRecNonEmpty] = n > 0;
+  put16(rec, kRecN, (uint64_t)n, 4);
+  put16(rec, kRecNGlobal, (uint64_t)n_global, 4);
+  put16(rec, kRecK, (uint32_t)k, 2);
+  rec[kRecHasVp] = viewpoint != nullptr;
+  rec[kRecOpt] = n > 0 && opt;
+  for (int a = 0; a < 3; ++a) {
+    uint64_t bits = 0;
+    if (viewpoint) memcpy(&bits, viewpoint + a, 8);
+    put16(rec, kRecVp + 4 * a, bits, 4);
+  }
+  int32_t* d_rec = nullptr;
+  NRM_CUDA(al.get((void**)&d_rec, sizeof(rec)));
+  NRM_CUDA(cudaMemcpyAsync(d_rec, rec, sizeof(rec), cudaMemcpyHostToDevice, st));
+  if (int32_t rc = rsc_ctx_allreduce(ctx, d_rec, kRecWords, st)) return rc;
+  NRM_CUDA(cudaMemcpyAsync(sum, d_rec, sizeof(sum), cudaMemcpyDeviceToHost, st));
+  NRM_CUDA(cudaStreamSynchronize(st));
+  const int64_t R = sum[kRecOne];
+  bool agree = true;
+  for (int w = kRecNGlobal; w < kRecWords; ++w)
+    if (w != kRecOpt) agree = agree && (int64_t)sum[w] == R * rec[w];
+  uint64_t sum_n = 0;
+  for (int p = 0; p < 4; ++p) sum_n += (uint64_t)(uint32_t)sum[kRecN + p] << (16 * p);
+  agree = agree && sum_n == (uint64_t)n_global;
+  agree = agree && (sum[kRecOpt] == 0 || sum[kRecOpt] == sum[kRecNonEmpty]);
+  // every buffer the collective steps need is allocated here, so that a rank short of memory fails with its peers
+  if (!own && agree && !reserve(sum[kRecOpt] > 0)) {
+    cudaGetLastError();  // (an allocation failure is not sticky: clear it)
+    own = "cannot allocate the device buffers of n_global points on this rank";
+  }
+  int32_t bad = own || !agree ? 1 : 0;
+  NRM_CUDA(cudaMemcpyAsync(d_rec, &bad, 4, cudaMemcpyHostToDevice, st));
+  if (int32_t rc = rsc_ctx_allreduce(ctx, d_rec, 1, st)) return rc;
+  NRM_CUDA(cudaMemcpyAsync(&bad, d_rec, 4, cudaMemcpyDeviceToHost, st));
+  NRM_CUDA(cudaStreamSynchronize(st));
+  if (bad > 0) {
+    const std::string msg = std::string(fn) + ": " +
+                            (own ? own : "the ranks' arguments disagree (k, n_global, viewpoint, optional outputs, or the sum of n)");
+    return fail(ctx, RSC_E_ARG, msg.c_str());
+  }
+  *opt_on = sum[kRecOpt] > 0;
+  return RSC_OK;
+}
+
+bool rsc::ShardBufs::reserve(rsc_ctx* ctx, int64_t n_global, bool with_nrm, int64_t row_words, KnnSearch& S) {
+  W = with_nrm ? 7 : 4;
+  words = row_words;
+  return knn_reserve(ctx, n_global, S) == RSC_OK && S.al.get((void**)&rec, (size_t)n_global * W * 4) == cudaSuccess &&
+         S.al.get((void**)&cnt, 3 * 8) == cudaSuccess && S.al.get((void**)&rows, (size_t)words * 4) == cudaSuccess &&
+         (!with_nrm || S.al.get((void**)&nrm, (size_t)n_global * 12) == cudaSuccess);
+}
+
+int32_t rsc::shard_gather(rsc_ctx* ctx, const char* fn, const float* xyz, const float* nrm, int64_t off, int64_t n,
+                          int64_t n_global, KnnSearch& S, const ShardBufs& B, ShardSlice& sl, PhaseClock& clk) {
+  cudaStream_t st = ctx->stream;
+  const int W = B.W;
+  int32_t* d_rec = B.rec;
+  unsigned long long* d_cnt = B.cnt;
+  float* d_nrm_all = B.nrm;
+  NRM_CUDA(cudaMemsetAsync(d_rec, 0, (size_t)n_global * W * 4, st));
+  NRM_CUDA(cudaMemsetAsync(d_cnt, 0, 3 * 8, st));
+  if (n > 0) {  // this rank's rows go through S.aos and d_nrm_all, which the unpack overwrites
+    NRM_CUDA(cudaMemcpyAsync(S.aos, xyz, (size_t)n * 12, cudaMemcpyHostToDevice, st));
+    if (d_nrm_all) NRM_CUDA(cudaMemcpyAsync(d_nrm_all, nrm, (size_t)n * 12, cudaMemcpyHostToDevice, st));
+    shard_pack_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(S.aos, d_nrm_all, n, off, W, d_rec);
+    NRM_CUDA(cudaGetLastError());
+  }
+  if (int32_t rc = rsc_ctx_allreduce(ctx, d_rec, n_global * W, st)) return rc;
+  shard_unpack_kernel<<<(unsigned)((n_global + 255) / 256), 256, 0, st>>>(d_rec, n_global, off, W, S.aos, d_nrm_all, d_cnt);
+  NRM_CUDA(cudaGetLastError());
+  unsigned long long got[3];
+  NRM_CUDA(cudaMemcpyAsync(got, d_cnt, sizeof(got), cudaMemcpyDeviceToHost, st));
+  NRM_CUDA(cudaStreamSynchronize(st));
+  clk.mark(ctx, 0);
+  if (got[0])  // the records are identical on every rank: all of them return here
+    return fail(ctx, RSC_E_ARG, (std::string(fn) + ": the ranks' ranges overlap or leave a gap in [0, n_global)").c_str());
+  if (int32_t rc = knn_sort(ctx, S)) return rc;
+  sl = ShardSlice{};
+  if (n > 0) {
+    const int64_t r = (int64_t)got[1], R = (int64_t)got[2], nf = S.nf;
+    sl.p_begin = nf * r / R;
+    sl.p_end = r == R - 1 ? n_global : nf * (r + 1) / R;
+  }
+  return RSC_OK;
+}
+
+rsc::PhaseClock::PhaseClock() {
+  const char* e = getenv("RSC_NORMALS_TRACE");
+  on = e && atoi(e) != 0;
+  if (on) t = std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count();
+}
+
+void rsc::PhaseClock::mark(rsc_ctx* ctx, int phase) {
+  if (!on) return;
+  cudaStreamSynchronize(ctx->stream);
+  const double now = std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count();
+  ms[phase] += 1e3 * (now - t);
+  t = now;
+}
+
+void rsc::PhaseClock::print(const char* fn, rsc_ctx* ctx) const {
+  if (on)
+    fprintf(stderr, "[%s] gather %.3f prepare %.3f search %.3f exchange %.3f forest %.3f ms | all-reduces %lld (%lld B)\n", fn,
+            ms[0], ms[1], ms[2], ms[3], ms[4], (long long)ctx->allreduce_calls, (long long)ctx->allreduce_bytes);
 }
 
 extern "C" int32_t rsc_estimate_normals(rsc_ctx* ctx, const float* xyz, int64_t n, int32_t k, const double* viewpoint, float* nrm,
@@ -445,7 +636,7 @@ extern "C" int32_t rsc_estimate_normals(rsc_ctx* ctx, const float* xyz, int64_t 
   if (int32_t rc = knn_prepare(ctx, xyz, n, S)) return rc;
   NRM_CUDA(S.al.get((void**)&d_nrm, (size_t)n * 12));
   if (nbr) NRM_CUDA(S.al.get((void**)&d_nbr, (size_t)n * k * 8));
-  if (int32_t rc = knn_run(ctx, S, k, viewpoint, d_nrm, d_nbr, nullptr)) return rc;
+  if (int32_t rc = knn_run(ctx, S, k, viewpoint, d_nrm, d_nbr, nullptr, 0, n)) return rc;
   cudaStream_t st = ctx->stream;
   if (int32_t rc = staged_d2h(ctx, nrm, d_nrm, (size_t)n * 12, st)) return rc;
   if (nbr)
@@ -453,7 +644,54 @@ extern "C" int32_t rsc_estimate_normals(rsc_ctx* ctx, const float* xyz, int64_t 
   unsigned long long np = 0;
   NRM_CUDA(cudaMemcpyAsync(&np, S.cnt + 1, 8, cudaMemcpyDeviceToHost, st));
   NRM_CUDA(cudaStreamSynchronize(st));
-#undef NRM_CUDA
   if (pairs) *pairs = (int64_t)np;
   return RSC_OK;
 }
+
+const char* rsc::shard_own_problem(int64_t n, int64_t off, int64_t n_global, int32_t k, const void* xyz, const void* out) {
+  if (k < 3 || k > 32) return "k must be in [3, 32]";
+  if (n_global < 1 || n_global >= ((int64_t)1 << 31)) return "n_global must be in [1, 2^31)";
+  if (n < 0 || off < 0 || off > n_global - n) return "[global_offset, global_offset + n) must lie in [0, n_global)";
+  if (n > 0 && (!xyz || !out)) return "the coordinates and the output normals must not be NULL when n > 0";
+  return nullptr;
+}
+
+extern "C" int32_t rsc_estimate_normals_shard(rsc_ctx* ctx, const float* xyz, int64_t n, int64_t global_offset, int64_t n_global,
+                                              int32_t k, const double* viewpoint, float* nrm, int64_t* nbr, int64_t* pairs) {
+  constexpr const char* fn = "estimate_normals_shard";
+  if (!ctx) return RSC_E_ARG;
+  KnnSearch S;
+  ShardBufs B;
+  PhaseClock clk;
+  bool with_nbr = false;
+  // the rows, zero-filled and completed by one all-reduce: [n_global k] int64 lists (when asked for), [3 n_global] normals
+  auto reserve = [&](bool lists) { return B.reserve(ctx, n_global, false, n_global * (3 + (lists ? 2 * (int64_t)k : 0)), S); };
+  if (int32_t rc = shard_check(ctx, S.al, fn, shard_own_problem(n, global_offset, n_global, k, xyz, nrm), n, n_global, k,
+                               viewpoint, nbr != nullptr, reserve, &with_nbr))
+    return rc;
+  ShardSlice sl;
+  if (int32_t rc = shard_gather(ctx, fn, xyz, nullptr, global_offset, n, n_global, S, B, sl, clk)) return rc;
+  clk.mark(ctx, 1);
+  const int64_t words = B.words;
+  int32_t* d_rows = B.rows;
+  int64_t* d_nbr = with_nbr ? reinterpret_cast<int64_t*>(d_rows) : nullptr;
+  float* d_nrm = reinterpret_cast<float*>(d_rows + (with_nbr ? 2 * (int64_t)k * n_global : 0));
+  cudaStream_t st = ctx->stream;
+  NRM_CUDA(cudaMemsetAsync(d_rows, 0, (size_t)words * 4, st));
+  if (int32_t rc = knn_run(ctx, S, k, viewpoint, d_nrm, d_nbr, nullptr, sl.p_begin, sl.p_end)) return rc;
+  clk.mark(ctx, 2);
+  if (int32_t rc = rsc_ctx_allreduce(ctx, d_rows, words, st)) return rc;
+  if (n > 0) {
+    if (int32_t rc = staged_d2h(ctx, nrm, d_nrm + 3 * global_offset, (size_t)n * 12, st)) return rc;
+    if (nbr)
+      if (int32_t rc = staged_d2h(ctx, nbr, d_nbr + global_offset * k, (size_t)n * k * 8, st)) return rc;
+  }
+  unsigned long long np = 0;
+  NRM_CUDA(cudaMemcpyAsync(&np, S.cnt + 1, 8, cudaMemcpyDeviceToHost, st));
+  NRM_CUDA(cudaStreamSynchronize(st));
+  clk.mark(ctx, 3);
+  clk.print(fn, ctx);
+  if (pairs) *pairs = (int64_t)np;
+  return RSC_OK;
+}
+#undef NRM_CUDA

@@ -258,40 +258,31 @@ inline unsigned blocks_of(int64_t n) { return (unsigned)((n + 255) / 256); }
 
 using namespace rsc;
 
-extern "C" int32_t rsc_orient_normals(rsc_ctx* ctx, const float* xyz, int64_t n, int32_t k, const float* nrm_in, float* nrm_out,
-                                      int64_t* edges, int64_t* stats) {
-  if (!ctx) return RSC_E_ARG;
-  if (!xyz || !nrm_out) return fail(ctx, RSC_E_ARG, "orient_normals: xyz and nrm_out must not be NULL");
-  if (k < 3 || k > 32) return fail(ctx, RSC_E_ARG, "orient_normals: k must be in [3, 32]");
-  if (n < 1 || n >= ((int64_t)1 << 31)) return fail(ctx, RSC_E_ARG, "orient_normals: n must be in [1, 2^31)");
-  KnnSearch S;
-  if (int32_t rc = knn_prepare(ctx, xyz, n, S)) return rc;
 #define ORI_CUDA(expr) RSC_CUDA(ctx, (expr))
+
+int32_t rsc::orient_reserve(rsc_ctx* ctx, Allocs& al, int64_t n, OrientScratch& O) {
+  ORI_CUDA(al.get((void**)&O.u, (size_t)n * 24));
+  ORI_CUDA(al.get((void**)&O.word, (size_t)n * 4));
+  ORI_CUDA(al.get((void**)&O.link, (size_t)n * 4));
+  ORI_CUDA(al.get((void**)&O.cnt, (size_t)n * 4));
+  ORI_CUDA(al.get((void**)&O.offs, (size_t)n * 8));
+  ORI_CUDA(al.get((void**)&O.best_w, (size_t)n * 8));
+  ORI_CUDA(al.get((void**)&O.best_e, (size_t)n * 8));
+  ORI_CUDA(al.get((void**)&O.tree, (size_t)n * 8));
+  ORI_CUDA(al.get((void**)&O.scal, 4 * 8));  // [0] vertices, [1] tree edges, [2] edges, [3] changed
+  ORI_CUDA(cudaMemsetAsync(O.scal, 0, 4 * 8, ctx->stream));
+  return RSC_OK;
+}
+
+int32_t rsc::orient_forest(rsc_ctx* ctx, Allocs& al, const OrientScratch& O, const float* d_xyz, float* d_nrm,
+                           const int32_t* d_lists, int64_t n, int32_t k, int64_t* edges, int64_t* stats) {
   cudaStream_t st = ctx->stream;
-  Allocs& al = S.al;
-  float* d_nrm = nullptr;
-  int32_t* d_lists = nullptr;
-  double* d_u = nullptr;
-  uint32_t *d_word = nullptr, *d_link = nullptr, *d_cnt = nullptr;
-  unsigned long long *d_best_w = nullptr, *d_best_e = nullptr, *d_tree = nullptr, *d_offs = nullptr, *d_scal = nullptr;
-  ORI_CUDA(al.get((void**)&d_nrm, (size_t)n * 12));
-  ORI_CUDA(al.get((void**)&d_lists, (size_t)n * k * 4));
-  ORI_CUDA(al.get((void**)&d_u, (size_t)n * 24));
-  ORI_CUDA(al.get((void**)&d_word, (size_t)n * 4));
-  ORI_CUDA(al.get((void**)&d_link, (size_t)n * 4));
-  ORI_CUDA(al.get((void**)&d_cnt, (size_t)n * 4));
-  ORI_CUDA(al.get((void**)&d_offs, (size_t)n * 8));
-  ORI_CUDA(al.get((void**)&d_best_w, (size_t)n * 8));
-  ORI_CUDA(al.get((void**)&d_best_e, (size_t)n * 8));
-  ORI_CUDA(al.get((void**)&d_tree, (size_t)n * 8));
-  ORI_CUDA(al.get((void**)&d_scal, 4 * 8));  // [0] vertices, [1] tree edges, [2] edges, [3] changed
-  ORI_CUDA(cudaMemsetAsync(d_scal, 0, 4 * 8, st));
-  if (nrm_in) ORI_CUDA(cudaMemcpyAsync(d_nrm, nrm_in, (size_t)n * 12, cudaMemcpyHostToDevice, st));
-  // one search: the lists, and the normals too when none are given
-  if (int32_t rc = knn_run(ctx, S, k, nullptr, nrm_in ? nullptr : d_nrm, nullptr, d_lists)) return rc;
+  double* d_u = O.u;
+  uint32_t *d_word = O.word, *d_link = O.link, *d_cnt = O.cnt;
+  unsigned long long *d_best_w = O.best_w, *d_best_e = O.best_e, *d_tree = O.tree, *d_offs = O.offs, *d_scal = O.scal;
 
   const unsigned nb = blocks_of(n);
-  setup_kernel<<<nb, 256, 0, st>>>(S.aos, d_nrm, n, d_u, d_word, d_scal);
+  setup_kernel<<<nb, 256, 0, st>>>(d_xyz, d_nrm, n, d_u, d_word, d_scal);
   ORI_CUDA(cudaGetLastError());
   edges_kernel<false><<<nb, 256, 0, st>>>(d_lists, k, n, d_word, d_u, d_cnt, nullptr, nullptr);
   ORI_CUDA(cudaGetLastError());
@@ -348,13 +339,13 @@ extern "C" int32_t rsc_orient_normals(rsc_ctx* ctx, const float* xyz, int64_t n,
 
   // roots and signs (d_best_w holds the root keys)
   ORI_CUDA(cudaMemsetAsync(d_best_w, 0, (size_t)n * 8, st));
-  root_kernel<<<nb, 256, 0, st>>>(n, S.aos, d_word, d_best_w);
+  root_kernel<<<nb, 256, 0, st>>>(n, d_xyz, d_word, d_best_w);
   ORI_CUDA(cudaGetLastError());
   sign_kernel<<<nb, 256, 0, st>>>(n, d_word, d_best_w, d_u, d_nrm, d_nrm);
   ORI_CUDA(cudaGetLastError());
   unsigned long long ntree = 0;
   ORI_CUDA(cudaMemcpyAsync(&ntree, d_scal + 1, 8, cudaMemcpyDeviceToHost, st));
-  if (int32_t rc = staged_d2h(ctx, nrm_out, d_nrm, (size_t)n * 12, st)) return rc;
+  ORI_CUDA(cudaStreamSynchronize(st));
   if (edges && ntree) {  // F's edges in ascending (lo, hi) order
     cub::DoubleBuffer<unsigned long long> kb(d_tree, d_best_e);
     size_t tmp_bytes = 0;
@@ -367,8 +358,6 @@ extern "C" int32_t rsc_orient_normals(rsc_ctx* ctx, const float* xyz, int64_t n,
     ORI_CUDA(cudaGetLastError());
     if (int32_t rc = staged_d2h(ctx, edges, d_pairs, (size_t)ntree * 16, st)) return rc;
   }
-  ORI_CUDA(cudaStreamSynchronize(st));
-#undef ORI_CUDA
   if (stats) {
     stats[0] = nvert;
     stats[1] = (int64_t)ntree;
@@ -377,3 +366,67 @@ extern "C" int32_t rsc_orient_normals(rsc_ctx* ctx, const float* xyz, int64_t n,
   }
   return RSC_OK;
 }
+
+extern "C" int32_t rsc_orient_normals(rsc_ctx* ctx, const float* xyz, int64_t n, int32_t k, const float* nrm_in, float* nrm_out,
+                                      int64_t* edges, int64_t* stats) {
+  if (!ctx) return RSC_E_ARG;
+  if (!xyz || !nrm_out) return fail(ctx, RSC_E_ARG, "orient_normals: xyz and nrm_out must not be NULL");
+  if (k < 3 || k > 32) return fail(ctx, RSC_E_ARG, "orient_normals: k must be in [3, 32]");
+  if (n < 1 || n >= ((int64_t)1 << 31)) return fail(ctx, RSC_E_ARG, "orient_normals: n must be in [1, 2^31)");
+  KnnSearch S;
+  OrientScratch O;
+  if (int32_t rc = knn_prepare(ctx, xyz, n, S)) return rc;
+  cudaStream_t st = ctx->stream;
+  float* d_nrm = nullptr;
+  int32_t* d_lists = nullptr;
+  ORI_CUDA(S.al.get((void**)&d_nrm, (size_t)n * 12));
+  ORI_CUDA(S.al.get((void**)&d_lists, (size_t)n * k * 4));
+  if (int32_t rc = orient_reserve(ctx, S.al, n, O)) return rc;
+  if (nrm_in) ORI_CUDA(cudaMemcpyAsync(d_nrm, nrm_in, (size_t)n * 12, cudaMemcpyHostToDevice, st));
+  // one search: the lists, and the normals too when none are given
+  if (int32_t rc = knn_run(ctx, S, k, nullptr, nrm_in ? nullptr : d_nrm, nullptr, d_lists, 0, n)) return rc;
+  if (int32_t rc = orient_forest(ctx, S.al, O, S.aos, d_nrm, d_lists, n, k, edges, stats)) return rc;
+  if (int32_t rc = staged_d2h(ctx, nrm_out, d_nrm, (size_t)n * 12, st)) return rc;
+  return RSC_OK;
+}
+
+extern "C" int32_t rsc_orient_normals_shard(rsc_ctx* ctx, const float* xyz, int64_t n, int64_t global_offset, int64_t n_global,
+                                            int32_t k, const float* nrm_in, float* nrm_out, int64_t* edges, int64_t* stats) {
+  constexpr const char* fn = "orient_normals_shard";
+  if (!ctx) return RSC_E_ARG;
+  KnnSearch S;
+  ShardBufs B;
+  OrientScratch O;
+  PhaseClock clk;
+  bool given = false;
+  // given normals travel with the coordinates; estimated ones come back with the lists: [n_global k] int32 lists,
+  // then [3 n_global] normals, zero-filled and completed by one all-reduce
+  auto reserve = [&](bool with_nrm) {
+    return B.reserve(ctx, n_global, with_nrm, n_global * ((int64_t)k + (with_nrm ? 0 : 3)), S) &&
+           orient_reserve(ctx, S.al, n_global, O) == RSC_OK;
+  };
+  if (int32_t rc = shard_check(ctx, S.al, fn, shard_own_problem(n, global_offset, n_global, k, xyz, nrm_out), n, n_global, k,
+                               nullptr, nrm_in != nullptr, reserve, &given))
+    return rc;
+  ShardSlice sl;
+  if (int32_t rc = shard_gather(ctx, fn, xyz, nrm_in, global_offset, n, n_global, S, B, sl, clk)) return rc;
+  clk.mark(ctx, 1);
+  const int64_t words = B.words;
+  int32_t* d_rows = B.rows;
+  float* d_nrm = given ? B.nrm : reinterpret_cast<float*>(d_rows + (int64_t)k * n_global);
+  cudaStream_t st = ctx->stream;
+  ORI_CUDA(cudaMemsetAsync(d_rows, 0, (size_t)words * 4, st));
+  if (int32_t rc = knn_run(ctx, S, k, nullptr, given ? nullptr : d_nrm, nullptr, d_rows, sl.p_begin, sl.p_end)) return rc;
+  clk.mark(ctx, 2);
+  if (int32_t rc = rsc_ctx_allreduce(ctx, d_rows, words, st)) return rc;
+  clk.mark(ctx, 3);
+  // the forest, replicated on identical inputs: identical on every rank
+  if (int32_t rc = orient_forest(ctx, S.al, O, S.aos, d_nrm, d_rows, n_global, k, edges, stats)) return rc;
+  if (n > 0)
+    if (int32_t rc = staged_d2h(ctx, nrm_out, d_nrm + 3 * global_offset, (size_t)n * 12, st)) return rc;
+  ORI_CUDA(cudaStreamSynchronize(st));
+  clk.mark(ctx, 4);
+  clk.print(fn, ctx);
+  return RSC_OK;
+}
+#undef ORI_CUDA

@@ -8,6 +8,9 @@ K5 hits and the cleared enabled words are summed with NCCL **inside the library*
 (`rsc_ctx_comm_init`; torch.distributed only carries the 128-byte NCCL id from rank 0 to the others).
 `ShardedContext` is the older replicated-storage layout (whole cloud on every rank + a range per rank),
 which also supports the extension switches; it can use the library's NCCL too or a host callback.
+`attach_comm` puts either communicator on a bare `Context`, for the sharded normals:
+
+    orient_normals(V[lo:hi], shard=(lo, n), ctx=ctx) -> ShardedCloud(V[lo:hi], N_lo_hi, subsets, (lo, hi), n) -> ransac()
 """
 from __future__ import annotations
 
@@ -93,13 +96,55 @@ def ShardedCloud(vertices_local, normals_local, subsets, rank_range: Tuple[int, 
     return pc
 
 
+def attach_comm(ctx, group=None, comm: str = "nccl") -> None:
+    """Puts a communicator on a bare `Context`, as the collective calls on it need (`estimate_normals(...,
+    shard=...)`, `orient_normals(..., shard=...)`, sharded clouds).  comm="nccl": the library's own NCCL
+    (`init_comm`); "callback": a host callback into torch.distributed on device tensors (rsc_ctx_set_allreduce);
+    "host": the same callback staged through host memory (any torch.distributed backend, e.g. gloo: ranks may then
+    share a GPU)."""
+    if comm == "nccl":
+        init_comm(ctx, group)
+        return
+    import torch
+    import torch.distributed as dist
+
+    ext = torch.cuda.ExternalStream(ctx.stream, device=torch.device("cuda", ctx.device))
+    host_staged = comm == "host"
+
+    def _allreduce(user, ptr, count, stream):
+        try:
+            t = torch.as_tensor(_DevInt32(ptr, count), device=torch.device("cuda", ctx.device))
+            with torch.cuda.stream(ext):
+                if host_staged:
+                    h = t.cpu()
+                    dist.all_reduce(h, group=group)
+                    t.copy_(h)
+                else:
+                    dist.all_reduce(t, group=group)
+            return 0
+        except Exception as e:  # never let an exception cross the C boundary
+            print(f"[rsc] all-reduce callback failed: {e!r}")
+            return 1
+
+    ctx._allreduce_cb = _lib.ALLREDUCE_FN(_allreduce)  # keep alive while installed
+    ctx.check(lib.rsc_ctx_set_allreduce(ctx.h, C.cast(ctx._allreduce_cb, C.c_void_p), None))
+
+
+def detach_comm(ctx) -> None:
+    """Removes what `attach_comm` put on `ctx`."""
+    if getattr(ctx, "_comm", False):
+        close_comm(ctx)
+    else:
+        lib.rsc_ctx_set_allreduce(ctx.h, None, None)
+        ctx._allreduce_cb = None
+
+
 class ShardedContext:
     """Replicated storage: installs an all-reduce (host callback into torch.distributed, or the library's
     NCCL with comm="nccl") on a context and the rank's point range on a cloud.  comm="host" stages the
     callback through host memory (any torch.distributed backend, e.g. gloo: ranks may then share a GPU)."""
 
     def __init__(self, pc, group=None, set_range: bool = True, comm: str = "callback"):
-        import torch
         import torch.distributed as dist
 
         self.pc = pc
@@ -107,39 +152,14 @@ class ShardedContext:
         self.world = dist.get_world_size(group)
         self.range = partition(pc.size, self.world)[self.rank]
         self.comm = comm
-        if comm == "nccl":
-            init_comm(pc.ctx, group)
-        else:
-            ext = torch.cuda.ExternalStream(pc.ctx.stream, device=torch.device("cuda", pc.ctx.device))
-            host_staged = comm == "host"  # e.g. a gloo group: several ranks may then share one GPU (tests)
-
-            def _allreduce(user, ptr, count, stream):
-                try:
-                    t = torch.as_tensor(_DevInt32(ptr, count), device=torch.device("cuda", pc.ctx.device))
-                    with torch.cuda.stream(ext):
-                        if host_staged:
-                            h = t.cpu()
-                            dist.all_reduce(h, group=group)
-                            t.copy_(h)
-                        else:
-                            dist.all_reduce(t, group=group)
-                    return 0
-                except Exception as e:  # never let an exception cross the C boundary
-                    print(f"[rsc] all-reduce callback failed: {e!r}")
-                    return 1
-
-            self._cb = _lib.ALLREDUCE_FN(_allreduce)  # keep alive
-            pc.ctx.check(lib.rsc_ctx_set_allreduce(pc.ctx.h, C.cast(self._cb, C.c_void_p), None))
+        attach_comm(pc.ctx, group, comm)
         if set_range:
             lo, hi = self.range  # an empty range (lo == hi) is a rank that only joins the all-reduces
             pc.ctx.check(lib.rsc_cloud_set_range(pc.handle, lo, hi))
             pc.ranged = True  # (ransac() keeps such a cloud out of rsc_ransac_run_user)
 
     def close(self):
-        if self.comm == "nccl":
-            close_comm(self.pc.ctx)
-        else:
-            lib.rsc_ctx_set_allreduce(self.pc.ctx.h, None, None)
+        detach_comm(self.pc.ctx)
 
 
 def gather_extracted(extracted, group=None):
